@@ -25,6 +25,7 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True        # the bench writes nothing into the tree it runs from (which may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "model-based-policy-optimizers_b200"))
 
@@ -67,6 +68,16 @@ def random_states(n, seed):
     rng = np.random.default_rng(seed)
     th, w = rng.uniform(-np.pi, np.pi, n), rng.uniform(-8, 8, n)
     return np.stack([np.cos(th), np.sin(th), w], -1).astype(np.float32)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy.  Floats keep their dtype; integer words (PRNG keys) are stored as
+    float64, which holds every uint32 exactly.  The plan workloads return at most ~0.6 MB per GPU, so everything is
+    written."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 class ClockSampler:
@@ -267,6 +278,14 @@ def run_ours(args, wl_name, wl):
     ms_per_step = ms_total / args.steps
     value = tr_step * world / (ms_per_step * 1e-3)
     clocks = clk.summary()
+    if args.dump_outputs:
+        # the last timed step's result, every rank's problems in global order
+        outs = {"best_sequence": new_state.best_sequence, "best_reward": new_state.best_reward,
+                "key": new_state.key.view(torch.int32)}
+        outs = {k: all_gather_blocks(v.contiguous(), total_B).cpu().numpy() for k, v in outs.items()}
+        outs["key"] = outs["key"].view(np.uint32)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
 
     # ---- end to end through the public API with host buffers ------------------------------------
     act_host = torch.empty((B, 1), dtype=torch.float32).pin_memory()
@@ -370,7 +389,7 @@ def measure_others(args):
                 continue
             a = SimpleNamespace(**vars(args))
             a.impl, a.workload = impl, name
-            a.steps = min(args.steps, 5) if impl == "ours" else 1
+            a.steps = args.steps if impl == "ours" else 1
             a.warmup = 3 if impl == "ours" else 1
             _CAPTURE = []
             try:
@@ -638,7 +657,7 @@ def run_ensemble(args):
         torch.cuda.synchronize(dev)
     for _ in range(max(args.warmup, 3)):
         opt.optimize(x0, state)
-    steps = min(args.steps, 20)
+    steps = args.steps
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     with ClockSampler(local_rank) as clk:
@@ -659,11 +678,11 @@ def run_ensemble(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize(dev)
     e0.record()
-    for _ in range(5):
+    for _ in range(steps):
         system.ensemble_returns(sp, x0, acts)
     e1.record()
     torch.cuda.synchronize(dev)
-    k_ms = e0.elapsed_time(e1) / 5
+    k_ms = e0.elapsed_time(e1) / steps
     act_host = torch.empty((B, 1), dtype=torch.float32).pin_memory()
     barrier()
     t0 = time.perf_counter()
@@ -774,7 +793,7 @@ def run_closed_loop(args):
     for _ in range(max(args.warmup, 3)):
         cem.closed_loop(x0, st, MPC_T)
     torch.cuda.synchronize(dev)
-    steps = min(args.steps, 20)
+    steps = args.steps
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)
@@ -848,12 +867,12 @@ def run_sweep(args):
         rows = []
         for B in (1, 8, 64, 512):
             w = dict(wl, B=B)
-            r = cpu_reference_step(w, steps=1, warmup=1, sample_B=B)
+            r = cpu_reference_step(w, steps=args.steps, warmup=args.warmup, sample_B=B)
             rows.append({"problems": B, "ms": r["ms_per_step"], "transitions_per_s": r["value"], "cores": r["cores"]})
         ncores, model = host_info()
         best = max(rows, key=lambda r: r["transitions_per_s"])
         emit_json({"impl": "reference", "metric": METRIC, "value": best["transitions_per_s"], "unit": UNIT,
-                   "n_gpus": args.gpus, "steps": 1, "warmup": 1, "ms_per_step": best["ms"], "higher_is_better": True,
+                   "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": best["ms"], "higher_is_better": True,
                    "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                    "config": {"workload": "config5_sweep", "horizon": H, "num_samples": 512},
                    "sweep": rows,
@@ -887,7 +906,6 @@ def run_sweep(args):
         if n > 0:
             state = opt.init(keys)
             x0 = torch.from_numpy(random_states(B, 0)[lo:hi].copy()).to(dev)
-        steps = 20 if B <= 4096 else (5 if B <= 32768 else 2)
         for _ in range(3):
             if n > 0:
                 opt.optimize(x0, state)
@@ -897,19 +915,19 @@ def run_sweep(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with ClockSampler(local_rank) as clk:
             e0.record()
-            for _ in range(steps):
+            for _ in range(args.steps):
                 if n > 0:
                     opt.optimize(x0, state)
             e1.record()
             torch.cuda.synchronize(dev)
-        ms = e0.elapsed_time(e1) / steps
+        ms = e0.elapsed_time(e1) / args.steps
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
         row = {"problems": B, "ms_per_plan_call": ms, "transitions_per_s": transitions_per_step(B, H, p) / (ms * 1e-3)}
         # end to end through iCemTO.act with host buffers (states from pinned memory, first actions back) at this B
-        e2e_steps = max(steps // 2, 1)
+        e2e_steps = args.steps
         if n > 0:
             xh = x0.cpu().pin_memory()
             ah = torch.empty((n, 1), dtype=torch.float32).pin_memory()
@@ -970,7 +988,7 @@ def run_sweep(args):
         best = max(rows, key=lambda r: r["transitions_per_s"])
         for row in rows:
             row["frac_algorithmic"] = row["transitions_per_s"] * ALGORITHMIC_LANE_INSTR_PER_TRANSITION / 1e12 / issue_peak
-        emit_json({"metric": METRIC, "value": top["transitions_per_s"], "unit": UNIT, "n_gpus": world, "steps": 2,
+        emit_json({"metric": METRIC, "value": top["transitions_per_s"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
                    "warmup": 3, "ms_per_step": top["ms_per_plan_call"], "higher_is_better": True, "scaling": "strong",
                    "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                    "config": {"workload": "config5_sweep", "problems_total": [r["problems"] for r in rows], "horizon": H,
@@ -978,7 +996,7 @@ def run_sweep(args):
                               "parallelism": "problems sharded x%d" % world,
                               "l2": "back-to-back launches; per-problem state is ~0.4 KB and the kernel works out of shared memory"},
                    "math_mode": args.math, "sweep": rows, "clocks": clocks,
-                   "gpu_launches": sum((20 if r["problems"] <= 4096 else (5 if r["problems"] <= 32768 else 2)) * 2 for r in rows),
+                   "gpu_launches": 2 * args.steps * len(rows),
                    "roofline": {"bound": "issue", "kernel": "icem_plan_pendulum_kernel (clusters below 148 problems)",
                                 "achieved": best["transitions_per_s"] * ALGORITHMIC_LANE_INSTR_PER_TRANSITION / 1e12,
                                 "peak": issue_peak, "unit": "T lane-instr/s", "frac": best["frac_algorithmic"],
@@ -1079,7 +1097,7 @@ def run_actor(args):
         torch.cuda.synchronize(dev)
     for _ in range(max(args.warmup, 3)):
         acting.get_experience(env, st, policy, key, T, env_offset=lo, total_envs=total_E)
-    steps = min(args.steps, 10)
+    steps = args.steps
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     with ClockSampler(local_rank) as clk:
@@ -1228,7 +1246,7 @@ def run_collect(args):
 
     for _ in range(max(args.warmup, 3)):
         norm, state, buf = col.get_experience(norm, params, state, buf, key); key = col.last_key
-    steps = min(args.steps, 20)
+    steps = args.steps
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     with ClockSampler(local_rank) as clk:
@@ -1384,7 +1402,7 @@ def run_bptt(args):
         return lv, g_a
     for _ in range(max(args.warmup, 3)):
         step(x0)
-    steps = min(args.steps, 20)
+    steps = args.steps
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
@@ -1609,7 +1627,10 @@ def run_replay(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed steps: every timed loop of the workload (and of the `others` entries of the default "
+                         "line; of every sweep point) runs exactly this many.  The `cpu_baseline` leg of a GPU line "
+                         "times one step on a bounded sample; --impl reference times --steps steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=sorted(WORKLOADS) + ["config1_closed_loop", "config3_env_rollouts", "config3_actor_rollouts",
@@ -1627,7 +1648,15 @@ def main():
                     help="config3_actor_rollouts: which kernel runs the policy network")
     ap.add_argument("--env-sequential", action="store_true",
                     help="config3_env_rollouts: time the one-thread-per-env scan instead of the episode-piece kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed plan call returned (best_sequence, best_reward, key) as "
+                         "DIR/<name>.npy; inputs are seeded, so runs with the same arguments compare output for output "
+                         "(the iCEM plan workloads of the CUDA path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs is implemented for the CUDA path of %s" % ", ".join(sorted(WORKLOADS)))
     global GUARD
     with _StdoutGuard() as GUARD:
         if args.workload == "config3_env_rollouts":

@@ -6,6 +6,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -31,15 +32,20 @@ def build(native: bool = False, out: str | None = None) -> str:
 
 
 def load(native: bool = False) -> C.CDLL:
-    path = LIB
     if native:
-        try:
-            path = build(native=True)
-        except Exception:
-            path = LIB
-    if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(os.path.join(_DIR, "mbpo_oracle.c")):
+        # built in a temporary directory, so that the tree stays untouched (it may be read-only); the loaded
+        # library outlives its deleted file
+        with tempfile.TemporaryDirectory(prefix="mbpo_oracle_") as tmp:
+            try:
+                return _declare(C.CDLL(build(native=True, out=os.path.join(tmp, "libmbpo_oracle_native.so"))))
+            except Exception:
+                pass
+    if not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(os.path.join(_DIR, "mbpo_oracle.c")):
         build()
-    lib = C.CDLL(path)
+    return _declare(C.CDLL(LIB))
+
+
+def _declare(lib: C.CDLL) -> C.CDLL:
     lib.orc_icem_optimize_batch.restype = C.c_int
     lib.orc_env_rollout.restype = C.c_int
     lib.orc_max_threads.restype = C.c_int

@@ -53,7 +53,8 @@ def _worker(rank, world, port, total, out_dir):
     st = iCemOptimizerState(key=keys, best_sequence=torch.zeros((total, 4, 1)), best_reward=torch.zeros(total))
     actions, new_state, (lo, hi) = plan_sharded(_FakeOptimizer(), x, st)
     want, _ = _FakeOptimizer().act(x, st)
-    assert actions.shape == (total, 1) and torch.equal(actions, want)          # gather == unsharded result
+    # gather == unsharded result (plan_sharded plans on the GPU when there is one)
+    assert actions.shape == (total, 1) and torch.equal(actions.cpu(), want)
     assert (lo, hi) == shard_bounds(total, rank, world)
     assert new_state.best_reward.shape[0] == hi - lo                           # state stays sharded
     blk = torch.arange(lo, hi, dtype=torch.float32).reshape(-1, 1)
