@@ -291,6 +291,22 @@ int mbpo_env_unroll(int system_kind, const void* sys_params_host, int math_mode,
                     float* observation_out, float* reward_out, float* discount_out,
                     float* next_observation_out, float* truncation_out, void* stream);
 
+/* mbpo_env_unroll for the general Systems (csrc/systems.cuh): MBPO_SYSTEM_NOISY_PENDULUM (X = 3, A = 1, keyed) and
+ * MBPO_SYSTEM_POINT_MASS (X = 4, A = 2).  MBPO_SYSTEM_PENDULUM is MBPO_EINVAL here (it keeps mbpo_env_unroll /
+ * mbpo_env_rollout); any other kind is MBPO_EUNSUPPORTED.  Same wrapper stack, layouts and overlapping-buffer
+ * convention as mbpo_env_unroll, with actions [T,E,A].  sys_keys_in / sys_keys_out: uint32 [E,2], every env's
+ * system_params.key before / after the T steps -- required for a keyed System, ignored (may be NULL) otherwise.
+ * Each System.step advances the key once (key, sub = split(key)), so it advances action_repeat times per env step,
+ * and AutoReset does not reset it.  The outgoing state may alias the incoming one.  T == 0 copies the state
+ * through.  X = 4 needs 16-byte aligned observation buffers. */
+int mbpo_env_unroll_general(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode,
+                            int episode_length, int action_repeat, const float* obs_in, const float* steps_in,
+                            const float* done_in, const uint32_t* sys_keys_in /*[E,2] or NULL*/, float* obs_out,
+                            float* steps_out, float* done_out, uint32_t* sys_keys_out, const float* first_obs,
+                            const float* actions /*[T,E,A]*/, int E, int T, float* observation_out,
+                            float* reward_out, float* discount_out, float* next_observation_out,
+                            float* truncation_out, void* stream);
+
 /* ---- policy in the env loop: SAC / PPO data collection ------------------------------------- */
 /* The stochastic policy of sac/sac_networks.py:58-73 + sac/parametric_distribution.py:97-125:
  * logits = MLP(obs) (swish; Dense = x @ W + b), loc, scale = split(logits, 2),
@@ -358,6 +374,24 @@ int mbpo_actor_rollout_extras(int system_kind, const void* sys_params_host, int 
                               float* action_out, float* reward_out, float* discount_out,
                               float* next_observation_out, float* truncation_out, uint32_t* key_out,
                               float* raw_action_out, float* log_prob_out, void* stream);
+
+/* mbpo_actor_rollout_extras for the general Systems (see mbpo_env_unroll_general for the kinds and their refusals):
+ * the policy kernel on the CUDA cores with obs_dim = X and action_dim = A (width 64, 1..4 hidden layers), the
+ * NormalTanh head, all three key conventions, deterministic mode and PPO's extras (log_prob summed over the A
+ * action dims, raw_action_out [T,E,A]).  The policy's draw is normal(key, (draw_total, A)) flattened: env e, dim a
+ * reads element (draw_offset + e) * A + a, so a sharded launch reproduces the unsharded one.  obs / steps / done are
+ * updated in place; sys_keys_in / sys_keys_out as in mbpo_env_unroll_general.  The general Systems have one math
+ * (every operation rounded once), so there is no math_mode.  MBPO_EUNSUPPORTED: MBPO_HEAD_BPTT_ACTOR (or
+ * shared_noise), kernel = MBPO_ACTOR_TCGEN05 / MBPO_ACTOR_TCGEN05_WIDE, and policy shapes other than the above;
+ * MBPO_ACTOR_AUTO selects the CUDA-core kernel. */
+int mbpo_actor_rollout_general(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode,
+                               const MbpoPolicyParams* policy_host, int deterministic, int key_convention,
+                               const uint32_t* key_in, int episode_length, int action_repeat, float* obs,
+                               float* steps, float* done, const uint32_t* sys_keys_in /*[E,2] or NULL*/,
+                               uint32_t* sys_keys_out, const float* first_obs, int E, int T, float* action_out,
+                               float* reward_out, float* discount_out, float* next_observation_out,
+                               float* truncation_out, uint32_t* key_out, float* raw_action_out,
+                               float* log_prob_out, void* stream);
 
 /* ---- reverse pass through System.step rollouts; lambda returns (BPTT) ----------------------- */
 /* The cotangent pass of jax.value_and_grad through rollout_policy(..., stop_grads=True)

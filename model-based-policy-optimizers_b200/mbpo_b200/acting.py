@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from .config import config
-from .envs import EnvState, VmappedSystemEnv
+from .envs import EnvState, VmappedSystemEnv, is_general, system_keys
 from .utils.optimizer_utils import Transition
 
 
@@ -36,8 +36,9 @@ class Policy:
         """obs_mean / obs_std: the running-statistics normaliser the reference passes as ``normalizer_params``
         (``policy_network.apply(normalizer_params, policy_params, obs)``: (obs - mean) / std); emit_extras: PPO's
         policy also returns {'log_prob', 'raw_action'} (ppo_network.py:72-80); kernel: "auto" (tcgen05 for 2..3
-        hidden layers -- the wide latency kernel when the envs do not fill the GPU --, CUDA cores otherwise),
-        "cuda_cores", "tcgen05" (throughput kernel) or "tcgen05_wide" (latency kernel)."""
+        hidden layers -- the wide latency kernel when the envs do not fill the GPU --, CUDA cores otherwise; the
+        CUDA-core kernel of mbpo_actor_rollout_general for NoisyPendulumSystem / PointMassSystem), "cuda_cores",
+        "tcgen05" (throughput kernel) or "tcgen05_wide" (latency kernel); the tcgen05 kernels hold the pendulum only."""
         w = [t.to(torch.float32).contiguous() for t in params.weights]
         b = [t.to(torch.float32).contiguous() for t in params.biases]
         if len(w) < 2 or len(w) != len(b) or len(w) > 5:
@@ -148,15 +149,28 @@ def _rollout(env: VmappedSystemEnv, env_state: EnvState, policy: Policy, key: to
     policy.struct.draw_offset = int(env_offset) if total_envs is not None else 0
     raw = torch.empty((T, E, A), dtype=torch.float32, device=dev) if policy.emit_extras else None
     logp = torch.empty((T, E), dtype=torch.float32, device=dev) if policy.emit_extras else None
+    system_params = env_state.system_params
     with _lib.cuda_guard(obs):
-        _lib.check(_lib.lib.mbpo_actor_rollout_extras(
-            system.system_kind, _lib.C.addressof(params), config.math_mode_id, config.prng_mode,
-            _lib.C.byref(policy.struct), int(policy.deterministic), key_convention, _lib.ptr(key), env.episode_length,
-            env.action_repeat, _lib.ptr(obs), _lib.ptr(steps), _lib.ptr(done), _lib.ptr(first), E, T, _lib.ptr(act),
-            _lib.ptr(r), _lib.ptr(d), _lib.ptr(buf[1:]), _lib.ptr(tr), _lib.ptr(key_out), _lib.ptr(raw), _lib.ptr(logp),
-            _lib.stream_ptr(dev)))
+        if is_general(system):
+            sys_keys = system_keys(system, system_params, E)
+            sys_keys_out = torch.empty_like(sys_keys) if sys_keys is not None else None
+            _lib.check(_lib.lib.mbpo_actor_rollout_general(
+                system.system_kind, _lib.C.byref(params), config.prng_mode, _lib.C.byref(policy.struct),
+                int(policy.deterministic), key_convention, _lib.ptr(key), env.episode_length, env.action_repeat,
+                _lib.ptr(obs), _lib.ptr(steps), _lib.ptr(done), _lib.ptr(sys_keys), _lib.ptr(sys_keys_out),
+                _lib.ptr(first), E, T, _lib.ptr(act), _lib.ptr(r), _lib.ptr(d), _lib.ptr(buf[1:]), _lib.ptr(tr),
+                _lib.ptr(key_out), _lib.ptr(raw), _lib.ptr(logp), _lib.stream_ptr(dev)))
+            if sys_keys_out is not None:
+                system_params = system_params.replace(key=sys_keys_out)
+        else:
+            _lib.check(_lib.lib.mbpo_actor_rollout_extras(
+                system.system_kind, _lib.C.addressof(params), config.math_mode_id, config.prng_mode,
+                _lib.C.byref(policy.struct), int(policy.deterministic), key_convention, _lib.ptr(key),
+                env.episode_length, env.action_repeat, _lib.ptr(obs), _lib.ptr(steps), _lib.ptr(done), _lib.ptr(first),
+                E, T, _lib.ptr(act), _lib.ptr(r), _lib.ptr(d), _lib.ptr(buf[1:]), _lib.ptr(tr), _lib.ptr(key_out),
+                _lib.ptr(raw), _lib.ptr(logp), _lib.stream_ptr(dev)))
     nstate = EnvState(obs=obs, reward=r[-1] if T else env_state.reward, done=done,
-                      system_params=env_state.system_params,
+                      system_params=system_params,
                       info=dict(steps=steps, truncation=tr[-1] if T else env_state.info["truncation"], first_obs=first))
     policy_extras = {"log_prob": logp, "raw_action": raw} if policy.emit_extras else {}
     extras = {"policy_extras": policy_extras, "state_extras": {f: tr for f in extra_fields}}
@@ -319,9 +333,12 @@ class GraphedRollout:
     def __init__(self, env: VmappedSystemEnv, env_state: EnvState, policy: Policy, key: torch.Tensor, num_env_steps: int,
                  key_convention: int = _lib.KEYS_SAC, extra_fields: Sequence[str] = ("truncation",)):
         dev = env_state.obs.device
+        params = env_state.system_params
+        keyed = is_general(env.system) and env.system.keyed     # the System's keys are replay state too
+        if keyed:
+            params = params.replace(key=system_keys(env.system, params, env_state.obs.shape[0]).clone())
         self._state = EnvState(obs=env_state.obs.clone(), reward=env_state.reward.clone(), done=env_state.done.clone(),
-                               system_params=env_state.system_params,
-                               info={k: v.clone() for k, v in env_state.info.items()})
+                               system_params=params, info={k: v.clone() for k, v in env_state.info.items()})
         self._key = key.reshape(2).clone()
         self._policy = policy                      # keeps the weight tensors (and the struct's pointers) alive
         side = torch.cuda.Stream(dev)
@@ -340,6 +357,8 @@ class GraphedRollout:
             self._state.done.copy_(nstate.done)
             self._state.info["steps"].copy_(nstate.info["steps"])
             self._key.copy_(key_out)
+            if keyed:
+                self._state.system_params.key.copy_(nstate.system_params.key)
         self._out = (key_out, nstate, tr)
 
     def __call__(self) -> Tuple[torch.Tensor, EnvState, Transition]:

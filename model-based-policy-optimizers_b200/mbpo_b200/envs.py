@@ -18,6 +18,25 @@ from .systems.base_systems import System, SystemParams, _Replaceable
 from .utils.optimizer_utils import Transition
 
 
+def is_general(system: System) -> bool:
+    """NoisyPendulumSystem / PointMassSystem: their collection runs mbpo_env_unroll_general /
+    mbpo_actor_rollout_general; the pendulum keeps its own tuned entry points."""
+    return getattr(system, "system_kind", None) in (_lib.SYSTEM_NOISY_PENDULUM, _lib.SYSTEM_POINT_MASS)
+
+
+def system_keys(system: System, system_params: SystemParams, E: int):
+    """The envs' system_params.key [E, 2] a keyed general System steps with (None for one that draws nothing)."""
+    if not getattr(system, "keyed", False):
+        return None
+    key = None if system_params is None else system_params.key
+    if key is None:
+        raise ValueError("%s draws from system_params.key: it must be set" % type(system).__name__)
+    key = key.reshape(-1, 2).contiguous()
+    if key.shape[0] != E:
+        raise ValueError("system_params.key holds %d keys for %d envs" % (key.shape[0], E))
+    return key
+
+
 @dataclass
 class EnvState(_Replaceable):
     """brax_utils/base.py:12-23 State, restricted to what the System path uses.  info holds
@@ -87,16 +106,15 @@ class VmappedSystemEnv:
         d = torch.empty((T, E), dtype=torch.float32, device=dev)
         tr = torch.empty((T, E), dtype=torch.float32, device=dev)
         params = self.system.pack_params(state.system_params)
+        keys_in = system_keys(self.system, state.system_params, E) if is_general(self.system) else None
+        keys_out = torch.empty_like(keys_in) if keys_in is not None else None
         if T == 0:
             obs, steps, done = obs_in.clone(), steps_in.clone(), done_in.clone()
         with _lib.cuda_guard(acts):
-            _lib.check(_lib.lib.mbpo_env_unroll(
-                self.system.system_kind, _lib.C.addressof(params), config.math_mode_id, X, A, self.episode_length,
-                self.action_repeat, _lib.ptr(obs_in), _lib.ptr(steps_in), _lib.ptr(done_in), _lib.ptr(obs),
-                _lib.ptr(steps), _lib.ptr(done), _lib.ptr(first), _lib.ptr(acts),
-                E, T, None, _lib.ptr(r), _lib.ptr(d), _lib.ptr(n), _lib.ptr(tr), _lib.stream_ptr(dev)))
+            self._launch(params, obs_in, steps_in, done_in, keys_in, obs, steps, done, keys_out, first, _lib.ptr(acts),
+                         E, T, _lib.ptr(r), _lib.ptr(d), _lib.ptr(n), _lib.ptr(tr), _lib.stream_ptr(dev))
         new_state = EnvState(obs=obs, reward=r[-1] if T else state.reward, done=done,
-                             system_params=state.system_params,
+                             system_params=self._params_after(state.system_params, keys_out),
                              info=dict(steps=steps, truncation=tr[-1] if T else state.info["truncation"],
                                        first_obs=first))
         transition = Transition(observation=o, action=acts, reward=r, discount=d, next_observation=n,
@@ -127,6 +145,9 @@ class VmappedSystemEnv:
         tr = torch.empty((T, E), dtype=torch.float32, device=dev)
         first = state.info["first_obs"].contiguous()
         cur = [state.obs.contiguous(), state.info["steps"].contiguous(), state.done.contiguous()]
+        keys = system_keys(self.system, state.system_params, E) if is_general(self.system) else None
+        if keys is not None:
+            cur.append(keys)
         nxt = [torch.empty_like(t) for t in cur]
         spare = [torch.empty_like(t) for t in cur]
         params = self.system.pack_params(state.system_params)
@@ -143,12 +164,10 @@ class VmappedSystemEnv:
         with _lib.cuda_guard(acts):
             for k, (t0, t1) in enumerate(bounds):
                 main.wait_event(ev_in[k])
-                _lib.check(_lib.lib.mbpo_env_unroll(
-                    self.system.system_kind, _lib.C.addressof(params), config.math_mode_id, X, A, self.episode_length,
-                    self.action_repeat, _lib.ptr(cur[0]), _lib.ptr(cur[1]), _lib.ptr(cur[2]), _lib.ptr(nxt[0]),
-                    _lib.ptr(nxt[1]), _lib.ptr(nxt[2]), _lib.ptr(first), acts[t0:t1].data_ptr(), E, t1 - t0, None,
-                    r[t0:t1].data_ptr(), d[t0:t1].data_ptr(), buf[1 + t0:1 + t1].data_ptr(), tr[t0:t1].data_ptr(),
-                    main.cuda_stream))
+                self._launch(params, cur[0], cur[1], cur[2], cur[3] if keys is not None else None, nxt[0], nxt[1],
+                             nxt[2], nxt[3] if keys is not None else None, first, acts[t0:t1].data_ptr(), E, t1 - t0,
+                             r[t0:t1].data_ptr(), d[t0:t1].data_ptr(), buf[1 + t0:1 + t1].data_ptr(),
+                             tr[t0:t1].data_ptr(), main.cuda_stream)
                 cur, nxt, spare = nxt, spare, cur
                 if reward_host is not None:
                     ev = torch.cuda.Event()
@@ -161,12 +180,35 @@ class VmappedSystemEnv:
         main.wait_stream(s_in)
         main.wait_stream(s_out)
         new_state = EnvState(obs=cur[0], reward=r[-1] if T else state.reward, done=cur[2],
-                             system_params=state.system_params,
+                             system_params=self._params_after(state.system_params,
+                                                              cur[3] if keys is not None else None),
                              info=dict(steps=cur[1], truncation=tr[-1] if T else state.info["truncation"],
                                        first_obs=first))
         transition = Transition(observation=buf[:T], action=acts, reward=r, discount=d, next_observation=buf[1:],
                                 extras={"state_extras": {"truncation": tr}})
         return new_state, transition
+
+    def _launch(self, params, obs_in, steps_in, done_in, keys_in, obs_out, steps_out, done_out, keys_out, first,
+                acts_ptr, E, T, r_ptr, d_ptr, n_ptr, tr_ptr, stream):
+        """One launch of T wrapped env steps (observation_out = NULL: observation[t] is next_observation[t-1])."""
+        X, A = self.system.x_dim, self.system.u_dim
+        if is_general(self.system):
+            _lib.check(_lib.lib.mbpo_env_unroll_general(
+                self.system.system_kind, _lib.C.byref(params), config.prng_mode, self.episode_length,
+                self.action_repeat, _lib.ptr(obs_in), _lib.ptr(steps_in), _lib.ptr(done_in), _lib.ptr(keys_in),
+                _lib.ptr(obs_out), _lib.ptr(steps_out), _lib.ptr(done_out), _lib.ptr(keys_out), _lib.ptr(first),
+                acts_ptr, E, T, None, r_ptr, d_ptr, n_ptr, tr_ptr, stream))
+            return
+        _lib.check(_lib.lib.mbpo_env_unroll(
+            self.system.system_kind, _lib.C.addressof(params), config.math_mode_id, X, A, self.episode_length,
+            self.action_repeat, _lib.ptr(obs_in), _lib.ptr(steps_in), _lib.ptr(done_in), _lib.ptr(obs_out),
+            _lib.ptr(steps_out), _lib.ptr(done_out), _lib.ptr(first), acts_ptr, E, T, None, r_ptr, d_ptr, n_ptr,
+            tr_ptr, stream))
+
+    @staticmethod
+    def _params_after(system_params: SystemParams, keys_out):
+        """system_params after the unroll: a keyed System carries its advanced keys on."""
+        return system_params if keys_out is None else system_params.replace(key=keys_out)
 
     def step(self, state: EnvState, action: torch.Tensor) -> EnvState:
         """One wrapped env step: action [E, A]."""
