@@ -1,7 +1,7 @@
 """Builds libmbpo_b200.so (sm_100a) in-tree with nvcc.
 
 One translation unit per compiled horizon (csrc/plan_inst.cu with -DMBPO_INST_H=<h>) plus the
-C-ABI units (csrc/mbpo_b200.cu, csrc/replay.cu, csrc/general_collection.cu) and the any-horizon plan (csrc/plan_rt.cu); units compile in parallel and are skipped when up to date.
+C-ABI units (csrc/mbpo_b200.cu, csrc/replay.cu, csrc/collection.cu) and the any-horizon plan (csrc/plan_rt.cu); units compile in parallel and are skipped when up to date.
 Usage:  python model-based-policy-optimizers_b200/build.py [--force]
 """
 from __future__ import annotations
@@ -51,7 +51,7 @@ def build(force: bool = False, verbose: bool = True) -> str:
     os.makedirs(OBJ_DIR, exist_ok=True)
     jobs = [(os.path.join(CSRC, "mbpo_b200.cu"), os.path.join(OBJ_DIR, "mbpo_b200.o"), []),
             (os.path.join(CSRC, "replay.cu"), os.path.join(OBJ_DIR, "replay.o"), []),
-            (os.path.join(CSRC, "general_collection.cu"), os.path.join(OBJ_DIR, "general_collection.o"), []),
+            (os.path.join(CSRC, "collection.cu"), os.path.join(OBJ_DIR, "collection.o"), []),
             (os.path.join(CSRC, "plan_rt.cu"), os.path.join(OBJ_DIR, "plan_rt.o"), [])]
     for h in HORIZONS:
         jobs.append((os.path.join(CSRC, "plan_inst.cu"), os.path.join(OBJ_DIR, "plan_h%d.o" % h),

@@ -25,6 +25,7 @@
 // CTAs are sized so that the envs spread evenly over the SMs in a single wave (one CTA per SM).
 #pragma once
 #include "env_kernels.cuh"
+#include "host_util.h"
 #include "mathx.cuh"
 #include "threefry.cuh"
 
@@ -64,6 +65,40 @@ struct ActorArgs {
   float* raw_action_out;        // [T,E] or NULL: PPO's policy_extras['raw_action'] (pre-tanh sample)
   float* log_prob_out;          // [T,E] or NULL: PPO's policy_extras['log_prob']
 };
+
+// Host side of both actor entry points (mbpo_actor_rollout_extras, mbpo_actor_rollout_general): checks the policy
+// against E envs of a System with X state and A action dims, and fills the fields ActorArgs and GeneralActorArgs
+// share.  `what` prefixes the messages.
+template <class Args>
+int fill_policy(const char* what, const MbpoPolicyParams* p, int E, int X, int A, Args& a) {
+  if (p->hidden != ACT_W || p->obs_dim != X || p->action_dim != A || p->num_hidden < 1 || p->num_hidden > ACT_MAX_HIDDEN)
+    return fail(MBPO_EUNSUPPORTED,
+                "%s: the policy kernel needs obs_dim == %d, action_dim == %d, 1..%d hidden layers of width %d "
+                "(got obs %d, act %d, %d x %d)",
+                what, X, A, ACT_MAX_HIDDEN, ACT_W, p->obs_dim, p->action_dim, p->num_hidden, p->hidden);
+  for (int l = 0; l <= p->num_hidden; ++l)
+    MBPO_REQUIRE(p->w[l] && p->b[l], "%s: null policy weights (layer %d)", what, l);
+  MBPO_REQUIRE((p->obs_mean_dev == nullptr) == (p->obs_std_dev == nullptr),
+               "%s: obs_mean_dev and obs_std_dev come together", what);
+  MBPO_REQUIRE(p->draw_total == 0 || (p->draw_offset >= 0 && p->draw_offset + E <= p->draw_total),
+               "%s: envs [%d, %d) are not inside draw_total %d", what, p->draw_offset, p->draw_offset + E,
+               p->draw_total);
+  a.num_hidden = p->num_hidden;
+  a.min_std = p->min_std;
+  a.normalize = p->normalize;
+  a.draw_total = p->draw_total > 0 ? p->draw_total : E;
+  a.draw_offset = p->draw_total > 0 ? p->draw_offset : 0;
+  for (size_t i = 0; i < sizeof(a.obs_mean) / sizeof(a.obs_mean[0]); ++i) {
+    a.obs_mean[i] = p->obs_mean[i];
+    a.obs_std[i] = p->obs_std[i];
+  }
+  a.obs_mean_dev = p->obs_mean_dev; a.obs_std_dev = p->obs_std_dev;
+  for (int l = 0; l <= ACT_MAX_HIDDEN; ++l) {
+    a.w[l] = l <= a.num_hidden ? p->w[l] : nullptr;
+    a.b[l] = l <= a.num_hidden ? p->b[l] : nullptr;
+  }
+  return MBPO_OK;
+}
 
 // jax.nn.swish(x) = x * sigmoid(x), sigmoid = 1 / (1 + exp(-x)).  ex2.approx (2^-22 relative) and rcp.approx
 // (1 ulp) keep the activation within ~5e-7 relative of the float32 reference at 5 instructions; the accurate

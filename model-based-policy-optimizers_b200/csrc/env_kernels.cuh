@@ -72,7 +72,7 @@ __device__ __forceinline__ void warp_store3(float* tile, float* dst, int lane, i
 // as brax's are.
 //
 // OBS: also write the separate observation buffer.  All of next_obs / reward / discount /
-// truncation are non-NULL (the C ABI falls back to the checked kernel otherwise).
+// truncation are non-NULL (otherwise the C ABI runs env_unroll_general_kernel, general_env_kernels.cuh).
 //
 // FAST (host-checked: action_repeat == 1, |target_angle| <= 6, E % 4 == 0, 16-byte aligned
 // observation buffers, T*E*3 < 2^31): warps whose 32 envs are all live and share their piece
@@ -253,62 +253,6 @@ __global__ void __launch_bounds__(ENV_THREADS, 18) env_rollout_pendulum_kernel(c
     }
   }
   if (live && t_beg < t_end && t_end == a.T) {  // the piece holding the last step owns the final state
-    a.obs[3 * e] = c; a.obs[3 * e + 1] = s; a.obs[3 * e + 2] = w;
-    a.steps[e] = steps;
-    a.done[e] = done;
-  }
-}
-
-// Fully checked variant: any output pointer may be NULL.
-template <int MATH>
-__global__ void __launch_bounds__(ENV_THREADS) env_rollout_pendulum_checked_kernel(const __grid_constant__ EnvArgs a) {
-  __shared__ float tiles[ENV_THREADS / 32][96];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int e = blockIdx.x * ENV_THREADS + threadIdx.x;
-  const int warp_e0 = e - lane;
-  if (warp_e0 >= a.E) return;
-  const bool live = e < a.E;
-  const int n_valid = ((a.E - warp_e0) < 32 ? (a.E - warp_e0) : 32) * 3;
-  const int ee = live ? e : a.E - 1;
-  const PendulumConsts pc(a.sys);
-  float* tile = tiles[warp];
-  float c = a.obs_in[3 * ee], s = a.obs_in[3 * ee + 1], w = a.obs_in[3 * ee + 2];
-  const float f_c = a.first_obs[3 * ee], f_s = a.first_obs[3 * ee + 1], f_w = a.first_obs[3 * ee + 2];
-  float steps = a.steps_in[ee], done = a.done_in[ee];
-  const float ep_len = static_cast<float>(a.episode_length);
-  const float rep = static_cast<float>(a.action_repeat);
-  for (int t = 0; t < a.T; ++t) {
-    const size_t row = static_cast<size_t>(t) * a.E;
-    const float u = __ldg(a.actions + row + ee);
-    steps = (done != 0.0f) ? 0.0f : steps;
-    done = 0.0f;
-    if (a.observation_out) warp_store3(tile, a.observation_out + (row + warp_e0) * 3 + lane, lane, n_valid, c, s, w);
-    float rew = 0.0f;
-    for (int r = 0; r < a.action_repeat; ++r) {
-      float rr;
-      if (MATH == MBPO_MATH_REFERENCE) {
-        pendulum_step_ref(pc, c, s, w, u, rr);
-      } else {
-        float th = atan2_bounded(s, c);
-        pendulum_step_theta(pc, th, w, u, rr);
-        sincos_bounded(th, s, c);
-      }
-      rew = __fadd_rn(rew, rr);
-    }
-    steps = __fadd_rn(steps, rep);
-    const bool over = steps >= ep_len;
-    const float trunc = over ? (1.0f - done) : 0.0f;
-    done = over ? 1.0f : done;
-    if (over) { c = f_c; s = f_s; w = f_w; }
-    if (a.next_observation_out)
-      warp_store3(tile, a.next_observation_out + (row + warp_e0) * 3 + lane, lane, n_valid, c, s, w);
-    if (live) {
-      if (a.reward_out) a.reward_out[row + e] = rew;
-      if (a.discount_out) a.discount_out[row + e] = 1.0f - done;
-      if (a.truncation_out) a.truncation_out[row + e] = trunc;
-    }
-  }
-  if (live) {
     a.obs[3 * e] = c; a.obs[3 * e + 1] = s; a.obs[3 * e + 2] = w;
     a.steps[e] = steps;
     a.done[e] = done;

@@ -10,7 +10,8 @@
 //             element (draw_offset + e) * A + a (the legacy layout pads draw_total * A to even inside random_bits_at).
 //   extras    PPO's log_prob sums over the A action dims; raw_action is [T,E,A].
 // One thread per env, state and keys in registers.  The observation rows leave through the warp transposes of
-// env_kernels.cuh (X = 3) or as one 16-byte store per env (X = 4).
+// env_kernels.cuh (X = 3) or as one 16-byte store per env (X = 4).  env_unroll_general_kernel also serves the
+// pendulum's env rollouts whose Transition buffers are not all present (collection.cu launch_env).
 #pragma once
 #include "actor_kernels.cuh"
 #include "systems.cuh"

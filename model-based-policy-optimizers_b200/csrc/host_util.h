@@ -3,7 +3,9 @@
 #include <cuda_runtime.h>
 
 #include <cstdarg>
+#include <cstdint>
 #include <cstdio>
+#include <type_traits>
 
 #include "../../include/mbpo_b200.h"
 
@@ -31,6 +33,32 @@ inline int check_launch(const char* what) {
   } while (0)
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+inline int copy_async(void* dst, const void* src, size_t bytes, cudaStream_t st, const char* what) {
+  if (bytes == 0 || dst == src) return MBPO_OK;
+  const cudaError_t ce = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st);
+  return ce == cudaSuccess ? MBPO_OK : fail(MBPO_ECUDA, "%s copy: %s", what, cudaGetErrorString(ce));
+}
+
+// Runtime mode -> template argument: f(std::integral_constant<int, MODE>) for a prng_mode (MBPO_PRNG_*) or
+// math_mode (MBPO_MATH_*) the caller has already checked to be 0 or 1, so that f can name kernel<MODE>.  Each
+// call site instantiates only the modes it dispatches on.
+template <class F>
+int with_prng(int prng_mode, F&& f) {
+  if (prng_mode == 0) return f(std::integral_constant<int, 0>{});
+  return f(std::integral_constant<int, 1>{});
+}
+template <class F>
+int with_math(int math_mode, F&& f) {
+  if (math_mode == 0) return f(std::integral_constant<int, 0>{});
+  return f(std::integral_constant<int, 1>{});
+}
+template <class F>
+int with_prng_math(int prng_mode, int math_mode, F&& f) {
+  return with_prng(prng_mode, [&](auto p) { return with_math(math_mode, [&](auto m) { return f(p, m); }); });
+}
 
 inline int device_sm_count() {
   int dev = 0, sms = 0;

@@ -13,7 +13,6 @@
 #include <tuple>
 
 #include "../../include/mbpo_b200.h"
-#include "env_kernels.cuh"
 #include "host_util.h"
 #include "mlp_tc_kernels.cuh"
 #include "actor_kernels.cuh"
@@ -84,11 +83,10 @@ int prng_draw(const uint32_t* keys, int M, int n, int prng_mode, int what, float
   MBPO_REQUIRE(keys && out, "prng: null pointer");
   const int threads = 256;
   const unsigned blocks = static_cast<unsigned>((total + threads - 1) / threads);
-  if (prng_mode == 0)
-    prng_draw_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, what, lo, hi, out);
-  else
-    prng_draw_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, what, lo, hi, out);
-  return check_launch("prng_draw_kernel");
+  return with_prng(prng_mode, [&](auto P) {
+    prng_draw_kernel<P><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, what, lo, hi, out);
+    return check_launch("prng_draw_kernel");
+  });
 }
 
 int validate_cfg(const MbpoIcemCfg* c) {
@@ -125,16 +123,14 @@ int launch_noise_rolled(const MbpoIcemCfg* cfg, const ScaleTable& tbl, const uin
   const int threads = STAGED_THREADS;
   const size_t smem = static_cast<size_t>(threads) * (cfg->horizon | 1) * sizeof(float);
   const unsigned blocks = static_cast<unsigned>((M + threads - 1) / threads);
-  auto k0 = powerlaw_noise_rt_kernel<0>;
-  auto k1 = powerlaw_noise_rt_kernel<1>;
-  const cudaError_t e = cudaFuncSetAttribute(cfg->prng_mode == 0 ? k0 : k1,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-  if (e != cudaSuccess) return fail(MBPO_ECUDA, "powerlaw_noise smem attr: %s", cudaGetErrorString(e));
-  if (cfg->prng_mode == 0)
-    k0<<<blocks, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, keys, M, noise_out, bits_out);
-  else
-    k1<<<blocks, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, keys, M, noise_out, bits_out);
-  return check_launch("powerlaw_noise_rt_kernel");
+  return with_prng(cfg->prng_mode, [&](auto P) {
+    auto kernel = powerlaw_noise_rt_kernel<P>;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               static_cast<int>(smem));
+    if (e != cudaSuccess) return fail(MBPO_ECUDA, "powerlaw_noise smem attr: %s", cudaGetErrorString(e));
+    kernel<<<blocks, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, keys, M, noise_out, bits_out);
+    return check_launch("powerlaw_noise_rt_kernel");
+  });
 }
 
 // ---- fused plan --------------------------------------------------------------------------
@@ -154,12 +150,21 @@ void fill_plan_args(PlanArgs& a, const MbpoIcemCfg* c, const MbpoPendulumParams*
   if (trace) a.trace = *trace;
 }
 
-bool general_system_kind(int k) { return k == MBPO_SYSTEM_NOISY_PENDULUM || k == MBPO_SYSTEM_POINT_MASS; }
+// The general Systems whose plans run the general kernels (icem_plan_general_kernel, general_objective_kernel); the
+// pendulum, a general System too, keeps its tuned plan kernels.
+bool general_plan_kind(int kind, int* X, int* A) {
+  bool keyed;
+  return kind != MBPO_SYSTEM_PENDULUM && general_system_dims(kind, X, A, &keyed) == MBPO_OK;
+}
+bool general_plan_kind(int kind) {
+  int X, A;
+  return general_plan_kind(kind, &X, &A);
+}
 
 int plan_fusable(const MbpoIcemCfg* c, bool set_error) {
   const char* why = nullptr;
-  if (general_system_kind(c->system_kind)) {
-    const int A = c->system_kind == MBPO_SYSTEM_POINT_MASS ? 2 : 1, X = c->system_kind == MBPO_SYSTEM_POINT_MASS ? 4 : 3;
+  int X, A;
+  if (general_plan_kind(c->system_kind, &X, &A)) {
     const size_t RS = static_cast<size_t>(c->horizon * A) | 1;
     const size_t words = static_cast<size_t>(c->num_samples + 1) * RS + (c->num_samples + c->num_prev_elites) +
                          3 * c->horizon * A + 2 * c->num_elites +
@@ -226,7 +231,7 @@ int run_plan(const MbpoIcemCfg* c, const void* sys_params_host, const float* x0,
   if (B == 0) return MBPO_OK;
   MBPO_REQUIRE(sys_params_host && x0 && key_in && best_seq_in && best_seq_out && key_out, "plan: null pointer");
   MBPO_REQUIRE(mpc != nullptr || best_value_out != nullptr, "plan: best_value_out is null");
-  if (general_system_kind(c->system_kind)) {
+  if (general_plan_kind(c->system_kind)) {
     if (mpc != nullptr)
       return fail(MBPO_EUNSUPPORTED, "closed loop in one launch exists for the pendulum System only");
     PlanArgs g;
@@ -379,9 +384,10 @@ int mbpo_prng_split(const uint32_t* keys, int M, int num, int prng_mode, uint32_
   MBPO_REQUIRE(keys && keys_out, "prng_split: null pointer");
   const int threads = 256;
   const unsigned blocks = static_cast<unsigned>((total + threads - 1) / threads);
-  if (prng_mode == 0) prng_split_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, num, keys_out);
-  else prng_split_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, num, keys_out);
-  return check_launch("prng_split_kernel");
+  return with_prng(prng_mode, [&](auto P) {
+    prng_split_kernel<P><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, num, keys_out);
+    return check_launch("prng_split_kernel");
+  });
 }
 
 int mbpo_prng_random_bits(const uint32_t* keys, int M, int n, int prng_mode, uint32_t* bits_out, void* stream) {
@@ -444,18 +450,16 @@ int mbpo_icem_sample_actions(const MbpoIcemCfg* cfg, const uint32_t* carry_key, 
     const size_t smem = static_cast<size_t>(threads) * (cfg->horizon | 1) * sizeof(float);
     const int N = cfg->num_samples, Np = cfg->num_prev_elites, A = cfg->action_dim;
     const dim3 grid(static_cast<unsigned>(((N + Np) * A + threads - 1) / threads), static_cast<unsigned>(B));
-    auto k0 = sample_actions_rt_kernel<0>;
-    auto k1 = sample_actions_rt_kernel<1>;
-    const cudaError_t e = cudaFuncSetAttribute(cfg->prng_mode == 0 ? k0 : k1,
-                                               cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-    if (e != cudaSuccess) return fail(MBPO_ECUDA, "sample_actions smem attr: %s", cudaGetErrorString(e));
-    if (cfg->prng_mode == 0)
-      k0<<<grid, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, carry_key, mean, std_, N, Np, A, cfg->u_min,
-                                                     cfg->u_max, actions_out, next_key_out, particle_keys_out);
-    else
-      k1<<<grid, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, carry_key, mean, std_, N, Np, A, cfg->u_min,
-                                                     cfg->u_max, actions_out, next_key_out, particle_keys_out);
-    return check_launch("sample_actions_rt_kernel");
+    return with_prng(cfg->prng_mode, [&](auto P) {
+      auto kernel = sample_actions_rt_kernel<P>;
+      const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 static_cast<int>(smem));
+      if (e != cudaSuccess) return fail(MBPO_ECUDA, "sample_actions smem attr: %s", cudaGetErrorString(e));
+      kernel<<<grid, threads, smem, as_stream(stream)>>>(tbl, tw, cfg->horizon, carry_key, mean, std_, N, Np, A,
+                                                         cfg->u_min, cfg->u_max, actions_out, next_key_out,
+                                                         particle_keys_out);
+      return check_launch("sample_actions_rt_kernel");
+    });
   }
   switch (cfg->horizon) {
 #define X(h)                                                                                                    \
@@ -483,11 +487,10 @@ int mbpo_system_step(int system_kind, const void* sys_params_host, int math_mode
   const MbpoPendulumParams sys = *static_cast<const MbpoPendulumParams*>(sys_params_host);
   const int threads = 128;
   const unsigned blocks = static_cast<unsigned>((R + threads - 1) / threads);
-  if (math_mode == 0)
-    system_step_pendulum_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(sys, x, u, R, x_next, reward);
-  else
-    system_step_pendulum_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(sys, x, u, R, x_next, reward);
-  return check_launch("system_step_pendulum_kernel");
+  return with_math(math_mode, [&](auto M) {
+    system_step_pendulum_kernel<M><<<blocks, threads, 0, as_stream(stream)>>>(sys, x, u, R, x_next, reward);
+    return check_launch("system_step_pendulum_kernel");
+  });
 }
 
 int mbpo_rollout_actions(int system_kind, const void* sys_params_host, int math_mode, int horizon, int action_dim,
@@ -516,65 +519,39 @@ int mbpo_rollout_actions(int system_kind, const void* sys_params_host, int math_
   if (smem > 227 * 1024) return fail(MBPO_EUNSUPPORTED, "rollout_actions: horizon %d too long to stage", horizon);
   const long long warps = (total + 31) / 32;
   const unsigned blocks = static_cast<unsigned>((warps + threads / 32 - 1) / (threads / 32));
-  cudaError_t e;
-  if (math_mode == 0) {
-    e = cudaFuncSetAttribute(rollout_actions_pendulum_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             static_cast<int>(smem));
+  return with_math(math_mode, [&](auto MATH) {
+    auto kernel = rollout_actions_pendulum_kernel<MATH>;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               static_cast<int>(smem));
     if (e != cudaSuccess) return fail(MBPO_ECUDA, "rollout_actions smem attr: %s", cudaGetErrorString(e));
-    rollout_actions_pendulum_kernel<0><<<blocks, threads, smem, as_stream(stream)>>>(
-        sys, horizon, x0, actions, B, M, returns_out, obs_out, reward_out, next_obs_out);
-  } else {
-    e = cudaFuncSetAttribute(rollout_actions_pendulum_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             static_cast<int>(smem));
-    if (e != cudaSuccess) return fail(MBPO_ECUDA, "rollout_actions smem attr: %s", cudaGetErrorString(e));
-    rollout_actions_pendulum_kernel<1><<<blocks, threads, smem, as_stream(stream)>>>(
-        sys, horizon, x0, actions, B, M, returns_out, obs_out, reward_out, next_obs_out);
-  }
-  return check_launch("rollout_actions_pendulum_kernel");
+    kernel<<<blocks, threads, smem, as_stream(stream)>>>(sys, horizon, x0, actions, B, M, returns_out, obs_out,
+                                                         reward_out, next_obs_out);
+    return check_launch("rollout_actions_pendulum_kernel");
+  });
 }
 
 // ---- general Systems (any action_dim, key-consuming) ---------------------------------------------
-extern "C++" {
-namespace {
-bool general_kind(int k) {
-  return k == MBPO_SYSTEM_PENDULUM || k == MBPO_SYSTEM_NOISY_PENDULUM || k == MBPO_SYSTEM_POINT_MASS;
-}
-int general_dims(int kind, int* X, int* A, bool* keyed) {
-  switch (kind) {
-    case MBPO_SYSTEM_PENDULUM: *X = 3; *A = 1; *keyed = false; return MBPO_OK;
-    case MBPO_SYSTEM_NOISY_PENDULUM: *X = 3; *A = 1; *keyed = true; return MBPO_OK;
-    case MBPO_SYSTEM_POINT_MASS: *X = 4; *A = 2; *keyed = false; return MBPO_OK;
-    default: return mbpo::fail(MBPO_EUNSUPPORTED, "system_kind %d is not one of the general Systems", kind);
-  }
-}
-}  // namespace
-}  // extern "C++"
-
 int mbpo_system_step_general(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode,
                              const float* x, const float* u, const uint32_t* keys_in, int R, float* x_next,
                              float* reward, uint32_t* keys_out, void* stream) {
   int X, A; bool keyed;
-  const int rc = general_dims(system_kind, &X, &A, &keyed);
-  if (rc != MBPO_OK) return rc;
+  if (general_system_dims(system_kind, &X, &A, &keyed) != MBPO_OK)
+    return fail(MBPO_EUNSUPPORTED, "system_step_general: system_kind %d is not one of the general Systems",
+                system_kind);
   MBPO_REQUIRE(prng_mode == 0 || prng_mode == 1, "system_step_general: bad prng_mode %d", prng_mode);
   MBPO_REQUIRE(R >= 0, "system_step_general: R < 0");
   if (R == 0) return MBPO_OK;
   MBPO_REQUIRE(params_host && x && u && x_next && reward, "system_step_general: null pointer");
   MBPO_REQUIRE(!keyed || keys_in, "system_step_general: this System draws from system_params.key: keys_in is null");
   const unsigned blocks = static_cast<unsigned>((R + 127) / 128);
-  cudaStream_t st = as_stream(stream);
-#define MBPO_LAUNCH_STEP(SYS)                                                                                     \
-  do {                                                                                                            \
-    if (prng_mode == 0) system_step_general_kernel<SYS, 0><<<blocks, 128, 0, st>>>(*params_host, x, u, keys_in, R, \
-                                                                                   x_next, reward, keys_out);     \
-    else system_step_general_kernel<SYS, 1><<<blocks, 128, 0, st>>>(*params_host, x, u, keys_in, R, x_next,       \
-                                                                    reward, keys_out);                            \
-  } while (0)
-  if (system_kind == MBPO_SYSTEM_PENDULUM) MBPO_LAUNCH_STEP(PendulumSys);
-  else if (system_kind == MBPO_SYSTEM_NOISY_PENDULUM) MBPO_LAUNCH_STEP(NoisyPendulumSys);
-  else MBPO_LAUNCH_STEP(PointMassSys);
-#undef MBPO_LAUNCH_STEP
-  return check_launch("system_step_general_kernel");
+  return with_system<PendulumSys, NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    using Sys = typename decltype(t)::type;
+    return with_prng(prng_mode, [&](auto P) {
+      system_step_general_kernel<Sys, P><<<blocks, 128, 0, as_stream(stream)>>>(*params_host, x, u, keys_in, R,
+                                                                                 x_next, reward, keys_out);
+      return check_launch("system_step_general_kernel");
+    });
+  });
 }
 
 int mbpo_system_objective(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode, int horizon,
@@ -582,8 +559,8 @@ int mbpo_system_objective(int system_kind, const MbpoGeneralSystemParams* params
                           int num_particles, int summarize, float* values_out, float* obs_out, float* reward_out,
                           float* next_obs_out, void* stream) {
   int X, A; bool keyed;
-  const int rc = general_dims(system_kind, &X, &A, &keyed);
-  if (rc != MBPO_OK) return rc;
+  if (general_system_dims(system_kind, &X, &A, &keyed) != MBPO_OK)
+    return fail(MBPO_EUNSUPPORTED, "system_objective: system_kind %d is not one of the general Systems", system_kind);
   MBPO_REQUIRE(prng_mode == 0 || prng_mode == 1, "system_objective: bad prng_mode %d", prng_mode);
   MBPO_REQUIRE(horizon >= 1 && B >= 0 && M >= 0 && num_particles >= 0, "system_objective: bad sizes");
   MBPO_REQUIRE(summarize == 0 || summarize == 1, "system_objective: bad summarize %d", summarize);
@@ -595,23 +572,15 @@ int mbpo_system_objective(int system_kind, const MbpoGeneralSystemParams* params
   MBPO_REQUIRE(num_particles == 0 || !(obs_out || reward_out || next_obs_out),
                "system_objective: Transition buffers exist for single rollouts (num_particles == 0) only");
   const unsigned blocks = static_cast<unsigned>((total + 127) / 128);
-  cudaStream_t st = as_stream(stream);
-#define MBPO_LAUNCH_OBJ(SYS)                                                                                        \
-  do {                                                                                                              \
-    if (prng_mode == 0)                                                                                             \
-      general_objective_kernel<SYS, 0><<<blocks, 128, 0, st>>>(*params_host, horizon, x0, actions, keys, B, M,     \
-                                                               num_particles, summarize, values_out, obs_out,       \
-                                                               reward_out, next_obs_out);                           \
-    else                                                                                                            \
-      general_objective_kernel<SYS, 1><<<blocks, 128, 0, st>>>(*params_host, horizon, x0, actions, keys, B, M,     \
-                                                               num_particles, summarize, values_out, obs_out,       \
-                                                               reward_out, next_obs_out);                           \
-  } while (0)
-  if (system_kind == MBPO_SYSTEM_PENDULUM) MBPO_LAUNCH_OBJ(PendulumSys);
-  else if (system_kind == MBPO_SYSTEM_NOISY_PENDULUM) MBPO_LAUNCH_OBJ(NoisyPendulumSys);
-  else MBPO_LAUNCH_OBJ(PointMassSys);
-#undef MBPO_LAUNCH_OBJ
-  return check_launch("general_objective_kernel");
+  return with_system<PendulumSys, NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    using Sys = typename decltype(t)::type;
+    return with_prng(prng_mode, [&](auto P) {
+      general_objective_kernel<Sys, P><<<blocks, 128, 0, as_stream(stream)>>>(
+          *params_host, horizon, x0, actions, keys, B, M, num_particles, summarize, values_out, obs_out, reward_out,
+          next_obs_out);
+      return check_launch("general_objective_kernel");
+    });
+  });
 }
 
 // ---- stage 3 -----------------------------------------------------------------------------------
@@ -666,7 +635,7 @@ int mbpo_icem_plan_clustered(const MbpoIcemCfg* cfg, const void* sys_params_host
 
 int mbpo_icem_plan_cluster_size(const MbpoIcemCfg* cfg, int B) {
   if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || !horizon_supported(cfg->horizon) ||
-      general_system_kind(cfg->system_kind) || cfg->num_samples + cfg->num_prev_elites < 36)
+      general_plan_kind(cfg->system_kind) || cfg->num_samples + cfg->num_prev_elites < 36)
     return 0;
   const ClusterCaps caps = cluster_caps(cfg, false);
   return plan_cluster_choice(B, cfg->num_samples, caps.cap);
@@ -674,7 +643,7 @@ int mbpo_icem_plan_cluster_size(const MbpoIcemCfg* cfg, int B) {
 
 int mbpo_icem_plan_cluster_capacity(const MbpoIcemCfg* cfg, int cluster_size) {
   if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || !horizon_supported(cfg->horizon) ||
-      general_system_kind(cfg->system_kind))
+      general_plan_kind(cfg->system_kind))
     return 0;
   const ClusterCaps caps = cluster_caps(cfg, false);
   switch (cluster_size) {
@@ -706,12 +675,11 @@ int mbpo_icem_plan_staged(const MbpoIcemCfg* cfg, const void* sys_params_host, c
   if (rc != MBPO_OK) return rc;
   MBPO_REQUIRE(sys_params_host, "plan_staged: null pointer");
   MBPO_REQUIRE(B >= 0 && B <= 65535, "plan_staged: B %d outside [0, 65535]", B);
-  const bool general = cfg->system_kind == MBPO_SYSTEM_NOISY_PENDULUM || cfg->system_kind == MBPO_SYSTEM_POINT_MASS;
+  int X, A;
+  const bool general = general_plan_kind(cfg->system_kind, &X, &A);
   if (cfg->system_kind != MBPO_SYSTEM_PENDULUM && cfg->system_kind != MBPO_SYSTEM_MLP_ENSEMBLE && !general)
     return fail(MBPO_EUNSUPPORTED, "plan_staged: unknown system_kind %d", cfg->system_kind);
   if (general) {
-    int X, A; bool keyed;
-    general_dims(cfg->system_kind, &X, &A, &keyed);
     MBPO_REQUIRE(cfg->action_dim == A && cfg->x_dim == X, "plan_staged: system_kind %d has x_dim %d, action_dim %d "
                  "(cfg says %d, %d)", cfg->system_kind, X, A, cfg->x_dim, cfg->action_dim);
   }
@@ -749,15 +717,12 @@ int mbpo_icem_plan_staged(const MbpoIcemCfg* cfg, const void* sys_params_host, c
 
   // ping-pong so that after S iterations the results land in slot 0 (= the caller's buffers)
   int cur = (cfg->num_steps % 2 == 0) ? 0 : 1;
-  if (cfg->prng_mode == 0)
-    plan_prologue_kernel<0><<<B, 64, 0, st>>>(B, static_cast<int>(D), cfg->action_dim, cfg->warm_start, cfg->init_std,
+  rc = with_prng(cfg->prng_mode, [&](auto P) {
+    plan_prologue_kernel<P><<<B, 64, 0, st>>>(B, static_cast<int>(D), cfg->action_dim, cfg->warm_start, cfg->init_std,
                                               key_in, best_seq_in, ckey[cur], key_out, mean[cur], std_[cur], bseq[cur],
                                               bval[cur]);
-  else
-    plan_prologue_kernel<1><<<B, 64, 0, st>>>(B, static_cast<int>(D), cfg->action_dim, cfg->warm_start, cfg->init_std,
-                                              key_in, best_seq_in, ckey[cur], key_out, mean[cur], std_[cur], bseq[cur],
-                                              bval[cur]);
-  rc = check_launch("plan_prologue_kernel");
+    return check_launch("plan_prologue_kernel");
+  });
   if (rc != MBPO_OK) return rc;
   for (int it = 0; it < cfg->num_steps; ++it) {
     const int nxt = cur ^ 1;
@@ -845,86 +810,6 @@ int mbpo_icem_mpc_closed_loop_clustered(const MbpoIcemCfg* cfg, const void* sys_
   m.actions_out = actions_out;
   return run_plan(cfg, sys_params_host, x0, key_in, best_seq_in, B, best_seq_out, nullptr, key_out, nullptr, &m,
                   cluster_size, stream);
-}
-
-// ---- env rollouts ----------------------------------------------------------------------------------
-extern "C++" {
-namespace {
-int launch_env(int system_kind, const void* sys_params_host, int math_mode, int x_dim, int action_dim,
-               int episode_length, int action_repeat, const float* obs_in, const float* steps_in,
-               const float* done_in, float* obs, float* steps, float* done, const float* first_obs,
-               const float* actions, int E, int T, float* observation_out, float* reward_out, float* discount_out,
-               float* next_observation_out, float* truncation_out, bool segmented, void* stream) {
-  using namespace mbpo;
-  if (system_kind != MBPO_SYSTEM_PENDULUM)
-    return fail(MBPO_EUNSUPPORTED, "env_rollout: only MBPO_SYSTEM_PENDULUM has an inlined step");
-  MBPO_REQUIRE(action_dim == 1 && x_dim == 3, "env_rollout: pendulum needs action_dim == 1, x_dim == 3");
-  MBPO_REQUIRE(math_mode == 0 || math_mode == 1, "env_rollout: bad math_mode %d", math_mode);
-  MBPO_REQUIRE(episode_length >= 1 && action_repeat >= 1, "env_rollout: episode_length/action_repeat < 1");
-  MBPO_REQUIRE(E >= 0 && T >= 0, "env_rollout: negative size");
-  if (E == 0 || T == 0) return MBPO_OK;     // empty arrays have no address
-  MBPO_REQUIRE(sys_params_host && obs_in && steps_in && done_in && obs && steps && done && first_obs && actions,
-               "env_rollout: null pointer");
-  EnvArgs a;
-  a.sys = *static_cast<const MbpoPendulumParams*>(sys_params_host);
-  a.E = E; a.T = T; a.episode_length = episode_length; a.action_repeat = action_repeat;
-  a.obs_in = obs_in; a.steps_in = steps_in; a.done_in = done_in;
-  a.obs = obs; a.steps = steps; a.done = done; a.first_obs = first_obs; a.actions = actions;
-  a.observation_out = observation_out; a.reward_out = reward_out; a.discount_out = discount_out;
-  a.next_observation_out = next_observation_out; a.truncation_out = truncation_out;
-  const bool all_out = reward_out && discount_out && next_observation_out && truncation_out;
-  // pieces between AutoReset points (env_kernels.cuh): the first is at least one step long
-  const long long len = (static_cast<long long>(episode_length) + action_repeat - 1) / action_repeat;
-  long long pieces = 1 + (static_cast<long long>(T) - 1 + len - 1) / len;
-  if (pieces > 65535) pieces = 1;
-  a.segmented = (segmented && all_out && pieces > 1) ? 1 : 0;
-  if (a.segmented)
-    MBPO_REQUIRE(obs != obs_in && steps != steps_in && done != done_in,
-                 "env_unroll: the outgoing env state must not alias the incoming one");
-  const dim3 blocks(static_cast<unsigned>((E + ENV_THREADS - 1) / ENV_THREADS),
-                    a.segmented ? static_cast<unsigned>(pieces) : 1u);
-  cudaStream_t st = as_stream(stream);
-  const auto aligned16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-  const bool fast = all_out && action_repeat == 1 && std::fabs(a.sys.target_angle) <= 6.0f && E % 4 == 0 &&
-                    aligned16(next_observation_out) && aligned16(observation_out) &&
-                    static_cast<long long>(T) * E * 3 < (1ll << 31);
-  const int sel = (all_out ? (observation_out ? 2 : 1) : 0) * 4 + math_mode * 2 + (fast ? 1 : 0);
-  switch (sel) {
-    case 0: case 1: env_rollout_pendulum_checked_kernel<0><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 2: case 3: env_rollout_pendulum_checked_kernel<1><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 4: env_rollout_pendulum_kernel<0, false, false><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 5: env_rollout_pendulum_kernel<0, false, true><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 6: env_rollout_pendulum_kernel<1, false, false><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 7: env_rollout_pendulum_kernel<1, false, true><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 8: env_rollout_pendulum_kernel<0, true, false><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 9: env_rollout_pendulum_kernel<0, true, true><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    case 10: env_rollout_pendulum_kernel<1, true, false><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-    default: env_rollout_pendulum_kernel<1, true, true><<<blocks, ENV_THREADS, 0, st>>>(a); break;
-  }
-  return check_launch("env_rollout_pendulum_kernel");
-}
-}  // namespace
-}  // extern "C++"
-
-int mbpo_env_rollout(int system_kind, const void* sys_params_host, int math_mode, int x_dim, int action_dim,
-                     int episode_length, int action_repeat, float* obs, float* steps, float* done,
-                     const float* first_obs, const float* actions, int E, int T, float* observation_out,
-                     float* reward_out, float* discount_out, float* next_observation_out, float* truncation_out,
-                     void* stream) {
-  return launch_env(system_kind, sys_params_host, math_mode, x_dim, action_dim, episode_length, action_repeat, obs,
-                    steps, done, obs, steps, done, first_obs, actions, E, T, observation_out, reward_out,
-                    discount_out, next_observation_out, truncation_out, false, stream);
-}
-
-int mbpo_env_unroll(int system_kind, const void* sys_params_host, int math_mode, int x_dim, int action_dim,
-                    int episode_length, int action_repeat, const float* obs_in, const float* steps_in,
-                    const float* done_in, float* obs_out, float* steps_out, float* done_out,
-                    const float* first_obs, const float* actions, int E, int T, float* observation_out,
-                    float* reward_out, float* discount_out, float* next_observation_out, float* truncation_out,
-                    void* stream) {
-  return launch_env(system_kind, sys_params_host, math_mode, x_dim, action_dim, episode_length, action_repeat,
-                    obs_in, steps_in, done_in, obs_out, steps_out, done_out, first_obs, actions, E, T,
-                    observation_out, reward_out, discount_out, next_observation_out, truncation_out, true, stream);
 }
 
 // ---- policy in the env loop: actor_step / generate_unroll / get_experience ------------------------------
@@ -1033,55 +918,26 @@ int mbpo_actor_rollout_extras(int system_kind, const void* sys_params_host, int 
   MBPO_REQUIRE(prng_mode == 0 || prng_mode == 1, "actor_rollout: bad prng_mode %d", prng_mode);
   MBPO_REQUIRE(key_convention >= 0 && key_convention <= 2, "actor_rollout: bad key_convention %d", key_convention);
   MBPO_REQUIRE(E >= 0 && T >= 0 && episode_length >= 1 && action_repeat >= 1, "actor_rollout: bad sizes");
-  if (policy_host->hidden != mbpo::ACT_W || policy_host->obs_dim != 3 || policy_host->action_dim != 1 ||
-      policy_host->num_hidden < 1 || policy_host->num_hidden > mbpo::ACT_MAX_HIDDEN)
-    return fail(MBPO_EUNSUPPORTED,
-                "actor_rollout: the policy kernel needs obs_dim == 3, action_dim == 1, 1..%d hidden layers of width %d "
-                "(got obs %d, act %d, %d x %d)",
-                mbpo::ACT_MAX_HIDDEN, mbpo::ACT_W, policy_host->obs_dim, policy_host->action_dim,
-                policy_host->num_hidden, policy_host->hidden);
-  for (int l = 0; l <= policy_host->num_hidden; ++l)
-    MBPO_REQUIRE(policy_host->w[l] && policy_host->b[l], "actor_rollout: null policy weights (layer %d)", l);
+  mbpo::ActorArgs a;
+  int rc = fill_policy("actor_rollout", policy_host, E, PendulumSys::X, PendulumSys::A, a);
+  if (rc != MBPO_OK) return rc;
   MBPO_REQUIRE(policy_host->head == MBPO_HEAD_NORMAL_TANH || policy_host->head == MBPO_HEAD_BPTT_ACTOR,
                "actor_rollout: bad policy head %d", policy_host->head);
-  if (E == 0 || T == 0) {
-    if (key_out && key_out != key_in) {
-      const cudaError_t ce = cudaMemcpyAsync(key_out, key_in, 2 * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
-                                             as_stream(stream));
-      if (ce != cudaSuccess) return fail(MBPO_ECUDA, "actor_rollout copy: %s", cudaGetErrorString(ce));
-    }
-    return MBPO_OK;
-  }
-  mbpo::ActorArgs a;
+  MBPO_REQUIRE(policy_host->kernel >= MBPO_ACTOR_AUTO && policy_host->kernel <= MBPO_ACTOR_TCGEN05_WIDE,
+               "actor_rollout: bad policy kernel selector %d", policy_host->kernel);
+  cudaStream_t st = as_stream(stream);
+  if (E == 0 || T == 0) return copy_async(key_out, key_in, key_out ? 2 * sizeof(uint32_t) : 0, st, "actor_rollout");
   a.sys = *static_cast<const MbpoPendulumParams*>(sys_params_host);
   a.E = E; a.T = T; a.episode_length = episode_length; a.action_repeat = action_repeat;
-  a.num_hidden = policy_host->num_hidden; a.deterministic = deterministic; a.key_convention = key_convention;
-  a.min_std = policy_host->min_std;
-  a.head = policy_host->head; a.shared_noise = policy_host->shared_noise; a.normalize = policy_host->normalize;
+  a.deterministic = deterministic; a.key_convention = key_convention;
+  a.head = policy_host->head; a.shared_noise = policy_host->shared_noise;
   a.sig_bias = policy_host->sig_bias; a.sig_min = policy_host->sig_min; a.sig_max = policy_host->sig_max;
   a.action_clip = policy_host->action_clip;
-  MBPO_REQUIRE(policy_host->draw_total == 0 ||
-                   (policy_host->draw_offset >= 0 && policy_host->draw_offset + E <= policy_host->draw_total),
-               "actor_rollout: envs [%d, %d) are not inside draw_total %d", policy_host->draw_offset,
-               policy_host->draw_offset + E, policy_host->draw_total);
-  a.draw_total = policy_host->draw_total > 0 ? policy_host->draw_total : E;
-  a.draw_offset = policy_host->draw_total > 0 ? policy_host->draw_offset : 0;
-  for (int i = 0; i < 3; ++i) { a.obs_mean[i] = policy_host->obs_mean[i]; a.obs_std[i] = policy_host->obs_std[i]; }
-  MBPO_REQUIRE((policy_host->obs_mean_dev == nullptr) == (policy_host->obs_std_dev == nullptr),
-               "actor_rollout: obs_mean_dev and obs_std_dev come together");
-  a.obs_mean_dev = policy_host->obs_mean_dev; a.obs_std_dev = policy_host->obs_std_dev;
-  for (int l = 0; l <= mbpo::ACT_MAX_HIDDEN; ++l) {
-    a.w[l] = l <= a.num_hidden ? policy_host->w[l] : nullptr;
-    a.b[l] = l <= a.num_hidden ? policy_host->b[l] : nullptr;
-  }
   a.key_in = key_in;
   a.obs = obs; a.steps = steps; a.done = done; a.first_obs = first_obs;
   a.action_out = action_out; a.reward_out = reward_out; a.discount_out = discount_out;
   a.next_observation_out = next_observation_out; a.truncation_out = truncation_out; a.key_out = key_out;
   a.raw_action_out = raw_action_out; a.log_prob_out = log_prob_out;
-  cudaStream_t st = as_stream(stream);
-  MBPO_REQUIRE(policy_host->kernel >= MBPO_ACTOR_AUTO && policy_host->kernel <= MBPO_ACTOR_TCGEN05_WIDE,
-               "actor_rollout: bad policy kernel selector %d", policy_host->kernel);
   const bool tc_ok = a.num_hidden >= 2 && a.num_hidden <= 1 + mbpo::atc::MAX_HH;
   if ((policy_host->kernel == MBPO_ACTOR_TCGEN05 || policy_host->kernel == MBPO_ACTOR_TCGEN05_WIDE) && !tc_ok)
     return fail(MBPO_EUNSUPPORTED, "actor_rollout: the tcgen05 kernel holds 1..%d hidden -> hidden layers (got %d hidden layers)",
@@ -1089,28 +945,11 @@ int mbpo_actor_rollout_extras(int system_kind, const void* sys_params_host, int 
   // few envs (at most one 128-env tile per SM): the latency kernel; otherwise the throughput kernel
   const bool wide = policy_host->kernel == MBPO_ACTOR_TCGEN05_WIDE ||
                     (policy_host->kernel == MBPO_ACTOR_AUTO && (E + mbpo::atc::TILE - 1) / mbpo::atc::TILE <= device_sm_count());
-  if (tc_ok && wide) {
-    switch (prng_mode * 2 + math_mode) {
-      case 0: return launch_actor_tc_wide<0, 0>(a, st);
-      case 1: return launch_actor_tc_wide<0, 1>(a, st);
-      case 2: return launch_actor_tc_wide<1, 0>(a, st);
-      default: return launch_actor_tc_wide<1, 1>(a, st);
-    }
-  }
-  if (tc_ok && policy_host->kernel != MBPO_ACTOR_CUDA_CORES) {
-    switch (prng_mode * 2 + math_mode) {
-      case 0: return launch_actor_tc<0, 0>(a, st);
-      case 1: return launch_actor_tc<0, 1>(a, st);
-      case 2: return launch_actor_tc<1, 0>(a, st);
-      default: return launch_actor_tc<1, 1>(a, st);
-    }
-  }
-  switch (prng_mode * 2 + math_mode) {
-    case 0: return launch_actor<0, 0>(a, st);
-    case 1: return launch_actor<0, 1>(a, st);
-    case 2: return launch_actor<1, 0>(a, st);
-    default: return launch_actor<1, 1>(a, st);
-  }
+  return with_prng_math(prng_mode, math_mode, [&](auto P, auto M) {
+    if (tc_ok && wide) return launch_actor_tc_wide<P, M>(a, st);
+    if (tc_ok && policy_host->kernel != MBPO_ACTOR_CUDA_CORES) return launch_actor_tc<P, M>(a, st);
+    return launch_actor<P, M>(a, st);
+  });
 }
 
 // ---- reverse pass through System.step rollouts, lambda returns (SURVEY 8f-4) ---------------------------

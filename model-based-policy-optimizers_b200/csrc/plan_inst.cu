@@ -160,30 +160,15 @@ int launch(const PlanArgs& a, const MpcArgs* mpc, cudaStream_t st) {
 template <>
 int plan_entry<MBPO_INST_H>(int prng_mode, int math_mode, const PlanArgs& a, const MpcArgs* mpc, cudaStream_t st,
                             int cluster) {
-  if (cluster > 1) {
-    switch (prng_mode * 2 + math_mode) {
-      case 0: return launch_cluster<0, 0>(a, mpc, st, cluster);
-      case 1: return launch_cluster<0, 1>(a, mpc, st, cluster);
-      case 2: return launch_cluster<1, 0>(a, mpc, st, cluster);
-      default: return launch_cluster<1, 1>(a, mpc, st, cluster);
-    }
-  }
-  switch (prng_mode * 2 + math_mode) {
-    case 0: return launch<0, 0>(a, mpc, st);
-    case 1: return launch<0, 1>(a, mpc, st);
-    case 2: return launch<1, 0>(a, mpc, st);
-    default: return launch<1, 1>(a, mpc, st);
-  }
+  return with_prng_math(prng_mode, math_mode, [&](auto P, auto M) {
+    return cluster > 1 ? launch_cluster<P, M>(a, mpc, st, cluster) : launch<P, M>(a, mpc, st);
+  });
 }
 
 template <>
 int plan_cluster_capacity<MBPO_INST_H>(int prng_mode, int math_mode, bool mpc, int N, int Np, int K, int cluster) {
-  switch (prng_mode * 2 + math_mode) {
-    case 0: return cluster_capacity<0, 0>(mpc, N, Np, K, cluster);
-    case 1: return cluster_capacity<0, 1>(mpc, N, Np, K, cluster);
-    case 2: return cluster_capacity<1, 0>(mpc, N, Np, K, cluster);
-    default: return cluster_capacity<1, 1>(mpc, N, Np, K, cluster);
-  }
+  return with_prng_math(prng_mode, math_mode,
+                        [&](auto P, auto M) { return cluster_capacity<P, M>(mpc, N, Np, K, cluster); });
 }
 
 namespace {
@@ -205,11 +190,9 @@ int launch_general(const PlanArgs& a, cudaStream_t st) {
 
 template <>
 int general_plan_entry<MBPO_INST_H>(int system_kind, int prng_mode, const PlanArgs& a, cudaStream_t st) {
-  if (system_kind == MBPO_SYSTEM_NOISY_PENDULUM)
-    return prng_mode == 0 ? launch_general<NoisyPendulumSys, 0>(a, st) : launch_general<NoisyPendulumSys, 1>(a, st);
-  if (system_kind == MBPO_SYSTEM_POINT_MASS)
-    return prng_mode == 0 ? launch_general<PointMassSys, 0>(a, st) : launch_general<PointMassSys, 1>(a, st);
-  return fail(MBPO_EUNSUPPORTED, "general fused plan: system_kind %d", system_kind);
+  return with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    return with_prng(prng_mode, [&](auto P) { return launch_general<typename decltype(t)::type, P>(a, st); });
+  });
 }
 
 template <>
@@ -217,9 +200,10 @@ int noise_entry<MBPO_INST_H>(int prng_mode, const ScaleTable& tbl, const uint32_
                              uint32_t* bits_out, cudaStream_t st) {
   const int threads = STAGED_THREADS;
   const unsigned blocks = static_cast<unsigned>((M + threads - 1) / threads);
-  if (prng_mode == 0) powerlaw_noise_kernel<kH, 0><<<blocks, threads, 0, st>>>(tbl, keys, M, noise_out, bits_out);
-  else powerlaw_noise_kernel<kH, 1><<<blocks, threads, 0, st>>>(tbl, keys, M, noise_out, bits_out);
-  return check_launch("powerlaw_noise_kernel");
+  return with_prng(prng_mode, [&](auto P) {
+    powerlaw_noise_kernel<kH, P><<<blocks, threads, 0, st>>>(tbl, keys, M, noise_out, bits_out);
+    return check_launch("powerlaw_noise_kernel");
+  });
 }
 
 template <>
@@ -228,13 +212,11 @@ int sample_entry<MBPO_INST_H>(int prng_mode, const ScaleTable& tbl, const uint32
                               float* actions, uint32_t* next_key, uint32_t* particle_keys, cudaStream_t st) {
   const int threads = STAGED_THREADS;
   const dim3 grid(static_cast<unsigned>(((N + Np) * A + threads - 1) / threads), static_cast<unsigned>(B));
-  if (prng_mode == 0)
-    sample_actions_kernel<kH, 0><<<grid, threads, 0, st>>>(tbl, carry_key, mean, std_, N, Np, A, u_min, u_max,
+  return with_prng(prng_mode, [&](auto P) {
+    sample_actions_kernel<kH, P><<<grid, threads, 0, st>>>(tbl, carry_key, mean, std_, N, Np, A, u_min, u_max,
                                                            actions, next_key, particle_keys);
-  else
-    sample_actions_kernel<kH, 1><<<grid, threads, 0, st>>>(tbl, carry_key, mean, std_, N, Np, A, u_min, u_max,
-                                                           actions, next_key, particle_keys);
-  return check_launch("sample_actions_kernel");
+    return check_launch("sample_actions_kernel");
+  });
 }
 
 #ifdef MBPO_CLUSTER_CLOCKS

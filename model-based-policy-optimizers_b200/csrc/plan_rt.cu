@@ -44,12 +44,7 @@ int launch_rt(const PlanArgs& a, const MpcArgs* mpc, cudaStream_t st) {
 }  // namespace
 
 int plan_entry_rt(int prng_mode, int math_mode, const PlanArgs& a, const MpcArgs* mpc, cudaStream_t st) {
-  switch (prng_mode * 2 + math_mode) {
-    case 0: return launch_rt<0, 0>(a, mpc, st);
-    case 1: return launch_rt<0, 1>(a, mpc, st);
-    case 2: return launch_rt<1, 0>(a, mpc, st);
-    default: return launch_rt<1, 1>(a, mpc, st);
-  }
+  return with_prng_math(prng_mode, math_mode, [&](auto P, auto M) { return launch_rt<P, M>(a, mpc, st); });
 }
 
 }  // namespace mbpo

@@ -423,11 +423,10 @@ int mbpo_prng_randint(const uint32_t* keys, int M, int n, int prng_mode, int min
   const uint32_t span = randint_span(minval, maxval);
   const int threads = 256;
   const unsigned blocks = static_cast<unsigned>((total + threads - 1) / threads);
-  if (prng_mode == 0)
-    prng_randint_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, minval, span, out);
-  else
-    prng_randint_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, minval, span, out);
-  return check_launch("prng_randint_kernel");
+  return with_prng(prng_mode, [&](auto P) {
+    prng_randint_kernel<P><<<blocks, threads, 0, as_stream(stream)>>>(keys, total, n, minval, span, out);
+    return check_launch("prng_randint_kernel");
+  });
 }
 
 int mbpo_replay_insert(MbpoReplayState* s, const MbpoReplayFields* fields, long long n_rows, void* stream) {
@@ -497,13 +496,11 @@ int mbpo_replay_sample(const MbpoReplayState* s, const uint32_t* key, int prng_m
   const uint32_t span = randint_span(minval, maxval);
   const int threads = 128;
   const unsigned blocks = static_cast<unsigned>((sample_batch_size + threads - 1) / threads);
-  if (prng_mode == 0)
-    replay_sample_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(
+  return with_prng(prng_mode, [&](auto P) {
+    replay_sample_kernel<P><<<blocks, threads, 0, as_stream(stream)>>>(
         s->data, s->capacity, s->row_width, s->head, key, sample_batch_size, minval, span, key_out, idx_out, batch_out);
-  else
-    replay_sample_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(
-        s->data, s->capacity, s->row_width, s->head, key, sample_batch_size, minval, span, key_out, idx_out, batch_out);
-  return check_launch("replay_sample_kernel");
+    return check_launch("replay_sample_kernel");
+  });
 }
 
 int mbpo_replay_read(const MbpoReplayState* s, long long first, long long n, float* rows_out, void* stream) {
@@ -538,15 +535,12 @@ int mbpo_env_reset_from_buffer(const MbpoReplayState* s, const uint32_t* rngs, i
   const uint32_t span = randint_span(minval, maxval);
   const int threads = 128;
   const unsigned blocks = static_cast<unsigned>((E + threads - 1) / threads);
-  if (prng_mode == 0)
-    env_reset_kernel<0><<<blocks, threads, 0, as_stream(stream)>>>(s->data, s->capacity, s->row_width, s->head, rngs, E,
+  return with_prng(prng_mode, [&](auto P) {
+    env_reset_kernel<P><<<blocks, threads, 0, as_stream(stream)>>>(s->data, s->capacity, s->row_width, s->head, rngs, E,
                                                                   sample_batch_size, minval, span, x_dim, reward_col,
                                                                   obs_out, reward_out, sys_key_out, idx_out);
-  else
-    env_reset_kernel<1><<<blocks, threads, 0, as_stream(stream)>>>(s->data, s->capacity, s->row_width, s->head, rngs, E,
-                                                                  sample_batch_size, minval, span, x_dim, reward_col,
-                                                                  obs_out, reward_out, sys_key_out, idx_out);
-  return check_launch("env_reset_kernel");
+    return check_launch("env_reset_kernel");
+  });
 }
 
 int mbpo_eval_metrics(const float* reward, const float* discount, const float* steps_in, const float* done_in,

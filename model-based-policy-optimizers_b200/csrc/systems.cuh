@@ -24,7 +24,7 @@
 namespace mbpo {
 
 struct PendulumSys {
-  static constexpr int X = 3, A = 1;
+  static constexpr int KIND = MBPO_SYSTEM_PENDULUM, X = 3, A = 1;
   static constexpr bool KEYED = false;
   PendulumConsts pc;
   __device__ explicit PendulumSys(const MbpoGeneralSystemParams& p) : pc(p.pendulum) {}
@@ -36,8 +36,21 @@ struct PendulumSys {
   }
 };
 
+// The pendulum under MBPO_MATH_THETA_CARRY where theta is not carried between steps: each step re-derives it from
+// [cos, sin], steps it with pendulum_step_theta and writes [cos, sin] back (system_step_pendulum_kernel<1>).
+struct PendulumThetaSys : PendulumSys {
+  using PendulumSys::PendulumSys;
+  template <int PRNG>
+  __device__ __forceinline__ float step(float (&x)[X], const float* u, int ustride, Key2&) const {
+    float th = atan2_bounded(x[1], x[0]), r;
+    pendulum_step_theta(pc, th, x[2], u[0], r);
+    sincos_bounded(th, x[1], x[0]);
+    return r;
+  }
+};
+
 struct NoisyPendulumSys {
-  static constexpr int X = 3, A = 1;
+  static constexpr int KIND = MBPO_SYSTEM_NOISY_PENDULUM, X = 3, A = 1;
   static constexpr bool KEYED = true;
   PendulumConsts pc;
   float noise_std;
@@ -59,7 +72,7 @@ struct NoisyPendulumSys {
 };
 
 struct PointMassSys {
-  static constexpr int X = 4, A = 2;
+  static constexpr int KIND = MBPO_SYSTEM_POINT_MASS, X = 4, A = 2;
   static constexpr bool KEYED = false;
   MbpoPointMassParams p;
   __device__ explicit PointMassSys(const MbpoGeneralSystemParams& g) : p(g.point_mass) {}
@@ -82,6 +95,28 @@ struct PointMassSys {
     return reward;
   }
 };
+
+template <class T>
+struct TypeTag { using type = T; };
+
+// Runtime system_kind -> System struct: f(TypeTag<Sys>{}) for the one of the listed Systems whose KIND is `kind`,
+// MBPO_EUNSUPPORTED (no message) when none is.  Each call site lists the Systems it serves, so only their kernels
+// are instantiated.
+template <class... Sys, class F>
+int with_system(int kind, F&& f) {
+  int rc = MBPO_EUNSUPPORTED;
+  (void)((kind == Sys::KIND && (rc = f(TypeTag<Sys>{}), true)) || ...);
+  return rc;
+}
+
+// X, A and KEYED of a general System; MBPO_EUNSUPPORTED (no message) for any other kind.
+inline int general_system_dims(int kind, int* X, int* A, bool* keyed) {
+  return with_system<PendulumSys, NoisyPendulumSys, PointMassSys>(kind, [&](auto t) {
+    using Sys = typename decltype(t)::type;
+    *X = Sys::X; *A = Sys::A; *keyed = Sys::KEYED;
+    return MBPO_OK;
+  });
+}
 
 // vmap(System.step): one thread per row.
 template <class Sys, int PRNG>

@@ -334,9 +334,9 @@ class GraphedRollout:
                  key_convention: int = _lib.KEYS_SAC, extra_fields: Sequence[str] = ("truncation",)):
         dev = env_state.obs.device
         params = env_state.system_params
-        keyed = is_general(env.system) and env.system.keyed     # the System's keys are replay state too
-        if keyed:
-            params = params.replace(key=system_keys(env.system, params, env_state.obs.shape[0]).clone())
+        keys = system_keys(env.system, params, env_state.obs.shape[0])   # a keyed System's keys are replay state too
+        if keys is not None:
+            params = params.replace(key=keys.clone())
         self._state = EnvState(obs=env_state.obs.clone(), reward=env_state.reward.clone(), done=env_state.done.clone(),
                                system_params=params, info={k: v.clone() for k, v in env_state.info.items()})
         self._key = key.reshape(2).clone()
@@ -357,7 +357,7 @@ class GraphedRollout:
             self._state.done.copy_(nstate.done)
             self._state.info["steps"].copy_(nstate.info["steps"])
             self._key.copy_(key_out)
-            if keyed:
+            if keys is not None:
                 self._state.system_params.key.copy_(nstate.system_params.key)
         self._out = (key_out, nstate, tr)
 

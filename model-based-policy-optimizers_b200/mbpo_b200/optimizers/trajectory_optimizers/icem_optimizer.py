@@ -21,6 +21,7 @@ import torch
 from ... import _lib
 from ... import random as jr
 from ...config import config
+from ...envs import is_general
 from ...systems.base_systems import System
 from ...utils.type_aliases import OptimizerState, OptimizerTrainingOutPut
 from ..base_optimizer import BaseOptimizer
@@ -258,7 +259,7 @@ class iCemTO(BaseOptimizer):
         with L.cuda_guard(x0):
             for _ in range(S):
                 nxt_carry = torch.empty_like(carry)
-                general = self.system.system_kind in (L.SYSTEM_NOISY_PENDULUM, L.SYSTEM_POINT_MASS)
+                general = is_general(self.system)
                 pkeys = torch.empty((B, M, 2), dtype=torch.uint32, device=dev) if general else None
                 L.check(L.lib.mbpo_icem_sample_actions(L.C.byref(cfg), L.ptr(carry), L.ptr(mean), L.ptr(std), B,
                                                        L.ptr(actions), L.ptr(nxt_carry), L.ptr(pkeys), st))

@@ -1085,15 +1085,28 @@ def test_env_rollout(mb, cuda_device, math_mode, E, T, episode_length, action_re
 
 
 def test_env_rollout_abi_variants(mb, cuda_device):
-    """Separate observation buffer (OBS kernel), NULL outputs (checked kernel) and the aliased
-    fast path produce identical bits."""
+    """Separate observation buffer (OBS kernel), NULL outputs (env_unroll_general_kernel) and the aliased
+    fast path, in both math modes.  In reference math all three produce identical bits.  Under theta-carry the
+    NULL-output path re-derives theta every step where the segmented kernel carries it, so it is checked instead
+    against a step-by-step loop of mbpo_system_step (the same atan2 -> step -> sincos) and the AutoReset
+    bookkeeping."""
+    try:
+        for math_mode in ("reference", "theta_carry"):
+            mb.config.math_mode = math_mode
+            _check_env_rollout_abi_variants(mb, cuda_device, math_mode)
+    finally:
+        mb.config.math_mode = "reference"
+
+
+def _check_env_rollout_abi_variants(mb, cuda_device, math_mode):
     L = mb._lib
     from mbpo_b200.envs import wrap
     from mbpo_b200.systems import PendulumSystem
-    E, T = 333, 23
+    E, T, ep_len = 333, 23, 9
+    M = mb.config.math_mode_id
     sys_ = PendulumSystem()
     sp = sys_.reset(device=cuda_device).system_params
-    env = wrap(sys_, sp, episode_length=9)
+    env = wrap(sys_, sp, episode_length=ep_len)
     x0 = _dev(_random_states(E, 61), cuda_device)
     acts = _dev(np.random.default_rng(62).uniform(-1, 1, (T, E, 1)).astype(np.float32), cuda_device)
     st = env.reset(x0)
@@ -1107,15 +1120,31 @@ def test_env_rollout_abi_variants(mb, cuda_device):
         r = torch.zeros((T, E), device=cuda_device)
         d = torch.zeros((T, E), device=cuda_device) if with_rest else None
         t_ = torch.zeros((T, E), device=cuda_device) if with_rest else None
-        L.check(L.lib.mbpo_env_rollout(0, L.C.addressof(pp), 0, 3, 1, 9, 1, L.ptr(obs), L.ptr(steps), L.ptr(done),
-                                       L.ptr(st.info["first_obs"]), L.ptr(acts), E, T, L.ptr(o), L.ptr(r), L.ptr(d),
-                                       L.ptr(n), L.ptr(t_), L.stream_ptr(cuda_device)))
+        L.check(L.lib.mbpo_env_rollout(0, L.C.addressof(pp), M, 3, 1, ep_len, 1, L.ptr(obs), L.ptr(steps),
+                                       L.ptr(done), L.ptr(st.info["first_obs"]), L.ptr(acts), E, T, L.ptr(o), L.ptr(r),
+                                       L.ptr(d), L.ptr(n), L.ptr(t_), L.stream_ptr(cuda_device)))
         return o, n, r, d, t_, obs
     o, n, r, d, t_, obs = call(True, True)                     # OBS kernel
     assert torch.equal(o, tr.observation) and torch.equal(n, tr.next_observation) and torch.equal(r, tr.reward)
     assert torch.equal(d, tr.discount) and torch.equal(t_, tr.extras["state_extras"]["truncation"])
-    o2, n2, r2, _, _, obs2 = call(True, False)                 # checked kernel (NULL discount / truncation)
-    assert torch.equal(o2, o) and torch.equal(n2, n) and torch.equal(r2, r) and torch.equal(obs2, obs)
+    o2, n2, r2, _, _, obs2 = call(True, False)                 # NULL discount / truncation
+    if math_mode == "reference":
+        assert torch.equal(o2, o) and torch.equal(n2, n) and torch.equal(r2, r) and torch.equal(obs2, obs)
+        return
+    x, steps, done = st.obs.clone(), st.info["steps"].clone(), st.done.clone()
+    first = st.info["first_obs"]
+    for t in range(T):
+        steps = torch.where(done != 0, torch.zeros_like(steps), steps)
+        assert torch.equal(o2[t], x)
+        xn, rew = torch.empty_like(x), torch.empty((E,), device=cuda_device)
+        L.check(L.lib.mbpo_system_step(0, L.C.addressof(pp), M, L.ptr(x), L.ptr(acts[t].contiguous()), E, L.ptr(xn),
+                                       L.ptr(rew), L.stream_ptr(cuda_device)))
+        steps = steps + 1.0
+        over = steps >= ep_len
+        done = over.to(torch.float32)
+        x = torch.where(over[:, None], first, xn)
+        assert torch.equal(r2[t], rew) and torch.equal(n2[t], x)
+    assert torch.equal(obs2, x)
 
 
 @pytest.mark.parametrize("E,T,episode_length,action_repeat", [(1000, 61, 13, 1), (95, 50, 11, 3), (64, 5, 200, 1)])
