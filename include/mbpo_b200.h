@@ -393,6 +393,27 @@ int mbpo_actor_rollout_general(int system_kind, const MbpoGeneralSystemParams* p
                                float* truncation_out, uint32_t* key_out, float* raw_action_out,
                                float* log_prob_out, void* stream);
 
+/* rollout_policy (mbpo/utils/optimizer_utils.py:62-116) for the general Systems: the plain scan of T System.steps
+ * from x0 [E,X] with the policy in the loop -- no Episode / AutoReset wrapper, so no step counter, done or
+ * truncation (discount is 1).  The policy runs on the CUDA cores as in mbpo_actor_rollout_general; its head is
+ * MBPO_HEAD_BPTT_ACTOR (BPTT.act, bptt_optimizer.py:123-142,306-326; with shared_noise the draw normal(key, (A,)) is
+ * the same for every trajectory, element a for action dim a) or MBPO_HEAD_NORMAL_TANH (the draw of
+ * mbpo_actor_rollout_general).  key_convention as there (BPTT: MBPO_KEYS_UNROLL, or MBPO_KEYS_AS_IS to evaluate).
+ * Outputs are time-major: action_out [T,E,A], reward_out [T,E], next_observation_out [T,E,X] (observation[t] =
+ * next_observation[t-1], observation[0] = x0).  sys_keys_in / sys_keys_out: a keyed System's system_params.key,
+ * uint32 [2] shared by every trajectory (sys_keys_shared = 1) or [E,2] -- required for a keyed System, ignored
+ * otherwise; each System.step advances it once.  key_in / key_out: the policy's carry key.  E or T == 0 copies the
+ * keys through.  X = 4 needs a 16-byte aligned next_observation_out.  MBPO_SYSTEM_PENDULUM is MBPO_EINVAL (it keeps
+ * mbpo_actor_rollout); MBPO_EUNSUPPORTED: any other non-general kind, kernel = MBPO_ACTOR_TCGEN05 /
+ * MBPO_ACTOR_TCGEN05_WIDE and policy shapes other than those of mbpo_actor_rollout_general. */
+int mbpo_rollout_policy_general(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode,
+                                const MbpoPolicyParams* policy_host, int deterministic, int key_convention,
+                                const uint32_t* key_in, const uint32_t* sys_keys_in /*[2] or [E,2] or NULL*/,
+                                int sys_keys_shared, const float* x0 /*[E,X]*/, int E, int T,
+                                float* action_out /*[T,E,A]*/, float* reward_out /*[T,E]*/,
+                                float* next_observation_out /*[T,E,X]*/, uint32_t* key_out, uint32_t* sys_keys_out,
+                                void* stream);
+
 /* ---- reverse pass through System.step rollouts; lambda returns (BPTT) ----------------------- */
 /* The cotangent pass of jax.value_and_grad through rollout_policy(..., stop_grads=True)
  * (mbpo/utils/optimizer_utils.py:62-116; bptt_optimizer.py:327-376): the policy sees
@@ -409,6 +430,20 @@ int mbpo_rollout_adjoint(int system_kind, const void* sys_params_host, int x_dim
                          long long stride_xe, const float* observation, const float* action,
                          const float* g_reward, const float* g_next_obs, const float* g_obs,
                          const float* g_action_in, float* g_action_out, float* g_x0_out, void* stream);
+
+/* mbpo_rollout_adjoint for the general Systems (the trajectory of mbpo_rollout_policy_general):
+ * MBPO_SYSTEM_NOISY_PENDULUM, whose noise does not depend on (x, u), so its Jacobians are the pendulum's at the
+ * stored noisy observation and no key is needed; and MBPO_SYSTEM_POINT_MASS (clip ties split the cotangent in half,
+ * as jnp.clip does).  stride_t / stride_e address g_reward; stride_xt / stride_xe the [.,.,X] arrays (observation,
+ * g_next_obs, g_obs); stride_at / stride_ae the [.,.,A] arrays (action, g_action_in, g_action_out), innermost
+ * stride 1 for both.  g_x0_out is [E,X].  MBPO_SYSTEM_PENDULUM is MBPO_EINVAL (it keeps mbpo_rollout_adjoint); any
+ * other non-general kind is MBPO_EUNSUPPORTED. */
+int mbpo_rollout_adjoint_general(int system_kind, const MbpoGeneralSystemParams* params_host, int E, int T,
+                                 long long stride_t, long long stride_e, long long stride_xt, long long stride_xe,
+                                 long long stride_at, long long stride_ae, const float* observation,
+                                 const float* action, const float* g_reward, const float* g_next_obs,
+                                 const float* g_obs, const float* g_action_in, float* g_action_out, float* g_x0_out,
+                                 void* stream);
 
 /* lambda_return (mbpo/utils/optimizer_utils.py:119-131): inputs = reward + discount * next_values *
  * (1 - lambda); returns[t] = inputs[t] + discount * lambda * returns[t+1], returns[T] = next_values[-1].

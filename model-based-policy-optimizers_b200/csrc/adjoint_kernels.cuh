@@ -9,8 +9,10 @@
 //     lam_t   = (df/dx)^T (g_next_obs[t] + lam_{t+1}) + g_reward[t] dr/dx          (state adjoint)
 //     ga_t    = g_action[t] + (df/da)^T (g_next_obs[t] + lam_{t+1}) + g_reward[t] dr/da
 // rollout_adjoint_pendulum_kernel runs that reverse scan for one trajectory per thread (the 3 x 3
-// Jacobian-transpose products written out for pendulum_dynamics.py:29-63 and pendulum_reward.py:27-42),
-// re-deriving the step's intermediates from the stored (observation, action) instead of saving them.
+// Jacobian-transpose products written out for pendulum_dynamics.py:29-63 and pendulum_reward.py:27-42,
+// pendulum.cuh pendulum_step_vjp), re-deriving the step's intermediates from the stored (observation, action)
+// instead of saving them; rollout_adjoint_general_kernel does the same for the general Systems through their
+// step_vjp (systems.cuh).
 // The parameter gradient sum_t (da_t/dtheta)^T ga_t has no sequential dependency left and is one
 // batched network backward over all T*E (obs, ga) rows -- the caller's autodiff.
 //
@@ -23,6 +25,7 @@
 // without copies; time-major makes every warp access a contiguous line.
 #pragma once
 #include "pendulum.cuh"
+#include "systems.cuh"
 
 namespace mbpo {
 
@@ -41,14 +44,6 @@ struct AdjointArgs {
   float* g_x0_out;                 // [E,3] cotangent of the initial state (NULL = not wanted)
 };
 
-// jnp.clip = minimum(maximum(x, lo), hi): lax.max / lax.min split the cotangent evenly at a tie.
-__device__ __forceinline__ float clip_grad(float x, float lo, float hi) {
-  const float a = (x > lo) ? 1.0f : (x == lo ? 0.5f : 0.0f);          // d max(x, lo) / dx
-  const float m = fmaxf(x, lo);
-  const float b = (m < hi) ? 1.0f : (m == hi ? 0.5f : 0.0f);          // d min(m, hi) / dm
-  return a * b;
-}
-
 __global__ void __launch_bounds__(128) rollout_adjoint_pendulum_kernel(const __grid_constant__ AdjointArgs a) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= a.E) return;
@@ -66,40 +61,69 @@ __global__ void __launch_bounds__(128) rollout_adjoint_pendulum_kernel(const __g
       const long long j3 = i3 + a.sx_t;
       gc += a.g_obs[j3]; gs += a.g_obs[j3 + 1]; gw += a.g_obs[j3 + 2];
     }
-    // forward intermediates of this step (pendulum_dynamics.py:35,59-62,40,43)
-    const float th = atan2_bounded(s, c);
-    float sin_th, cos_th;
-    sincos_bounded(th, sin_th, cos_th);
-    const float uu = __fmul_rn(fminf(fmaxf(u, -1.0f), 1.0f), pc.max_torque);
-    const float thdd = fmaf(pc.c_g, sin_th, __fmul_rn(pc.c_u, uu));
-    const float v = fmaf(thdd, pc.dt, w);
-    const float nw = fminf(fmaxf(v, -pc.max_speed), pc.max_speed);
-    const float nth = fmaf(nw, pc.dt, th);
-    float sn, cn;
-    sincos_bounded(nth, sn, cn);
-    // x_next = [cos(nth), sin(nth), nw]
-    const float g_nth = cn * gs - sn * gc;
-    const float g_nw = gw + pc.dt * g_nth;
-    const float g_v = g_nw * clip_grad(v, -pc.max_speed, pc.max_speed);
-    const float g_thdd = pc.dt * g_v;
-    // reward on (x_t, a_t) (pendulum_reward.py:32-39); d/dth of the wrapped difference is 1
-    const float diff = wrap_diff(th - pc.target_angle);
-    float g_th = g_nth + g_thdd * pc.c_g * cos_th - gr * 2.0f * pc.angle_cost * diff;
-    const float g_w = g_v - gr * 0.2f * w;
-    float g_u = g_thdd * pc.c_u * pc.max_torque * clip_grad(u, -1.0f, 1.0f) - gr * 2.0f * pc.control_cost * u;
+    float g_u;
+    pendulum_step_vjp(pc, c, s, w, u, gc, gs, gw, gr, lc, ls, lw, g_u);
     if (a.g_action_in) g_u += a.g_action_in[i1];
     a.g_action_out[i1] = g_u;
-    // th = atan2(s, c): dth/dc = -s / (c^2 + s^2), dth/ds = c / (c^2 + s^2)
-    const float r2 = c * c + s * s;
-    const float inv = r2 > 0.0f ? 1.0f / r2 : 0.0f;
-    lc = -g_th * s * inv;
-    ls = g_th * c * inv;
-    lw = g_w;
   }
   if (a.g_x0_out) {
     float gc = lc, gs = ls, gw = lw;
     if (a.g_obs && a.T > 0) { gc += a.g_obs[bx]; gs += a.g_obs[bx + 1]; gw += a.g_obs[bx + 2]; }
     a.g_x0_out[3 * e] = gc; a.g_x0_out[3 * e + 1] = gs; a.g_x0_out[3 * e + 2] = gw;
+  }
+}
+
+struct AdjointGeneralArgs {
+  MbpoGeneralSystemParams sys;
+  int E, T;
+  long long st_t, st_e;            // strides of g_reward, in elements
+  long long sx_t, sx_e;            // strides of the [.,.,X] arrays (innermost stride 1)
+  long long sa_t, sa_e;            // strides of the [.,.,A] arrays: action, g_action_in, g_action_out (innermost 1)
+  const float* observation;        // as AdjointArgs
+  const float* action;
+  const float* g_reward;
+  const float* g_next_obs;
+  const float* g_obs;
+  const float* g_action_in;
+  float* g_action_out;
+  float* g_x0_out;                 // [E,X]
+};
+
+// The same reverse scan for a general System (systems.cuh), through its step_vjp: X-float state adjoint, A action
+// cotangents per step.  A keyed System's noise enters its step additively and depends on neither x nor u, so the
+// scan needs no keys.
+template <class Sys>
+__global__ void __launch_bounds__(128) rollout_adjoint_general_kernel(const __grid_constant__ AdjointGeneralArgs a) {
+  constexpr int X = Sys::X, A = Sys::A;
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= a.E) return;
+  const Sys sys(a.sys);
+  const long long be = static_cast<long long>(e) * a.st_e, bx = static_cast<long long>(e) * a.sx_e;
+  const long long ba = static_cast<long long>(e) * a.sa_e;
+  float lam[X];                              // lam_{t+1}
+#pragma unroll
+  for (int k = 0; k < X; ++k) lam[k] = 0.0f;
+  for (int t = a.T - 1; t >= 0; --t) {
+    const long long i1 = be + t * a.st_t, ix = bx + t * a.sx_t, ia = ba + t * a.sa_t;
+    float x[X], u[A], g[X], g_u[A];
+#pragma unroll
+    for (int k = 0; k < X; ++k) {
+      x[k] = a.observation[ix + k];
+      g[k] = lam[k];
+      if (a.g_next_obs) g[k] += a.g_next_obs[ix + k];
+      if (a.g_obs && t + 1 < a.T) g[k] += a.g_obs[ix + a.sx_t + k];   // observation[t+1] = next_observation[t]
+    }
+#pragma unroll
+    for (int j = 0; j < A; ++j) u[j] = a.action[ia + j];
+    const float gr = a.g_reward ? a.g_reward[i1] : 0.0f;
+    sys.step_vjp(x, u, g, gr, lam, g_u);
+#pragma unroll
+    for (int j = 0; j < A; ++j) a.g_action_out[ia + j] = a.g_action_in ? g_u[j] + a.g_action_in[ia + j] : g_u[j];
+  }
+  if (a.g_x0_out) {
+#pragma unroll
+    for (int k = 0; k < X; ++k)
+      a.g_x0_out[static_cast<long long>(e) * X + k] = (a.g_obs && a.T > 0) ? lam[k] + a.g_obs[bx + k] : lam[k];
   }
 }
 

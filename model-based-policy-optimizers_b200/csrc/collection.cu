@@ -1,7 +1,10 @@
 // C ABI of the SAC / PPO env rollouts (declared in include/mbpo_b200.h): mbpo_env_rollout and mbpo_env_unroll for
 // the pendulum (env_kernels.cuh), mbpo_env_unroll_general and mbpo_actor_rollout_general for the general Systems
-// (general_env_kernels.cuh).  The pendulum's policy-in-the-loop entry points stay in mbpo_b200.cu: its tcgen05
-// kernels include mlp_tc_kernels.cuh, whose stage-4 kernel would otherwise be compiled into both units.
+// (general_env_kernels.cuh), and BPTT's forward on them, mbpo_rollout_policy_general.  The pendulum's
+// policy-in-the-loop entry points stay in mbpo_b200.cu: its tcgen05 kernels include mlp_tc_kernels.cuh, whose
+// stage-4 kernel would otherwise be compiled into both units.  For the same reason (adjoint_kernels.cuh holds
+// non-template kernels) the general Systems' adjoint, mbpo_rollout_adjoint_general, sits beside the pendulum's in
+// mbpo_b200.cu.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -36,29 +39,54 @@ int launch_env_general(const GeneralEnvArgs& a, int prng_mode, cudaStream_t st) 
   });
 }
 
+// Dynamic shared memory of the CUDA-core policy kernels for a network of num_hidden layers on an X -> 2A System.
 template <class Sys>
-int launch_actor_general(const GeneralActorArgs& a, int prng_mode, cudaStream_t st) {
+GeneralActorSmem general_policy_smem(int num_hidden) {
   constexpr int X = Sys::X, A = Sys::A;
   GeneralActorSmem lay;
   int off = 0;
   auto take = [&](int n) { const int o = off; off += (n + 3) / 4 * 4; return o; };
   lay.w[0] = take(X * ACT_W);
-  for (int l = 1; l < a.num_hidden; ++l) lay.w[l] = take(ACT_W * ACT_W);
-  lay.w[a.num_hidden] = take(ACT_W * 2 * A);
-  for (int l = 0; l < a.num_hidden; ++l) lay.b[l] = take(ACT_W);
-  lay.b[a.num_hidden] = take(2 * A);
+  for (int l = 1; l < num_hidden; ++l) lay.w[l] = take(ACT_W * ACT_W);
+  lay.w[num_hidden] = take(ACT_W * 2 * A);
+  for (int l = 0; l < num_hidden; ++l) lay.b[l] = take(ACT_W);
+  lay.b[num_hidden] = take(2 * A);
   lay.h = take(ACT_W * GEN_ACT_THREADS);
   lay.total = off;
-  const size_t smem = static_cast<size_t>(off) * sizeof(float);
+  return lay;
+}
+
+// One launch of a CUDA-core policy kernel (actor_rollout_general_kernel / rollout_policy_general_kernel): E threads
+// in blocks of GEN_ACT_THREADS, with the dynamic shared memory `lay` asks for.
+template <class Kernel, class Args>
+int launch_general_policy_kernel(Kernel kernel, const char* what, const Args& a, const GeneralActorSmem& lay,
+                                 cudaStream_t st) {
+  const size_t smem = static_cast<size_t>(lay.total) * sizeof(float);
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             static_cast<int>(smem));
+  if (e != cudaSuccess) return fail(MBPO_ECUDA, "%s: smem attribute (%zu B): %s", what, smem, cudaGetErrorString(e));
+  const unsigned blocks = static_cast<unsigned>((a.E + GEN_ACT_THREADS - 1) / GEN_ACT_THREADS);
+  kernel<<<blocks, GEN_ACT_THREADS, smem, st>>>(a, lay);
+  return MBPO_OK;
+}
+
+template <class Sys>
+int launch_actor_general(const GeneralActorArgs& a, int prng_mode, cudaStream_t st) {
+  const GeneralActorSmem lay = general_policy_smem<Sys>(a.num_hidden);
   return with_prng(prng_mode, [&](auto P) {
-    auto kernel = actor_rollout_general_kernel<Sys, P>;
-    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                               static_cast<int>(smem));
-    if (e != cudaSuccess)
-      return fail(MBPO_ECUDA, "actor_rollout_general: smem attribute (%zu B): %s", smem, cudaGetErrorString(e));
-    const unsigned blocks = static_cast<unsigned>((a.E + GEN_ACT_THREADS - 1) / GEN_ACT_THREADS);
-    kernel<<<blocks, GEN_ACT_THREADS, smem, st>>>(a, lay);
-    return check_launch("actor_rollout_general_kernel");
+    const int rc = launch_general_policy_kernel(actor_rollout_general_kernel<Sys, P>, "actor_rollout_general", a,
+                                                lay, st);
+    return rc != MBPO_OK ? rc : check_launch("actor_rollout_general_kernel");
+  });
+}
+
+template <class Sys>
+int launch_rollout_policy_general(const GeneralPolicyArgs& a, int prng_mode, cudaStream_t st) {
+  const GeneralActorSmem lay = general_policy_smem<Sys>(a.num_hidden);
+  return with_prng(prng_mode, [&](auto P) {
+    const int rc = launch_general_policy_kernel(rollout_policy_general_kernel<Sys, P>, "rollout_policy_general", a,
+                                                lay, st);
+    return rc != MBPO_OK ? rc : check_launch("rollout_policy_general_kernel");
   });
 }
 
@@ -249,5 +277,58 @@ int mbpo_actor_rollout_general(int system_kind, const MbpoGeneralSystemParams* p
   a.log_prob_out = deterministic ? nullptr : log_prob_out;
   return with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
     return launch_actor_general<typename decltype(t)::type>(a, prng_mode, st);
+  });
+}
+
+int mbpo_rollout_policy_general(int system_kind, const MbpoGeneralSystemParams* params_host, int prng_mode,
+                                const MbpoPolicyParams* policy_host, int deterministic, int key_convention,
+                                const uint32_t* key_in, const uint32_t* sys_keys_in, int sys_keys_shared,
+                                const float* x0, int E, int T, float* action_out, float* reward_out,
+                                float* next_observation_out, uint32_t* key_out, uint32_t* sys_keys_out, void* stream) {
+  int X, A;
+  bool keyed;
+  int rc = collection_system("rollout_policy_general", system_kind, &X, &A, &keyed);
+  if (rc != MBPO_OK) return rc;
+  MBPO_REQUIRE(params_host && policy_host && key_in, "rollout_policy_general: null pointer");
+  MBPO_REQUIRE(prng_mode == 0 || prng_mode == 1, "rollout_policy_general: bad prng_mode %d", prng_mode);
+  MBPO_REQUIRE(key_convention >= 0 && key_convention <= 2, "rollout_policy_general: bad key_convention %d",
+               key_convention);
+  MBPO_REQUIRE(E >= 0 && T >= 0, "rollout_policy_general: negative size");
+  MBPO_REQUIRE(policy_host->head == MBPO_HEAD_NORMAL_TANH || policy_host->head == MBPO_HEAD_BPTT_ACTOR,
+               "rollout_policy_general: bad policy head %d", policy_host->head);
+  MBPO_REQUIRE(policy_host->kernel >= MBPO_ACTOR_AUTO && policy_host->kernel <= MBPO_ACTOR_TCGEN05_WIDE,
+               "rollout_policy_general: bad policy kernel selector %d", policy_host->kernel);
+  if (policy_host->kernel == MBPO_ACTOR_TCGEN05 || policy_host->kernel == MBPO_ACTOR_TCGEN05_WIDE)
+    return fail(MBPO_EUNSUPPORTED, "rollout_policy_general: the tcgen05 policy kernels hold the pendulum only; the "
+                "general Systems run the CUDA-core kernel (MBPO_ACTOR_AUTO or MBPO_ACTOR_CUDA_CORES)");
+  GeneralPolicyArgs a;
+  rc = fill_policy("rollout_policy_general", policy_host, E, X, A, a);
+  if (rc != MBPO_OK) return rc;
+  const size_t sys_key_words = keyed ? (sys_keys_shared ? 2 : 2 * static_cast<size_t>(E)) : 0;
+  MBPO_REQUIRE(sys_key_words == 0 || (sys_keys_in && sys_keys_out),
+               "rollout_policy_general: this System draws from system_params.key: sys_keys_in / sys_keys_out are "
+               "null");
+  cudaStream_t st = as_stream(stream);
+  if (E == 0 || T == 0) {        // empty arrays have no address; keys pass through
+    int r = copy_async(key_out, key_in, key_out ? 2 * sizeof(uint32_t) : 0, st, "rollout_policy_general");
+    if (r == MBPO_OK) r = copy_async(sys_keys_out, sys_keys_in, sizeof(uint32_t) * sys_key_words, st,
+                                     "rollout_policy_general");
+    return r;
+  }
+  MBPO_REQUIRE(x0 && action_out && reward_out && next_observation_out, "rollout_policy_general: null pointer");
+  MBPO_REQUIRE(X != 4 || aligned16(next_observation_out),
+               "rollout_policy_general: next_observation_out of a 4-float state must be 16-byte aligned");
+  a.sys = *params_host;
+  a.E = E; a.T = T;
+  a.deterministic = deterministic; a.key_convention = key_convention;
+  a.head = policy_host->head; a.shared_noise = policy_host->shared_noise;
+  a.sig_bias = policy_host->sig_bias; a.sig_min = policy_host->sig_min; a.sig_max = policy_host->sig_max;
+  a.action_clip = policy_host->action_clip;
+  a.key_in = key_in; a.key_out = key_out;
+  a.x0 = x0;
+  a.sys_keys_in = sys_keys_in; a.sys_keys_out = sys_keys_out; a.sys_keys_shared = sys_keys_shared ? 1 : 0;
+  a.action_out = action_out; a.reward_out = reward_out; a.next_observation_out = next_observation_out;
+  return with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    return launch_rollout_policy_general<typename decltype(t)::type>(a, prng_mode, st);
   });
 }

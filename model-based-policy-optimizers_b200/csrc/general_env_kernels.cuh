@@ -12,6 +12,8 @@
 // One thread per env, state and keys in registers.  The observation rows leave through the warp transposes of
 // env_kernels.cuh (X = 3) or as one 16-byte store per env (X = 4).  env_unroll_general_kernel also serves the
 // pendulum's env rollouts whose Transition buffers are not all present (collection.cu launch_env).
+// rollout_policy_general_kernel is BPTT's forward on the same policy network: the plain scan of rollout_policy
+// (no wrapper), with BPTT's actor head.
 #pragma once
 #include "actor_kernels.cuh"
 #include "systems.cuh"
@@ -180,6 +182,84 @@ struct GeneralActorSmem {
   int w[ACT_MAX_HIDDEN + 1], b[ACT_MAX_HIDDEN + 1], h, total;
 };
 
+// The policy's weights and biases into shared memory at `lay`, the normaliser's statistics into norm_sm (mean
+// [0..3], std [4..7]); every thread of the block takes part, and a barrier must follow.  Args is GeneralActorArgs or
+// GeneralPolicyArgs.
+template <int X, int A, class Args>
+__device__ __forceinline__ void load_general_policy(const Args& a, const GeneralActorSmem& lay, float* gsm,
+                                                    float* norm_sm, int tid, int nthr) {
+  if (tid < X) {
+    norm_sm[tid] = a.obs_mean_dev ? a.obs_mean_dev[tid] : a.obs_mean[tid];
+    norm_sm[4 + tid] = a.obs_std_dev ? a.obs_std_dev[tid] : a.obs_std[tid];
+  }
+  const int L = a.num_hidden;
+  for (int i = tid; i < X * ACT_W; i += nthr) gsm[lay.w[0] + i] = a.w[0][i];
+  for (int l = 1; l < L; ++l)
+    for (int i = tid; i < ACT_W * ACT_W; i += nthr) gsm[lay.w[l] + i] = a.w[l][i];
+  for (int i = tid; i < ACT_W * 2 * A; i += nthr) gsm[lay.w[L] + i] = a.w[L][i];
+  for (int l = 0; l < L; ++l)
+    for (int i = tid; i < ACT_W; i += nthr) gsm[lay.b[l] + i] = a.b[l][i];
+  if (tid < 2 * A) gsm[lay.b[L] + tid] = a.b[L][tid];
+}
+
+// The policy network on one thread's state x: the normaliser (x - mean) / std when a.normalize, then the MLP in
+// float32 on the CUDA cores (swish), whose hidden layers pass through the thread's shared-memory column h_col, and
+// the 2A logits (loc / mu first, then the raw scale) with their biases added.  gsm holds the weights at `lay`,
+// norm_sm the normaliser's mean [0..3] and std [4..7].
+template <int X, int A, class Args>
+__device__ __forceinline__ void general_policy_logits(const Args& a, const float (&x)[X], const float* gsm,
+                                                      const GeneralActorSmem& lay, const float* norm_sm,
+                                                      float* h_col, int nthr, float (&logits)[2 * A]) {
+  float xin[X];
+#pragma unroll
+  for (int i = 0; i < X; ++i)
+    xin[i] = a.normalize ? __fdiv_rn(__fsub_rn(x[i], norm_sm[i]), norm_sm[4 + i]) : x[i];
+  float h[ACT_W];
+  {
+    const float* w0 = gsm + lay.w[0];   // [X][64]
+    const float* b0 = gsm + lay.b[0];
+#pragma unroll
+    for (int j = 0; j < ACT_W; ++j) {
+      float acc = xin[0] * w0[j];
+#pragma unroll
+      for (int i = 1; i < X; ++i) acc = fmaf(xin[i], w0[i * ACT_W + j], acc);
+      h[j] = swish_exact(acc + b0[j]);
+    }
+  }
+#pragma unroll 1
+  for (int l = 1; l < a.num_hidden; ++l) {
+    const float* wl = gsm + lay.w[l];
+    const float* bl = gsm + lay.b[l];
+#pragma unroll 1
+    for (int jc = 0; jc < ACT_W / 8; ++jc) {
+      float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      const float4* wrow = reinterpret_cast<const float4*>(wl + jc * 8);
+#pragma unroll
+      for (int k = 0; k < ACT_W; ++k) {
+        const float4 wa = wrow[k * (ACT_W / 4)], wb = wrow[k * (ACT_W / 4) + 1];
+        acc[0] = fmaf(h[k], wa.x, acc[0]); acc[1] = fmaf(h[k], wa.y, acc[1]);
+        acc[2] = fmaf(h[k], wa.z, acc[2]); acc[3] = fmaf(h[k], wa.w, acc[3]);
+        acc[4] = fmaf(h[k], wb.x, acc[4]); acc[5] = fmaf(h[k], wb.y, acc[5]);
+        acc[6] = fmaf(h[k], wb.z, acc[6]); acc[7] = fmaf(h[k], wb.w, acc[7]);
+      }
+#pragma unroll
+      for (int i = 0; i < 8; ++i) h_col[(jc * 8 + i) * nthr] = swish_exact(acc[i] + bl[jc * 8 + i]);
+    }
+#pragma unroll
+    for (int k = 0; k < ACT_W; ++k) h[k] = h_col[k * nthr];
+  }
+  const float* wo = gsm + lay.w[a.num_hidden];   // [64][2A]
+  const float* bo = gsm + lay.b[a.num_hidden];
+#pragma unroll
+  for (int j = 0; j < 2 * A; ++j) logits[j] = 0.0f;
+#pragma unroll
+  for (int k = 0; k < ACT_W; ++k)
+#pragma unroll
+    for (int j = 0; j < 2 * A; ++j) logits[j] = fmaf(h[k], wo[k * 2 * A + j], logits[j]);
+#pragma unroll
+  for (int j = 0; j < 2 * A; ++j) logits[j] += bo[j];
+}
+
 // T steps of actor_step for E envs: policy MLP (float32 on the CUDA cores), NormalTanh sample, the wrapped env step
 // with the System's key, Transition out.  One thread per env; the activations of the current layer live in
 // registers, the next layer's pass through the thread's own shared-memory column.
@@ -191,20 +271,7 @@ __global__ void __launch_bounds__(GEN_ACT_THREADS) actor_rollout_general_kernel(
   __shared__ float tiles[GEN_ACT_THREADS / 32][96];
   __shared__ float norm_sm[8];     // normaliser mean [0..3], std [4..7]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = blockDim.x;
-  if (tid < X) {
-    norm_sm[tid] = a.obs_mean_dev ? a.obs_mean_dev[tid] : a.obs_mean[tid];
-    norm_sm[4 + tid] = a.obs_std_dev ? a.obs_std_dev[tid] : a.obs_std[tid];
-  }
-  {
-    const int L = a.num_hidden;
-    for (int i = tid; i < X * ACT_W; i += nthr) gsm[lay.w[0] + i] = a.w[0][i];
-    for (int l = 1; l < L; ++l)
-      for (int i = tid; i < ACT_W * ACT_W; i += nthr) gsm[lay.w[l] + i] = a.w[l][i];
-    for (int i = tid; i < ACT_W * 2 * A; i += nthr) gsm[lay.w[L] + i] = a.w[L][i];
-    for (int l = 0; l < L; ++l)
-      for (int i = tid; i < ACT_W; i += nthr) gsm[lay.b[l] + i] = a.b[l][i];
-    if (tid < 2 * A) gsm[lay.b[L] + tid] = a.b[L][tid];
-  }
+  load_general_policy<X, A>(a, lay, gsm, norm_sm, tid, nthr);
   __syncthreads();
   const int e = blockIdx.x * nthr + tid;
   const int warp_e0 = e - lane;
@@ -239,57 +306,8 @@ __global__ void __launch_bounds__(GEN_ACT_THREADS) actor_rollout_general_kernel(
       else { k_actor = first_k; key = second_k; }
     }
     // ---- policy network --------------------------------------------------------------------------------------
-    float xin[X];
-#pragma unroll
-    for (int i = 0; i < X; ++i)
-      xin[i] = a.normalize ? __fdiv_rn(__fsub_rn(x[i], norm_sm[i]), norm_sm[4 + i]) : x[i];
-    float h[ACT_W];
-    {
-      const float* w0 = gsm + lay.w[0];   // [X][64]
-      const float* b0 = gsm + lay.b[0];
-#pragma unroll
-      for (int j = 0; j < ACT_W; ++j) {
-        float acc = xin[0] * w0[j];
-#pragma unroll
-        for (int i = 1; i < X; ++i) acc = fmaf(xin[i], w0[i * ACT_W + j], acc);
-        h[j] = swish_exact(acc + b0[j]);
-      }
-    }
-#pragma unroll 1
-    for (int l = 1; l < a.num_hidden; ++l) {
-      const float* wl = gsm + lay.w[l];
-      const float* bl = gsm + lay.b[l];
-#pragma unroll 1
-      for (int jc = 0; jc < ACT_W / 8; ++jc) {
-        float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        const float4* wrow = reinterpret_cast<const float4*>(wl + jc * 8);
-#pragma unroll
-        for (int k = 0; k < ACT_W; ++k) {
-          const float4 wa = wrow[k * (ACT_W / 4)], wb = wrow[k * (ACT_W / 4) + 1];
-          acc[0] = fmaf(h[k], wa.x, acc[0]); acc[1] = fmaf(h[k], wa.y, acc[1]);
-          acc[2] = fmaf(h[k], wa.z, acc[2]); acc[3] = fmaf(h[k], wa.w, acc[3]);
-          acc[4] = fmaf(h[k], wb.x, acc[4]); acc[5] = fmaf(h[k], wb.y, acc[5]);
-          acc[6] = fmaf(h[k], wb.z, acc[6]); acc[7] = fmaf(h[k], wb.w, acc[7]);
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) h_col[(jc * 8 + i) * nthr] = swish_exact(acc[i] + bl[jc * 8 + i]);
-      }
-#pragma unroll
-      for (int k = 0; k < ACT_W; ++k) h[k] = h_col[k * nthr];
-    }
     float logits[2 * A];
-    {
-      const float* wo = gsm + lay.w[a.num_hidden];   // [64][2A]
-      const float* bo = gsm + lay.b[a.num_hidden];
-#pragma unroll
-      for (int j = 0; j < 2 * A; ++j) logits[j] = 0.0f;
-#pragma unroll
-      for (int k = 0; k < ACT_W; ++k)
-#pragma unroll
-        for (int j = 0; j < 2 * A; ++j) logits[j] = fmaf(h[k], wo[k * 2 * A + j], logits[j]);
-#pragma unroll
-      for (int j = 0; j < 2 * A; ++j) logits[j] += bo[j];
-    }
+    general_policy_logits<X, A>(a, x, gsm, lay, norm_sm, h_col, nthr, logits);
     // ---- NormalTanh head (actor_kernels.cuh actor_head), A dims ----------------------------------------------
     const size_t row = static_cast<size_t>(t) * E;
     float u[A], log_prob = 0.0f;
@@ -334,6 +352,118 @@ __global__ void __launch_bounds__(GEN_ACT_THREADS) actor_rollout_general_kernel(
     a.steps[e] = steps;
     a.done[e] = done;
     if (Sys::KEYED) { a.sys_keys_out[2 * e] = skey.k0; a.sys_keys_out[2 * e + 1] = skey.k1; }
+  }
+  if (blockIdx.x == 0 && tid == 0 && a.key_out) { a.key_out[0] = key.k0; a.key_out[1] = key.k1; }
+}
+
+struct GeneralPolicyArgs {
+  MbpoGeneralSystemParams sys;
+  int E, T;
+  int num_hidden, deterministic, key_convention;   // MBPO_KEYS_*
+  float min_std;
+  int head, shared_noise, normalize;               // MBPO_HEAD_*
+  int draw_offset, draw_total;   // env sharding of the NormalTanh draw normal(key, (draw_total, A))
+  float sig_bias, sig_min, sig_max, action_clip;   // the BPTT head
+  float obs_mean[4], obs_std[4];
+  const float* obs_mean_dev;     // device-resident statistics (override obs_mean / obs_std when non-null)
+  const float* obs_std_dev;
+  const float* w[ACT_MAX_HIDDEN + 1];   // as GeneralActorArgs
+  const float* b[ACT_MAX_HIDDEN + 1];
+  const uint32_t* key_in;        // [2] the policy's carry key
+  uint32_t* key_out;             // [2]
+  const float* x0;               // [E,X]
+  const uint32_t* sys_keys_in;   // keyed Systems: [2] (sys_keys_shared) or [E,2]
+  uint32_t* sys_keys_out;        // same shape
+  int sys_keys_shared;
+  float* action_out;             // [T,E,A]
+  float* reward_out;             // [T,E]
+  float* next_observation_out;   // [T,E,X]
+};
+
+// rollout_policy (optimizer_utils.py:62-116) for E trajectories of T steps: per step the policy network (as
+// actor_rollout_general_kernel), its head, then the plain System.step -- no Episode / AutoReset wrapper, so no step
+// counter, done or truncation.  The head is BPTT's actor (bptt_optimizer.py:137-142,306-326: sig = clip(softplus(sig
+// + sig_bias), sig_min, sig_max), a = clip(tanh(mu + eps * sig), +-action_clip), clip(tanh(mu)) when deterministic)
+// or SAC's NormalTanh; with shared_noise the draw is normal(k_actor, (A,)), the same for every trajectory.  A keyed
+// System's key is per trajectory or one shared by all; a shared key advances identically in every thread.
+template <class Sys, int PRNG>
+__global__ void __launch_bounds__(GEN_ACT_THREADS) rollout_policy_general_kernel(const __grid_constant__ GeneralPolicyArgs a,
+                                                                                const GeneralActorSmem lay) {
+  constexpr int X = Sys::X, A = Sys::A;
+  extern __shared__ __align__(16) float gsm[];
+  __shared__ float tiles[GEN_ACT_THREADS / 32][96];
+  __shared__ float norm_sm[8];     // normaliser mean [0..3], std [4..7]
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = blockDim.x;
+  load_general_policy<X, A>(a, lay, gsm, norm_sm, tid, nthr);
+  __syncthreads();
+  const int e = blockIdx.x * nthr + tid;
+  const int warp_e0 = e - lane;
+  if (warp_e0 >= a.E) return;
+  const bool live = e < a.E;
+  const int ee = live ? e : a.E - 1;
+  const int n_valid = min(a.E - warp_e0, 32);
+  float* tile = tiles[warp];
+  float* h_col = gsm + lay.h + tid;
+  const Sys sys(a.sys);
+  float x[X];
+#pragma unroll
+  for (int k = 0; k < X; ++k) x[k] = a.x0[static_cast<size_t>(ee) * X + k];
+  Key2 skey{0u, 0u};
+  if (Sys::KEYED) {
+    const int ks = a.sys_keys_shared ? 0 : ee;
+    skey = Key2{a.sys_keys_in[2 * ks], a.sys_keys_in[2 * ks + 1]};
+  }
+  Key2 key{a.key_in[0], a.key_in[1]};
+  const size_t E = static_cast<size_t>(a.E);
+  const bool bptt = a.head == MBPO_HEAD_BPTT_ACTOR;
+  const uint32_t n_draw = a.shared_noise ? static_cast<uint32_t>(A) : static_cast<uint32_t>(a.draw_total) * A;
+  const uint32_t i_draw0 = a.shared_noise ? 0u : static_cast<uint32_t>(a.draw_offset + ee) * A;
+
+#pragma unroll 1
+  for (int t = 0; t < a.T; ++t) {
+    // ---- key plumbing (actor_kernels.cuh): BPTT.act splits as MBPO_KEYS_UNROLL, evaluate keeps it as is ----------
+    Key2 k_actor = key;
+    if (a.key_convention != MBPO_KEYS_AS_IS) {
+      Key2 first_k, second_k;
+      split2<PRNG>(key, first_k, second_k);
+      if (a.key_convention == MBPO_KEYS_SAC) { key = first_k; k_actor = second_k; }
+      else { k_actor = first_k; key = second_k; }
+    }
+    float logits[2 * A];
+    general_policy_logits<X, A>(a, x, gsm, lay, norm_sm, h_col, nthr, logits);
+    // ---- the head, A dims ----------------------------------------------------------------------------------------
+    float u[A];
+#pragma unroll
+    for (int j = 0; j < A; ++j) {
+      const float mu = logits[j];
+      const float eps = a.deterministic ? 0.0f : bits_to_normal(random_bits_at<PRNG>(k_actor, n_draw, i_draw0 + j));
+      if (bptt) {
+        float pre = mu;
+        if (!a.deterministic) {
+          const float sig = fminf(fmaxf(softplus_exact(__fadd_rn(logits[A + j], a.sig_bias)), a.sig_min), a.sig_max);
+          pre = __fadd_rn(pre, __fmul_rn(eps, sig));
+        }
+        u[j] = fminf(fmaxf(tanhf(pre), -a.action_clip), a.action_clip);
+      } else if (a.deterministic) {
+        u[j] = tanhf(mu);
+      } else {
+        const float scale = softplus_exact(logits[A + j]) + a.min_std;
+        u[j] = tanhf(__fadd_rn(__fmul_rn(scale, eps), mu));
+      }
+    }
+    // ---- System.step ------------------------------------------------------------------------------------------
+    const size_t row = static_cast<size_t>(t) * E;
+    const float rew = sys.template step<PRNG>(x, u, 1, skey);
+    store_obs_row<X>(tile, a.next_observation_out, row + warp_e0, lane, live, n_valid, x);
+    if (live) {
+#pragma unroll
+      for (int j = 0; j < A; ++j) a.action_out[(row + e) * A + j] = u[j];
+      a.reward_out[row + e] = rew;
+    }
+  }
+  if (Sys::KEYED && (a.sys_keys_shared ? e == 0 : live)) {
+    a.sys_keys_out[2 * e] = skey.k0;
+    a.sys_keys_out[2 * e + 1] = skey.k1;
   }
   if (blockIdx.x == 0 && tid == 0 && a.key_out) { a.key_out[0] = key.k0; a.key_out[1] = key.k1; }
 }

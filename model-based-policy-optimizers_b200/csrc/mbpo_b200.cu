@@ -973,6 +973,36 @@ int mbpo_rollout_adjoint(int system_kind, const void* sys_params_host, int x_dim
   return check_launch("rollout_adjoint_pendulum_kernel");
 }
 
+int mbpo_rollout_adjoint_general(int system_kind, const MbpoGeneralSystemParams* params_host, int E, int T,
+                                 long long stride_t, long long stride_e, long long stride_xt, long long stride_xe,
+                                 long long stride_at, long long stride_ae, const float* observation,
+                                 const float* action, const float* g_reward, const float* g_next_obs,
+                                 const float* g_obs, const float* g_action_in, float* g_action_out, float* g_x0_out,
+                                 void* stream) {
+  if (system_kind == MBPO_SYSTEM_PENDULUM)
+    return fail(MBPO_EINVAL, "rollout_adjoint_general: MBPO_SYSTEM_PENDULUM has its own entry point "
+                "(mbpo_rollout_adjoint)");
+  int X, A;
+  bool keyed;
+  if (general_system_dims(system_kind, &X, &A, &keyed) != MBPO_OK)
+    return fail(MBPO_EUNSUPPORTED, "rollout_adjoint_general: system_kind %d is not one of the general Systems "
+                "(NOISY_PENDULUM, POINT_MASS)", system_kind);
+  MBPO_REQUIRE(E >= 0 && T >= 0, "rollout_adjoint_general: negative size");
+  if (E == 0) return MBPO_OK;
+  MBPO_REQUIRE(params_host && (T == 0 || (observation && action && g_action_out)),   // T == 0: only g_x0_out
+               "rollout_adjoint_general: null pointer");
+  mbpo::AdjointGeneralArgs a;
+  a.sys = *params_host;
+  a.E = E; a.T = T; a.st_t = stride_t; a.st_e = stride_e; a.sx_t = stride_xt; a.sx_e = stride_xe;
+  a.sa_t = stride_at; a.sa_e = stride_ae;
+  a.observation = observation; a.action = action; a.g_reward = g_reward; a.g_next_obs = g_next_obs;
+  a.g_obs = g_obs; a.g_action_in = g_action_in; a.g_action_out = g_action_out; a.g_x0_out = g_x0_out;
+  return with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    mbpo::rollout_adjoint_general_kernel<typename decltype(t)::type><<<(E + 127) / 128, 128, 0, as_stream(stream)>>>(a);
+    return check_launch("rollout_adjoint_general_kernel");
+  });
+}
+
 extern "C++" {
 namespace {
 mbpo::LambdaArgs lambda_args(int E, int T, long long stride_t, long long stride_e, double discount, double lambda_) {

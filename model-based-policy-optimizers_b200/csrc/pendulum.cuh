@@ -125,4 +125,48 @@ __device__ __forceinline__ void pendulum_step_theta(const PendulumConsts& p, flo
   w = nw;
 }
 
+// jnp.clip = minimum(maximum(x, lo), hi): lax.max / lax.min split the cotangent evenly at a tie.
+__device__ __forceinline__ float clip_grad(float x, float lo, float hi) {
+  const float a = (x > lo) ? 1.0f : (x == lo ? 0.5f : 0.0f);          // d max(x, lo) / dx
+  const float m = fmaxf(x, lo);
+  const float b = (m < hi) ? 1.0f : (m == hi ? 0.5f : 0.0f);          // d min(m, hi) / dm
+  return a * b;
+}
+
+// Cotangents of one pendulum System.step at state [c, s, w] and action u (the 3 x 3 Jacobian-transpose products
+// written out for pendulum_dynamics.py:29-63 and pendulum_reward.py:27-42), re-deriving the step's intermediates:
+// [gc, gs, gw] is the cotangent of x_next, gr that of the reward; out come the cotangent [lc, ls, lw] of the state
+// and g_u of the action.  [c, s] need not be a unit vector: the atan2 derivative divides by c^2 + s^2.
+__device__ __forceinline__ void pendulum_step_vjp(const PendulumConsts& pc, float c, float s, float w, float u,
+                                                  float gc, float gs, float gw, float gr, float& lc, float& ls,
+                                                  float& lw, float& g_u) {
+  // forward intermediates of this step (pendulum_dynamics.py:35,59-62,40,43)
+  const float th = atan2_bounded(s, c);
+  float sin_th, cos_th;
+  sincos_bounded(th, sin_th, cos_th);
+  const float uu = __fmul_rn(fminf(fmaxf(u, -1.0f), 1.0f), pc.max_torque);
+  const float thdd = fmaf(pc.c_g, sin_th, __fmul_rn(pc.c_u, uu));
+  const float v = fmaf(thdd, pc.dt, w);
+  const float nw = fminf(fmaxf(v, -pc.max_speed), pc.max_speed);
+  const float nth = fmaf(nw, pc.dt, th);
+  float sn, cn;
+  sincos_bounded(nth, sn, cn);
+  // x_next = [cos(nth), sin(nth), nw]
+  const float g_nth = cn * gs - sn * gc;
+  const float g_nw = gw + pc.dt * g_nth;
+  const float g_v = g_nw * clip_grad(v, -pc.max_speed, pc.max_speed);
+  const float g_thdd = pc.dt * g_v;
+  // reward on (x_t, a_t) (pendulum_reward.py:32-39); d/dth of the wrapped difference is 1
+  const float diff = wrap_diff(th - pc.target_angle);
+  float g_th = g_nth + g_thdd * pc.c_g * cos_th - gr * 2.0f * pc.angle_cost * diff;
+  const float g_w = g_v - gr * 0.2f * w;
+  g_u = g_thdd * pc.c_u * pc.max_torque * clip_grad(u, -1.0f, 1.0f) - gr * 2.0f * pc.control_cost * u;
+  // th = atan2(s, c): dth/dc = -s / (c^2 + s^2), dth/ds = c / (c^2 + s^2)
+  const float r2 = c * c + s * s;
+  const float inv = r2 > 0.0f ? 1.0f / r2 : 0.0f;
+  lc = -g_th * s * inv;
+  ls = g_th * c * inv;
+  lw = g_w;
+}
+
 }  // namespace mbpo

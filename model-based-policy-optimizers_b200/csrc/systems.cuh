@@ -69,6 +69,13 @@ struct NoisyPendulumSys {
     key = next;
     return r;
   }
+  // Cotangents of step: g_next of x_next, g_r of the reward -> g_x, g_u.  The noise is added to the mean and
+  // depends on neither x nor u, so the Jacobians are the pendulum's at the stored (noisy) state.
+  __device__ __forceinline__ void step_vjp(const float (&x)[X], const float (&u)[A], const float (&g_next)[X],
+                                           float g_r, float (&g_x)[X], float (&g_u)[A]) const {
+    pendulum_step_vjp(pc, x[0], x[1], x[2], u[0], g_next[0], g_next[1], g_next[2], g_r, g_x[0], g_x[1], g_x[2],
+                      g_u[0]);
+  }
 };
 
 struct PointMassSys {
@@ -93,6 +100,22 @@ struct PointMassSys {
     x[2] = v0;
     x[3] = v1;
     return reward;
+  }
+  // Cotangents of step, per axis k with pre = v + a dt: g_v' = g_next_v + dt g_next_p; g_pre = g_v' clip'(pre);
+  // g_v = g_pre - g_r 2 speed_cost v; g_p = g_next_p - g_r 2 (p - target);
+  // g_u = g_pre dt max_accel clip'(u) - g_r 2 control_cost u.
+  __device__ __forceinline__ void step_vjp(const float (&x)[X], const float (&u)[A], const float (&g_next)[X],
+                                           float g_r, float (&g_x)[X], float (&g_u)[A]) const {
+    const float target[2] = {p.target_x, p.target_y};
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const float ak = __fmul_rn(fminf(fmaxf(u[k], -1.0f), 1.0f), p.max_accel);
+      const float pre = __fadd_rn(x[2 + k], __fmul_rn(ak, p.dt));                // as step rounds it: same clip ties
+      const float g_pre = (g_next[2 + k] + p.dt * g_next[k]) * clip_grad(pre, -p.max_speed, p.max_speed);
+      g_x[k] = g_next[k] - g_r * 2.0f * (x[k] - target[k]);
+      g_x[2 + k] = g_pre - g_r * 2.0f * p.speed_cost * x[2 + k];
+      g_u[k] = g_pre * p.dt * p.max_accel * clip_grad(u[k], -1.0f, 1.0f) - g_r * 2.0f * p.control_cost * u[k];
+    }
   }
 };
 

@@ -148,7 +148,11 @@ SIGNATURES = {
                                      _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_actor_rollout_general": (_I, [_I, C.POINTER(GeneralSystemParamsC), _I, C.POINTER(PolicyParamsC), _I, _I, _P,
                                         _I, _I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "mbpo_rollout_policy_general": (_I, [_I, C.POINTER(GeneralSystemParamsC), _I, C.POINTER(PolicyParamsC), _I, _I,
+                                         _P, _P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_rollout_adjoint": (_I, [_I, _P, _I, _I, _I, _I, _LL, _LL, _LL, _LL, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "mbpo_rollout_adjoint_general": (_I, [_I, C.POINTER(GeneralSystemParamsC), _I, _I, _LL, _LL, _LL, _LL, _LL, _LL,
+                                          _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mbpo_lambda_return": (_I, [_P, _P, _I, _I, _LL, _LL, C.c_double, C.c_double, _P, _P]),
     "mbpo_lambda_return_vjp": (_I, [_P, _I, _I, _LL, _LL, C.c_double, C.c_double, _P, _P, _P]),
     "mbpo_mlp_dynamics_forward": (_I, [C.POINTER(MlpEnsembleParamsC), _P, _P, _I, _P, _P]),

@@ -6,9 +6,10 @@ fields.  Batched forms replace ``jax.vmap(rollout_actions)``:
     init_state [B,X], actions [B, M, H, A]  -> fields [B, M, H, ...]  (M sequences per state)
 
 rollout_policy (optimizer_utils.py:62-116) runs the policy inside the horizon loop in one kernel launch
-(mbpo_actor_rollout); ``rollout_policy_vjp`` is the cotangent pass jax.grad takes through it with
-stop_grads=True (mbpo_rollout_adjoint), ``lambda_return`` / ``lambda_return_vjp`` the Dreamer lambda return
-(:119-131) and its transpose.
+(mbpo_actor_rollout; mbpo_rollout_policy_general for NoisyPendulumSystem / PointMassSystem); ``rollout_policy_vjp``
+is the cotangent pass jax.grad takes through it with stop_grads=True (mbpo_rollout_adjoint /
+mbpo_rollout_adjoint_general), ``lambda_return`` / ``lambda_return_vjp`` the Dreamer lambda return (:119-131) and
+its transpose.
 """
 from __future__ import annotations
 
@@ -87,9 +88,14 @@ def rollout_policy(system: System, system_params: SystemParams, init_state: torc
     init_state [B, X] -> fields [B, H, ...] (vmap over init_state with the policy state shared, as
     bptt_optimizer.py:366-368).  The fields are strided views of time-major buffers.  The carried key is returned
     in ``extras['policy_state_key']``.  stop_grads=False (policy differentiated w.r.t. its observation) is not
-    what BPTT uses (:337) and has no kernel."""
+    what BPTT uses (:337) and has no kernel.
+
+    NoisyPendulumSystem / PointMassSystem run mbpo_rollout_policy_general.  A keyed System's ``system_params.key``
+    is either [2], one key every trajectory steps with (BPTT vmaps over initial states only, so its system_params
+    are unbatched and every trajectory sees the same noise), or [B, 2], one per trajectory; the advanced key comes
+    back in the same shape in ``extras['system_params']``."""
     from .. import acting
-    from ..envs import VmappedSystemEnv
+    from ..envs import VmappedSystemEnv, is_general
     if not stop_grads:
         raise _lib.MbpoUnsupported(_lib.MBPO_EUNSUPPORTED, "rollout_policy: only stop_grads=True has a CUDA path")
     if not isinstance(policy, acting.Policy):
@@ -98,14 +104,51 @@ def rollout_policy(system: System, system_params: SystemParams, init_state: torc
     single = init_state.dim() == 1
     x0 = init_state.reshape(1, -1) if single else init_state
     key = policy_state.key if hasattr(policy_state, "key") else policy_state
-    env = VmappedSystemEnv(system, system_params, episode_length=1 << 30)      # no Episode / AutoReset wrapper here
     # act(evaluate=False) splits the key every step (sample_key, key = split(key, 2), :321-323); evaluate leaves it
     convention = _lib.KEYS_AS_IS if policy.deterministic else _lib.KEYS_UNROLL
-    _, tr, key_out = acting._rollout(env, env.reset(x0), policy, key, int(horizon), convention, ())
-    fields = [f.transpose(0, 1) for f in (tr.observation, tr.action, tr.reward, tr.discount, tr.next_observation)]
+    if is_general(system):
+        fields, extras = _rollout_policy_general(system, system_params, x0, policy, key, int(horizon), convention)
+    else:
+        env = VmappedSystemEnv(system, system_params, episode_length=1 << 30)  # no Episode / AutoReset wrapper here
+        _, tr, key_out = acting._rollout(env, env.reset(x0), policy, key, int(horizon), convention, ())
+        fields = (tr.observation, tr.action, tr.reward, tr.discount, tr.next_observation)
+        extras = {"policy_state_key": key_out}
+    fields = [f.transpose(0, 1) for f in fields]
     if single:
         fields = [f[0] for f in fields]
-    return Transition(*fields, extras={"policy_state_key": key_out})
+    return Transition(*fields, extras=extras)
+
+
+def _rollout_policy_general(system: System, system_params: SystemParams, x0: torch.Tensor, policy, key: torch.Tensor,
+                            T: int, convention: int):
+    """rollout_policy's launch for a general System: time-major fields [T, E, ...] and the extras."""
+    from ..envs import system_keys
+    X, A = system.x_dim, system.u_dim
+    x0 = x0.to(torch.float32)
+    E = x0.shape[0]
+    dev = x0.device
+    sys_key = None if system_params is None else system_params.key
+    shared = bool(system.keyed) and sys_key is not None and sys_key.dim() == 1
+    sys_keys = system_keys(system, system_params, 1 if shared else E)
+    sys_keys_out = torch.empty_like(sys_keys) if sys_keys is not None else None
+    key = key.reshape(2).contiguous()
+    key_out = torch.empty_like(key)
+    buf = torch.empty((T + 1, E, X), dtype=torch.float32, device=dev)       # observation / next_observation views
+    buf[0].copy_(x0)
+    act = torch.empty((T, E, A), dtype=torch.float32, device=dev)
+    rew = torch.empty((T, E), dtype=torch.float32, device=dev)
+    params = system.pack_params(system_params)
+    policy.struct.draw_total = policy.struct.draw_offset = 0                 # the launch owns every trajectory
+    with _lib.cuda_guard(x0):
+        _lib.check(_lib.lib.mbpo_rollout_policy_general(
+            system.system_kind, _lib.C.byref(params), config.prng_mode, _lib.C.byref(policy.struct),
+            int(policy.deterministic), convention, _lib.ptr(key), _lib.ptr(sys_keys), int(shared), _lib.ptr(buf[0]),
+            E, T, _lib.ptr(act), _lib.ptr(rew), _lib.ptr(buf[1:]), _lib.ptr(key_out), _lib.ptr(sys_keys_out),
+            _lib.stream_ptr(dev)))
+    extras = {"policy_state_key": key_out}
+    if sys_keys_out is not None:
+        extras["system_params"] = system_params.replace(key=sys_keys_out.reshape(sys_key.shape))
+    return (buf[:T], act, rew, torch.ones_like(rew), buf[1:]), extras
 
 
 def _strides(t: torch.Tensor, per_step_dims: int) -> Tuple[int, int]:
@@ -123,7 +166,9 @@ def rollout_policy_vjp(system: System, system_params: SystemParams, trajectory: 
     (bptt_optimizer.py:361-376).  trajectory: the [B, H, ...] Transition ``rollout_policy`` returned; g_*: the
     cotangents of its fields (None = zero), same shapes.  Returns (g_action_total [B, H, A], g_init_state [B, X]).
     g_action_total[b, t] is what reaches a_t = policy(stop_gradient(obs_t)); the parameter gradient is one
-    batched backward of the policy network over all (obs_t, g_action_total_t) rows."""
+    batched backward of the policy network over all (obs_t, g_action_total_t) rows.  For NoisyPendulumSystem /
+    PointMassSystem (mbpo_rollout_adjoint_general) the [B, H, A] arrays have their own stride pair."""
+    from ..envs import is_general
     obs, act = trajectory.observation, trajectory.action
     B, H, X = obs.shape
     A = act.shape[-1]
@@ -139,6 +184,27 @@ def rollout_policy_vjp(system: System, system_params: SystemParams, trajectory: 
             buf.copy_(t)
             t = buf
         return t
+
+    def p(t):
+        return None if t is None else t.data_ptr()
+    params = system.pack_params(system_params)
+    if is_general(system):
+        act = act.to(torch.float32)
+        if act.stride(-1) != 1:
+            act = act.contiguous()
+        g_act_out = torch.empty_strided(act.shape, act.stride(), dtype=torch.float32, device=dev)
+        g_x0 = torch.empty((B, X), dtype=torch.float32, device=dev)
+        g_r = like(trajectory.reward, g_reward)
+        g_n, g_o = like(obs, g_next_observation), like(obs, g_observation)
+        g_a = like(act, g_action)
+        st_t, st_e = _strides(trajectory.reward, 0)
+        sx_t, sx_e = _strides(obs, 1)
+        sa_t, sa_e = _strides(act, 1)
+        with _lib.cuda_guard(obs):
+            _lib.check(_lib.lib.mbpo_rollout_adjoint_general(
+                system.system_kind, _lib.C.byref(params), B, H, st_t, st_e, sx_t, sx_e, sa_t, sa_e, p(obs), p(act),
+                p(g_r), p(g_n), p(g_o), p(g_a), p(g_act_out), p(g_x0), _lib.stream_ptr(dev)))
+        return g_act_out, g_x0
     rew_like = trajectory.reward
     if act.reshape(B, H).stride() != rew_like.stride():
         rew_like = act.reshape(B, H)
@@ -151,10 +217,6 @@ def rollout_policy_vjp(system: System, system_params: SystemParams, trajectory: 
     g_x0 = torch.empty((B, X), dtype=torch.float32, device=dev)
     st_t, st_e = _strides(rew_like, 0)
     sx_t, sx_e = _strides(obs, 1)
-    params = system.pack_params(system_params)
-
-    def p(t):
-        return None if t is None else t.data_ptr()
     with _lib.cuda_guard(obs):
         _lib.check(_lib.lib.mbpo_rollout_adjoint(system.system_kind, _lib.C.addressof(params), X, A, B, H, st_t, st_e,
                                                  sx_t, sx_e, p(obs), p(act2), p(g_r), p(g_n), p(g_o), p(g_a),

@@ -193,6 +193,23 @@ def run() -> dict:
                             out[tag + "_" + fname] = f
                         if kind == L.SYSTEM_NOISY_PENDULUM:
                             out[tag + "_sys_key"] = sko
+        # the pendulum's reverse scan, time-major [T, E, ...] and dense [E, T, ...], with NULL cotangents
+        if kind == L.SYSTEM_PENDULUM:
+            obs_t = _t(_state(rng, E * T, X).reshape(T, E, X))
+            cot = [_t(rng.normal(size=s)) for s in ((T, E), (T, E, X), (T, E, X), (T, E))]
+            for layout in ("time_major", "dense"):
+                f = (lambda v: v) if layout == "time_major" else (lambda v: v.transpose(0, 1).contiguous())
+                ob, ac = f(obs_t), f(acts[..., 0])
+                st_t, st_e = (E, 1) if layout == "time_major" else (1, T)
+                sx_t, sx_e = (E * X, X) if layout == "time_major" else (X, T * X)
+                for use in ((1, 1, 1, 1), (1, 0, 0, 0), (0, 1, 0, 1)):
+                    gr, gn, go, ga = (f(c) if u else None for c, u in zip(cot, use))
+                    g_act, g_x0 = torch.empty_like(ac), torch.empty((E, X), device=DEV)
+                    chk("rollout_adjoint", L.lib.mbpo_rollout_adjoint(
+                        kind, C.addressof(PEND), X, A, E, T, st_t, st_e, sx_t, sx_e, L.ptr(ob), L.ptr(ac), L.ptr(gr),
+                        L.ptr(gn), L.ptr(go), L.ptr(ga), L.ptr(g_act), L.ptr(g_x0), st))
+                    tag = "%s_adjoint_%s_%d%d%d%d" % ((sname, layout) + use)
+                    out.update({tag + "_g_action": g_act, tag + "_g_x0": g_x0})
         # the plans, fused and staged
         params = C.addressof(PEND) if kind == L.SYSTEM_PENDULUM else C.addressof(GEN)
         for prng in (0, 1):
