@@ -111,21 +111,9 @@ __device__ __forceinline__ float swish_exact(float x) {
 // jax.nn.softplus(x) = logaddexp(x, 0) = max(x, 0) + log1p(exp(-|x|))
 __device__ __forceinline__ float softplus_exact(float x) { return fmaxf(x, 0.0f) + log1pf(expf(-fabsf(x))); }
 
-// Packed float32 pair arithmetic (sm_100: FFMA2 takes a scalar and a register pair).  A 3-register FFMA issues
-// every other cycle per scheduler; the packed form retires two FMAs per issue slot, IEEE-rounded per element.
-typedef unsigned long long f32x2_t;
-__device__ __forceinline__ f32x2_t pack2(float lo, float hi) {
-  f32x2_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void unpack2(f32x2_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-// acc += s * v  (s scalar, v and acc pairs)
-__device__ __forceinline__ void fma2_scalar(f32x2_t& acc, float s, f32x2_t w) {
-  asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(pack2(s, s)), "l"(w));
-}
+// acc += s * v  (s scalar, v and acc packed pairs, mathx.cuh).  A 3-register FFMA issues every other cycle per
+// scheduler; FFMA2 takes the scalar and a register pair and retires two FMAs per issue slot.
+__device__ __forceinline__ void fma2_scalar(f32x2_t& acc, float s, f32x2_t w) { acc = fma2(splat2(s), w, acc); }
 
 struct ActorSmem {
   // float offsets into dynamic shared memory

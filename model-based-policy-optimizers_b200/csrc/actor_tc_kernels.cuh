@@ -138,17 +138,6 @@ __device__ __forceinline__ void split_tf32(float v, float& hi, float& lo) {
   hi = to_tf32(v);
   lo = to_tf32(v - hi);
 }
-// packed float32 pairs (one issue slot for two lanes of work; IEEE-rounded per element)
-__device__ __forceinline__ f32x2_t add2(f32x2_t x, f32x2_t y) {
-  f32x2_t r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(x), "l"(y));
-  return r;
-}
-__device__ __forceinline__ f32x2_t mul2(f32x2_t x, f32x2_t y) {
-  f32x2_t r;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(x), "l"(y));
-  return r;
-}
 __device__ __forceinline__ float ex2_approx(float x) {
   float r;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -182,11 +171,6 @@ __device__ __forceinline__ void split_tf32_2(float v0, float v1, float& h0, floa
   unpack2(add2(pack2(v0, v1), pack2(-h0, -h1)), d0, d1);
   l0 = __uint_as_float(__float_as_uint(d0) + 0x1000u);
   l1 = __uint_as_float(__float_as_uint(d1) + 0x1000u);
-}
-__device__ __forceinline__ f32x2_t fma2(f32x2_t x, f32x2_t y, f32x2_t z) {
-  f32x2_t r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(x), "l"(y), "l"(z));
-  return r;
 }
 
 template <int PRNG, int MATH>

@@ -41,26 +41,23 @@ __device__ __forceinline__ float rollout_return(const PendulumConsts& pc, float 
 
 // Two independent rollouts from the same initial state (th0 = atan2(s0, c0), computed once per problem by the
 // caller), interleaved step by step: the horizon recurrence is a serial dependency chain, so a second chain in
-// the same thread doubles the instruction-level parallelism at a cost of ~8 registers.
-template <int MATH, bool SMALL>
+// the same thread doubles the instruction-level parallelism at a cost of ~8 registers.  The two chains run as the
+// halves of packed pairs (pendulum.cuh pair forms): one FFMA2 / FMUL2 / FADD2 issue slot serves both, same bits as
+// two scalar steps.  SMALL only (|target_angle| <= 6, host-checked).
+template <int MATH>
 __device__ __forceinline__ void rollout_return2(const PendulumConsts& pc, float th0, float w0, int H,
                                                 const float* __restrict__ row_a, const float* __restrict__ row_b,
                                                 float& ret_a, float& ret_b) {
-  float acc_a = 0.0f, acc_b = 0.0f;
-  float tha = th0, wa = w0, thb = th0, wb = w0;
+  f32x2_t acc = splat2(0.0f), th = splat2(th0), w = splat2(w0);
 #pragma unroll 1
   for (int t = 0; t < H; ++t) {
-    float ra, rb;
-    if (MATH == MBPO_MATH_REFERENCE) {
-      pendulum_step_ref_th<SMALL>(pc, tha, wa, row_a[t], ra);
-      pendulum_step_ref_th<SMALL>(pc, thb, wb, row_b[t], rb);
-    } else {
-      pendulum_step_theta<SMALL>(pc, tha, wa, row_a[t], ra);
-      pendulum_step_theta<SMALL>(pc, thb, wb, row_b[t], rb);
-    }
-    acc_a = __fadd_rn(acc_a, ra);
-    acc_b = __fadd_rn(acc_b, rb);
+    f32x2_t neg_r;
+    if (MATH == MBPO_MATH_REFERENCE) pendulum_step_ref_th2(pc, th, w, pack2(row_a[t], row_b[t]), neg_r);
+    else pendulum_step_theta2(pc, th, w, pack2(row_a[t], row_b[t]), neg_r);
+    acc = sub2(acc, neg_r);   // acc + reward
   }
+  float acc_a, acc_b;
+  unpack2(acc, acc_a, acc_b);
   ret_a = __fdiv_rn(acc_a, static_cast<float>(H));
   ret_b = __fdiv_rn(acc_b, static_cast<float>(H));
 }
@@ -249,8 +246,8 @@ __device__ __forceinline__ void plan_problem(const PlanArgs& a, const PlanCtaSme
       }
       const int r0 = n0 < N ? n0 : N, r1 = n1 < N ? n1 : N;   // idle slots roll out the zero row
       float ret0, ret1;
-      rollout_return2<MATH, true>(pc, x_th, x_w, H, act + static_cast<size_t>(r0) * HS,
-                                  act + static_cast<size_t>(r1) * HS, ret0, ret1);
+      rollout_return2<MATH>(pc, x_th, x_w, H, act + static_cast<size_t>(r0) * HS, act + static_cast<size_t>(r1) * HS,
+                            ret0, ret1);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int n = h ? n1 : n0;

@@ -72,24 +72,31 @@ __device__ __forceinline__ void stage_normals_task(Key2 key, const float* __rest
                                                    uint32_t* bits_out, int j) {
   using S = NoiseShape<H>;
   constexpr int LASTK = S::EVEN ? S::F - 1 : S::F;
-  auto put = [&](int k, uint32_t word) {
+  // v = bits_to_normal(word) * scale[k]
+  auto put = [&](int k, uint32_t word, float v) {
     if (bits_out) bits_out[k] = word;
     if (!IMAG) {
-      stage[k] = bits_to_normal(word) * scale[k];
+      stage[k] = v;
     } else if (k >= 1 && k < LASTK) {
-      stage[S::F + k - 1] = bits_to_normal(word) * scale[k];
+      stage[S::F + k - 1] = v;
     }
   };
   if (MODE == 1) {
     uint32_t x0 = 0u, x1 = static_cast<uint32_t>(j);
     threefry2x32(key.k0, key.k1, x0, x1);
-    put(j, x0 ^ x1);
+    put(j, x0 ^ x1, bits_to_normal(x0 ^ x1) * scale[j]);
   } else {
     uint32_t x0 = static_cast<uint32_t>(j);
     uint32_t x1 = (S::HALF + j < S::F) ? static_cast<uint32_t>(S::HALF + j) : 0u;
     threefry2x32(key.k0, key.k1, x0, x1);
-    put(j, x0);
-    if (S::HALF + j < S::F) put(S::HALF + j, x1);
+    if (S::HALF + j < S::F) {   // both words are normals: one packed chain
+      float v0, v1;
+      unpack2(mul2(bits_to_normal2(x0, x1), pack2(scale[j], scale[S::HALF + j])), v0, v1);
+      put(j, x0, v0);
+      put(S::HALF + j, x1, v1);
+    } else {
+      put(j, x0, bits_to_normal(x0) * scale[j]);
+    }
   }
 }
 

@@ -125,6 +125,74 @@ __device__ __forceinline__ void pendulum_step_theta(const PendulumConsts& p, flo
   w = nw;
 }
 
+// ---- pair forms: two independent chains in one thread (rollout_return2), SMALL only ---------------------------
+// Each packs the scalar function's float additions, multiplications and FMAs into FADD2 / FMUL2 / FFMA2 on the same
+// operands in the same order; clips, compares and the conditional +-2 pi run per element.  Same bits per element.
+
+// wrap_diff<true> of both elements.
+__device__ __forceinline__ f32x2_t wrap_diff_small2(f32x2_t d) {
+  float r[2];
+  unpack2(add2(d, splat2(MBPO_PI_F)), r[0], r[1]);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    if (r[i] >= MBPO_TWO_PI_F) r[i] -= MBPO_TWO_PI_F;
+    if (r[i] <= -MBPO_TWO_PI_F) r[i] += MBPO_TWO_PI_F;
+    if (r[i] < 0.0f) r[i] += MBPO_TWO_PI_F;
+  }
+  return sub2(pack2(r[0], r[1]), splat2(MBPO_PI_F));
+}
+
+// MINUS the reward of both elements: reward_from<true> computes fma(-control_cost, u*u, -t); this is
+// fma(control_cost, u*u, t), its exact negation under round-to-nearest except that an exact zero comes out +0 where
+// the reward is -0.  Subtracted from a sum that starts at +0 it gives the bits adding the reward gives.
+__device__ __forceinline__ f32x2_t neg_reward_small2(const PendulumConsts& p, f32x2_t th, f32x2_t thdot, f32x2_t u) {
+  const f32x2_t diff = wrap_diff_small2(sub2(th, splat2(p.target_angle)));
+  const f32x2_t t = fma2(splat2(0.1f), mul2(thdot, thdot), mul2(splat2(p.angle_cost), mul2(diff, diff)));
+  return fma2(splat2(p.control_cost), mul2(u, u), t);
+}
+
+// pendulum_next_thdot of both elements.
+__device__ __forceinline__ f32x2_t pendulum_next_thdot2(const PendulumConsts& p, f32x2_t sin_th, f32x2_t w,
+                                                        f32x2_t u) {
+  float u0, u1;
+  unpack2(u, u0, u1);
+  const f32x2_t uu = mul2(pack2(fminf(fmaxf(u0, -1.0f), 1.0f), fminf(fmaxf(u1, -1.0f), 1.0f)), splat2(p.max_torque));
+  const f32x2_t thdd = fma2(splat2(p.c_g), sin_th, mul2(splat2(p.c_u), uu));
+  float v0, v1;
+  unpack2(fma2(thdd, splat2(p.dt), w), v0, v1);
+  return pack2(fminf(fmaxf(v0, -p.max_speed), p.max_speed), fminf(fmaxf(v1, -p.max_speed), p.max_speed));
+}
+
+// pendulum_step_ref_th<true> of two chains; neg_reward as neg_reward_small2.
+__device__ __forceinline__ void pendulum_step_ref_th2(const PendulumConsts& p, f32x2_t& th, f32x2_t& w, f32x2_t u,
+                                                      f32x2_t& neg_reward) {
+  neg_reward = neg_reward_small2(p, th, w, u);
+  f32x2_t s, c;
+  sincos_bounded2(th, s, c);
+  const f32x2_t nw = pendulum_next_thdot2(p, s, w, u);
+  sincos_bounded2(fma2(nw, splat2(p.dt), th), s, c);
+  th = atan2_bounded_unit2(s, c);
+  w = nw;
+}
+
+// pendulum_step_theta<true> of two chains; neg_reward as neg_reward_small2.
+__device__ __forceinline__ void pendulum_step_theta2(const PendulumConsts& p, f32x2_t& th, f32x2_t& w, f32x2_t u,
+                                                     f32x2_t& neg_reward) {
+  neg_reward = neg_reward_small2(p, th, w, u);
+  f32x2_t s, c;
+  sincos_bounded2(th, s, c);
+  const f32x2_t nw = pendulum_next_thdot2(p, s, w, u);
+  float nth[2];
+  unpack2(fma2(nw, splat2(p.dt), th), nth[0], nth[1]);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    if (nth[i] > MBPO_PI_F) nth[i] -= MBPO_TWO_PI_F;
+    if (nth[i] < -MBPO_PI_F) nth[i] += MBPO_TWO_PI_F;
+  }
+  th = pack2(nth[0], nth[1]);
+  w = nw;
+}
+
 // jnp.clip = minimum(maximum(x, lo), hi): lax.max / lax.min split the cotangent evenly at a tie.
 __device__ __forceinline__ float clip_grad(float x, float lo, float hi) {
   const float a = (x > lo) ? 1.0f : (x == lo ? 0.5f : 0.0f);          // d max(x, lo) / dx

@@ -109,7 +109,7 @@ def run() -> dict:
         # System.step and the objective
         for mode in (0, 1):
             u = _t(rng.uniform(-1.5, 1.5, (E, A)))
-            xn, r, ko = torch.empty_like(x0), torch.empty(E, device=DEV), torch.empty_like(sk)
+            xn, r, ko = torch.empty_like(x0), torch.empty(E, device=DEV), torch.zeros_like(sk)   # ko: keyed only
             chk("step_general", L.lib.mbpo_system_step_general(kind, C.byref(GEN), mode, L.ptr(x0), L.ptr(u), L.ptr(sk),
                                                               E, L.ptr(xn), L.ptr(r), L.ptr(ko), st))
             out.update({"%s_step%d_x" % (sname, mode): xn, "%s_step%d_r" % (sname, mode): r,
@@ -238,6 +238,38 @@ def run() -> dict:
                                                                        L.ptr(val), L.ptr(kout), L.ptr(ws), nb, st))
                     tag = "%s_plan%d%d_%s" % (sname, prng, math, "fused" if fused else "staged")
                     out.update({tag + "_seq": seq, tag + "_val": val, tag + "_key": kout})
+                if kind != L.SYSTEM_PENDULUM:
+                    continue
+                # the pendulum's fused plan at the flagship size (H = 30, 512 samples; white and colored noise), an
+                # any-horizon instance (H = 23), cluster plans and the one-launch closed loop
+                for H, exponent, B, cluster in ((30, 0.0, 40, 1), (30, 2.0, 40, 1), (30, 0.0, 1, 16), (30, 2.0, 3, 4),
+                                                (23, 1.0, 5, 1)):
+                    cfg = L.IcemCfgC()
+                    chk("cfg", L.lib.mbpo_icem_cfg_init(C.byref(cfg), H, A, X, 1, 512, 50, 0.5, 0.1, 5, exponent,
+                                                        0.3, -2.0, 2.0, 1, 1e4))
+                    cfg.prng_mode, cfg.system_kind, cfg.math_mode = prng, kind, math
+                    xo = _t(_state(rng, B, X))
+                    kin = _keys(rng, B)
+                    seq_in = _t(rng.uniform(-1, 1, (B, H, A)))
+                    seq, val = torch.empty_like(seq_in), torch.empty(B, device=DEV)
+                    kout = torch.empty((B, 2), dtype=torch.uint32, device=DEV)
+                    chk("plan_clustered", L.lib.mbpo_icem_plan_clustered(
+                        C.byref(cfg), params, L.ptr(xo), L.ptr(kin), L.ptr(seq_in), B, L.ptr(seq), L.ptr(val),
+                        L.ptr(kout), None, cluster, st))
+                    tag = "%s_plan%d%d_H%d_e%g_B%d_c%d" % (sname, prng, math, H, exponent, B, cluster)
+                    out.update({tag + "_seq": seq, tag + "_val": val, tag + "_key": kout})
+                    if H != 30 or exponent != 0.0:
+                        continue
+                    n_mpc = 4   # closed-loop steps (T above stays the env / actor rollout length)
+                    sto, rwo = torch.empty((n_mpc, B, X), device=DEV), torch.empty((n_mpc, B), device=DEV)
+                    aco, seq = torch.empty((n_mpc, B, A), device=DEV), torch.empty_like(seq_in)
+                    kout = torch.empty((B, 2), dtype=torch.uint32, device=DEV)
+                    chk("mpc", L.lib.mbpo_icem_mpc_closed_loop_clustered(
+                        C.byref(cfg), params, L.ptr(xo), L.ptr(kin), L.ptr(seq_in), B, n_mpc, L.ptr(sto), L.ptr(rwo),
+                        L.ptr(aco), L.ptr(seq), L.ptr(kout), cluster, st))
+                    tag = "%s_mpc%d%d_H%d_B%d_c%d" % (sname, prng, math, H, B, cluster)
+                    out.update({tag + "_states": sto, tag + "_rewards": rwo, tag + "_actions": aco, tag + "_seq": seq,
+                                tag + "_key": kout})
     torch.cuda.synchronize(DEV)
     return {k: (v.cpu().view(torch.int32) if v.dtype == torch.uint32 else v.cpu()).numpy() for k, v in out.items()}
 
