@@ -469,6 +469,27 @@ int mbpo_mlp_dynamics_forward(const MbpoMlpEnsembleParams* params_host, const fl
 int mbpo_ensemble_rollout(const MbpoMlpEnsembleParams* params_host, int horizon, const float* x0,
                           const float* actions, int B, int M, int summarize, float* returns_out, void* stream);
 
+/* The learned ensemble as a SAC / PPO env: T wrapped env steps of E envs (the Episode / AutoReset stack of
+ * mbpo_env_unroll_general around x_next = x + MLP_m([x, u]), the reward the pendulum reward on (x, u); a System's
+ * own done is 0), env e rolled through member m[e] for all T steps.  env_order [E] (int32) lists the envs stably
+ * sorted by member, and member_offsets [num_members + 1] (int32) bounds each member's run in it; envs whose member
+ * is outside [0, num_members) are in no run and are not stepped.  obs [E,3] / steps [E] / done [E] are read and
+ * overwritten in place.  policy_host == NULL: the actions are given, actions [T,E,1]; otherwise the policy runs in
+ * the loop as in mbpo_actor_rollout_general (NormalTanh head, deterministic, key_convention, key_in / key_out, the
+ * draw window, raw_action_out / log_prob_out), writing action_out [T,E,1].  Every env's rows are written at its own
+ * index: reward_out, discount_out, truncation_out [T,E], next_observation_out [T,E,3] (observation[t] =
+ * next_observation[t-1]).  E or T == 0 copies the carry key through.  MBPO_EUNSUPPORTED: ensembles other than
+ * hidden 256, x_dim 3, u_dim 1; the BPTT head; the tcgen05 policy kernels; a policy too large for the shared memory
+ * beside the ensemble's (1..2 hidden layers of width 64 fit). */
+int mbpo_ensemble_env_rollout(const MbpoMlpEnsembleParams* params_host, int prng_mode,
+                              const MbpoPolicyParams* policy_host /* NULL: actions given */, int deterministic,
+                              int key_convention, const uint32_t* key_in, int episode_length, int action_repeat,
+                              const int32_t* env_order, const int32_t* member_offsets, float* obs, float* steps,
+                              float* done, const float* first_obs, int E, int T, const float* actions,
+                              float* action_out, float* reward_out, float* discount_out,
+                              float* next_observation_out, float* truncation_out, uint32_t* key_out,
+                              float* raw_action_out, float* log_prob_out, void* stream);
+
 /* ---- replay buffer (brax UniformSamplingQueue) and BraxWrapper.reset ---------------------------
  * The data format either side of the env rollouts: SAC appends every collected Transition to a
  * brax UniformSamplingQueue (mbpo/optimizers/policy_optimizers/sac/sac.py:202-205,303) and

@@ -19,6 +19,7 @@
 #include "actor_tc_kernels.cuh"
 #include "actor_tc_wide_kernels.cuh"
 #include "adjoint_kernels.cuh"
+#include "ensemble_env_kernels.cuh"
 #include "ensemble_pp_kernels.cuh"
 #include "plan_dispatch.h"
 #include "staged_kernels.cuh"
@@ -1065,6 +1066,112 @@ int mbpo_ensemble_rollout(const MbpoMlpEnsembleParams* p, int horizon, const flo
                                               as_stream(stream), g_err, sizeof(g_err));
   if (rc != MBPO_OK) return rc;
   return check_launch("ensemble_rollout_kernel");
+}
+
+// ---- the learned ensemble as a SAC / PPO env (ensemble_env_kernels.cuh) ----------------------------------------
+int mbpo_ensemble_env_rollout(const MbpoMlpEnsembleParams* p, int prng_mode, const MbpoPolicyParams* policy_host,
+                              int deterministic, int key_convention, const uint32_t* key_in, int episode_length,
+                              int action_repeat, const int32_t* env_order, const int32_t* member_offsets, float* obs,
+                              float* steps, float* done, const float* first_obs, int E, int T, const float* actions,
+                              float* action_out, float* reward_out, float* discount_out, float* next_observation_out,
+                              float* truncation_out, uint32_t* key_out, float* raw_action_out, float* log_prob_out,
+                              void* stream) {
+  using namespace mbpo;
+  using namespace mbpo::ens;
+  MBPO_REQUIRE(p, "ensemble_env_rollout: null pointer");
+  MBPO_REQUIRE(p->w_in && p->b_in && p->w_h && p->b_h && p->w_out && p->b_out, "ensemble_env_rollout: null weights");
+  if (p->hidden != HID || p->x_dim != 3 || p->u_dim != 1 || p->num_members < 1)
+    return fail(MBPO_EUNSUPPORTED, "ensemble_env_rollout: the tcgen05 kernel needs hidden == 256, x_dim == 3, "
+                "u_dim == 1 and at least one member (got %d, %d, %d, %d members)", p->hidden, p->x_dim, p->u_dim,
+                p->num_members);
+  MBPO_REQUIRE(prng_mode == 0 || prng_mode == 1, "ensemble_env_rollout: bad prng_mode %d", prng_mode);
+  MBPO_REQUIRE(E >= 0 && T >= 0 && episode_length >= 1 && action_repeat >= 1, "ensemble_env_rollout: bad sizes");
+  MBPO_REQUIRE(static_cast<long long>(T) * action_repeat < (1ll << 31), "ensemble_env_rollout: T * action_repeat "
+               "overflows int");
+  EnsEnvArgs a = {};
+  size_t smem = ens::Smem::TOTAL;
+  if (policy_host) {
+    MBPO_REQUIRE(key_in, "ensemble_env_rollout: null pointer");
+    MBPO_REQUIRE((raw_action_out == nullptr) == (log_prob_out == nullptr),
+                 "ensemble_env_rollout: raw_action_out and log_prob_out come together");
+    MBPO_REQUIRE(key_convention >= 0 && key_convention <= 2, "ensemble_env_rollout: bad key_convention %d",
+                 key_convention);
+    MBPO_REQUIRE(policy_host->head == MBPO_HEAD_NORMAL_TANH || policy_host->head == MBPO_HEAD_BPTT_ACTOR,
+                 "ensemble_env_rollout: bad policy head %d", policy_host->head);
+    MBPO_REQUIRE(policy_host->kernel >= MBPO_ACTOR_AUTO && policy_host->kernel <= MBPO_ACTOR_TCGEN05_WIDE,
+                 "ensemble_env_rollout: bad policy kernel selector %d", policy_host->kernel);
+    if (policy_host->head != MBPO_HEAD_NORMAL_TANH || policy_host->shared_noise)
+      return fail(MBPO_EUNSUPPORTED, "ensemble_env_rollout: the BPTT actor head (one shared draw) runs on the "
+                  "pendulum only; the learned ensemble takes the NormalTanh head");
+    if (policy_host->kernel == MBPO_ACTOR_TCGEN05 || policy_host->kernel == MBPO_ACTOR_TCGEN05_WIDE)
+      return fail(MBPO_EUNSUPPORTED, "ensemble_env_rollout: the tcgen05 policy kernels hold the pendulum only; in "
+                  "the ensemble's env kernel the policy runs on the CUDA cores (MBPO_ACTOR_AUTO or "
+                  "MBPO_ACTOR_CUDA_CORES)");
+    const int rc = fill_policy("ensemble_env_rollout", policy_host, E, 3, 1, a.pol);
+    if (rc != MBPO_OK) return rc;
+    // the policy's weights and biases at their flax shapes, past the model's shared memory
+    GeneralActorSmem lay;
+    int off = 0;
+    auto take = [&](int n) { const int o = off; off += (n + 3) / 4 * 4; return o; };
+    lay.w[0] = take(3 * ACT_W);
+    for (int l = 1; l < a.pol.num_hidden; ++l) lay.w[l] = take(ACT_W * ACT_W);
+    lay.w[a.pol.num_hidden] = take(ACT_W * 2);
+    for (int l = 0; l < a.pol.num_hidden; ++l) lay.b[l] = take(ACT_W);
+    lay.b[a.pol.num_hidden] = take(2);
+    lay.h = 0;
+    lay.total = off;
+    a.lay = lay;
+    smem = ENV_POLICY_W + static_cast<size_t>(off) * sizeof(float);
+    if (smem > 227 * 1024)
+      return fail(MBPO_EUNSUPPORTED, "ensemble_env_rollout: a policy of %d hidden layers needs %zu B of shared memory "
+                  "beside the ensemble's %u B; a CTA has 232448 B (1..2 hidden layers of width 64 fit)",
+                  a.pol.num_hidden, static_cast<size_t>(off) * sizeof(float), ENV_POLICY_W);
+  }
+  cudaStream_t st = as_stream(stream);
+  if (E == 0 || T == 0)          // empty arrays have no address; the carry key passes through
+    return policy_host ? copy_async(key_out, key_in, key_out ? 2 * sizeof(uint32_t) : 0, st, "ensemble_env_rollout")
+                       : MBPO_OK;
+  MBPO_REQUIRE(env_order && member_offsets && obs && steps && done && first_obs, "ensemble_env_rollout: null pointer");
+  MBPO_REQUIRE(reward_out && discount_out && next_observation_out && truncation_out && (policy_host ? action_out : actions),
+               "ensemble_env_rollout: every Transition buffer is required (actions, or action_out with a policy)");
+  EncodeTiledFn enc = encode_tiled_fn();
+  if (!enc) return fail(MBPO_ECUDA, "ensemble_env_rollout: cuTensorMapEncodeTiled is not available from the driver");
+  CUtensorMap map;
+  const cuuint64_t dims[2] = {static_cast<cuuint64_t>(HID), static_cast<cuuint64_t>(p->num_members) * 2 * HID};
+  const cuuint64_t strides[1] = {static_cast<cuuint64_t>(HID) * 2};
+  const cuuint32_t box[2] = {8, 128};
+  const cuuint32_t estr[2] = {1, 1};
+  const CUresult cr = enc(&map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<uint16_t*>(p->w_h), dims, strides, box,
+                          estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (cr != CUDA_SUCCESS)
+    return fail(MBPO_ECUDA, "ensemble_env_rollout: cuTensorMapEncodeTiled failed (CUresult %d)", static_cast<int>(cr));
+  a.num_members = p->num_members; a.E = E; a.T = T; a.episode_length = episode_length; a.action_repeat = action_repeat;
+  // each member's envs fill whole tiles but its last: at most one partial tile per member
+  const long long tiles = (static_cast<long long>(E) + 2 * TILE_M - 1) / (2 * TILE_M) + p->num_members - 1;
+  a.num_tiles = static_cast<int>(tiles);
+  a.policy = policy_host ? 1 : 0;
+  a.deterministic = deterministic ? 1 : 0;
+  a.key_convention = policy_host ? key_convention : 0;
+  a.w_in = p->w_in; a.b_in = p->b_in; a.b_h = p->b_h; a.w_out = p->w_out; a.b_out = p->b_out; a.reward = p->reward;
+  a.env_order = env_order; a.member_offsets = member_offsets;
+  a.obs = obs; a.steps = steps; a.done = done; a.first_obs = first_obs; a.actions = actions;
+  a.key_in = policy_host ? key_in : nullptr; a.key_out = policy_host ? key_out : nullptr;
+  a.action_out = action_out; a.reward_out = reward_out; a.discount_out = discount_out;
+  a.next_observation_out = next_observation_out; a.truncation_out = truncation_out;
+  a.raw_action_out = (policy_host && !deterministic) ? raw_action_out : nullptr;
+  a.log_prob_out = (policy_host && !deterministic) ? log_prob_out : nullptr;
+  const int pairs_max = device_sm_count() / 2;
+  const int pairs = static_cast<int>(tiles < pairs_max ? tiles : pairs_max);
+  return with_prng(prng_mode, [&](auto P) {
+    auto kernel = ensemble_env_kernel<P>;
+    const cudaError_t ce = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                static_cast<int>(smem));
+    if (ce != cudaSuccess)
+      return fail(MBPO_ECUDA, "ensemble_env_rollout: smem attribute (%zu B): %s", smem, cudaGetErrorString(ce));
+    kernel<<<2 * pairs, ENS_THREADS, smem, st>>>(a, map);
+    return check_launch("ensemble_env_kernel");
+  });
 }
 
 }  // extern "C"

@@ -157,6 +157,8 @@ SIGNATURES = {
     "mbpo_lambda_return_vjp": (_I, [_P, _I, _I, _LL, _LL, C.c_double, C.c_double, _P, _P, _P]),
     "mbpo_mlp_dynamics_forward": (_I, [C.POINTER(MlpEnsembleParamsC), _P, _P, _I, _P, _P]),
     "mbpo_ensemble_rollout": (_I, [C.POINTER(MlpEnsembleParamsC), _I, _P, _P, _I, _I, _I, _P, _P]),
+    "mbpo_ensemble_env_rollout": (_I, [C.POINTER(MlpEnsembleParamsC), _I, C.POINTER(PolicyParamsC), _I, _I, _P, _I,
+                                       _I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mbpo_prng_randint": (_I, [_P, _I, _I, _I, _I, _I, _P, _P]),
     "mbpo_replay_insert": (_I, [C.POINTER(ReplayStateC), C.POINTER(ReplayFieldsC), _LL, _P]),
     "mbpo_replay_sample": (_I, [C.POINTER(ReplayStateC), _P, _I, _I, _P, _P, _P, _P]),

@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from .config import config
-from .envs import EnvState, VmappedSystemEnv, is_general, system_keys
+from .envs import EnvState, VmappedSystemEnv, is_ensemble, is_general, system_keys
 from .utils.optimizer_utils import Transition
 
 
@@ -37,8 +37,10 @@ class Policy:
         (``policy_network.apply(normalizer_params, policy_params, obs)``: (obs - mean) / std); emit_extras: PPO's
         policy also returns {'log_prob', 'raw_action'} (ppo_network.py:72-80); kernel: "auto" (tcgen05 for 2..3
         hidden layers -- the wide latency kernel when the envs do not fill the GPU --, CUDA cores otherwise; the
-        CUDA-core kernel of mbpo_actor_rollout_general for NoisyPendulumSystem / PointMassSystem), "cuda_cores",
-        "tcgen05" (throughput kernel) or "tcgen05_wide" (latency kernel); the tcgen05 kernels hold the pendulum only."""
+        CUDA-core kernel of mbpo_actor_rollout_general for NoisyPendulumSystem / PointMassSystem; for
+        MLPEnsembleSystem the policy runs on the CUDA cores inside the ensemble's tcgen05 env kernel,
+        mbpo_ensemble_env_rollout, with 1..2 hidden layers), "cuda_cores", "tcgen05" (throughput kernel) or
+        "tcgen05_wide" (latency kernel); the tcgen05 kernels hold the pendulum only."""
         w = [t.to(torch.float32).contiguous() for t in params.weights]
         b = [t.to(torch.float32).contiguous() for t in params.biases]
         if len(w) < 2 or len(w) != len(b) or len(w) > 5:
@@ -151,7 +153,15 @@ def _rollout(env: VmappedSystemEnv, env_state: EnvState, policy: Policy, key: to
     logp = torch.empty((T, E), dtype=torch.float32, device=dev) if policy.emit_extras else None
     system_params = env_state.system_params
     with _lib.cuda_guard(obs):
-        if is_general(system):
+        if is_ensemble(system):
+            order, offsets = system.env_grouping(system_params, E, dev)
+            _lib.check(_lib.lib.mbpo_ensemble_env_rollout(
+                _lib.C.byref(params), config.prng_mode, _lib.C.byref(policy.struct), int(policy.deterministic),
+                key_convention, _lib.ptr(key), env.episode_length, env.action_repeat, _lib.ptr(order),
+                _lib.ptr(offsets), _lib.ptr(obs), _lib.ptr(steps), _lib.ptr(done), _lib.ptr(first), E, T, None,
+                _lib.ptr(act), _lib.ptr(r), _lib.ptr(d), _lib.ptr(buf[1:]), _lib.ptr(tr), _lib.ptr(key_out),
+                _lib.ptr(raw), _lib.ptr(logp), _lib.stream_ptr(dev)))
+        elif is_general(system):
             sys_keys = system_keys(system, system_params, E)
             sys_keys_out = torch.empty_like(sys_keys) if sys_keys is not None else None
             _lib.check(_lib.lib.mbpo_actor_rollout_general(

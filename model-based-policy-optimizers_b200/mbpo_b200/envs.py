@@ -24,6 +24,12 @@ def is_general(system: System) -> bool:
     return getattr(system, "system_kind", None) in (_lib.SYSTEM_NOISY_PENDULUM, _lib.SYSTEM_POINT_MASS)
 
 
+def is_ensemble(system: System) -> bool:
+    """MLPEnsembleSystem: its collection runs mbpo_ensemble_env_rollout (env e rolled through
+    dynamics_params.member[e])."""
+    return getattr(system, "system_kind", None) == _lib.SYSTEM_MLP_ENSEMBLE
+
+
 def system_keys(system: System, system_params: SystemParams, E: int):
     """The envs' system_params.key [E, 2] a keyed general System steps with (None for one that draws nothing)."""
     if not getattr(system, "keyed", False):
@@ -106,6 +112,7 @@ class VmappedSystemEnv:
         d = torch.empty((T, E), dtype=torch.float32, device=dev)
         tr = torch.empty((T, E), dtype=torch.float32, device=dev)
         params = self.system.pack_params(state.system_params)
+        self._grouping = self.system.env_grouping(state.system_params, E, dev) if is_ensemble(self.system) else None
         keys_in = system_keys(self.system, state.system_params, E) if is_general(self.system) else None
         keys_out = torch.empty_like(keys_in) if keys_in is not None else None
         if T == 0:
@@ -151,6 +158,7 @@ class VmappedSystemEnv:
         nxt = [torch.empty_like(t) for t in cur]
         spare = [torch.empty_like(t) for t in cur]
         params = self.system.pack_params(state.system_params)
+        self._grouping = self.system.env_grouping(state.system_params, E, dev) if is_ensemble(self.system) else None
         s_in.wait_stream(main)              # acts / buf exist before the copies start
         s_out.wait_stream(main)
         bounds = [(t0, min(t0 + chunk_steps, T)) for t0 in range(0, T, max(int(chunk_steps), 1))]
@@ -192,6 +200,17 @@ class VmappedSystemEnv:
                 acts_ptr, E, T, r_ptr, d_ptr, n_ptr, tr_ptr, stream):
         """One launch of T wrapped env steps (observation_out = NULL: observation[t] is next_observation[t-1])."""
         X, A = self.system.x_dim, self.system.u_dim
+        if is_ensemble(self.system):
+            # the ensemble's kernel steps the env state in place
+            for src, dst in ((obs_in, obs_out), (steps_in, steps_out), (done_in, done_out)):
+                if dst.data_ptr() != src.data_ptr():
+                    dst.copy_(src)
+            order, offsets = self._grouping
+            _lib.check(_lib.lib.mbpo_ensemble_env_rollout(
+                _lib.C.byref(params), config.prng_mode, None, 0, 0, None, self.episode_length, self.action_repeat,
+                _lib.ptr(order), _lib.ptr(offsets), _lib.ptr(obs_out), _lib.ptr(steps_out), _lib.ptr(done_out),
+                _lib.ptr(first), E, T, acts_ptr, None, r_ptr, d_ptr, n_ptr, tr_ptr, None, None, None, stream))
+            return
         if is_general(self.system):
             _lib.check(_lib.lib.mbpo_env_unroll_general(
                 self.system.system_kind, _lib.C.byref(params), config.prng_mode, self.episode_length,

@@ -95,6 +95,48 @@ class MLPEnsembleSystem(System):
     def pack_params(self, system_params: SystemParams):
         return self.packed(system_params).struct
 
+    def _checked_member(self, member: torch.Tensor, E: int, num_members: int) -> torch.Tensor:
+        """dynamics_params.member as int32 [E], checked on the host once per tensor: one read-back at its first use,
+        cached by identity (as ``packed`` caches the weights).  A wrong shape or a member outside [0, num_members)
+        raises ValueError before anything is launched."""
+        cached = getattr(self, "_member_cache", None)
+        if cached is not None and cached[0] is member and cached[1] == (E, num_members):
+            return cached[2]
+        if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+            raise ValueError("dynamics_params.member is checked on the host at its first use, which cannot happen "
+                             "inside a CUDA graph capture: run the call once before capturing it")
+        if member.dtype.is_floating_point or member.dtype == torch.bool or member.numel() != E or \
+                (member.dim() > 1 and tuple(member.shape) != (E, 1)):
+            raise ValueError("dynamics_params.member must be an integer tensor [E] = [%d] (got %s %s)"
+                             % (E, member.dtype, tuple(member.shape)))
+        m = member.to(torch.int32).reshape(E).contiguous()
+        if E:
+            lo, hi = (int(v) for v in torch.stack([m.min(), m.max()]).cpu())
+            if lo < 0 or hi >= num_members:
+                raise ValueError("dynamics_params.member holds members in [%d, %d]; the ensemble has %d"
+                                 % (lo, hi, num_members))
+        self._member_cache = (member, (E, num_members), m)
+        return m
+
+    def env_grouping(self, system_params: SystemParams, E: int, device):
+        """The envs grouped by ensemble member for mbpo_ensemble_env_rollout: (env_order int32 [E], the env indices
+        stably sorted by member; member_offsets int32 [num_members + 1], where member k's envs start in env_order).
+        Env e is rolled through dynamics_params.member[e], or member 0 when member is None.  Computed on the device
+        without a synchronisation (a CUDA graph captures it); the members are checked once per tensor."""
+        dyn = system_params.dynamics_params
+        num_members = dyn.num_members
+        if dyn.member is None:
+            order = torch.arange(E, dtype=torch.int32, device=device)
+            offsets = torch.full((num_members + 1,), E, dtype=torch.int32, device=device)
+            offsets[0] = 0
+            return order, offsets
+        m = self._checked_member(dyn.member, E, num_members).to(device)
+        sorted_m, order = torch.sort(m, stable=True)
+        # searchsorted takes any value: no index reaches the device unchecked
+        bounds = torch.arange(num_members + 1, dtype=torch.int32, device=device)
+        offsets = torch.searchsorted(sorted_m, bounds).to(torch.int32)
+        return order.to(torch.int32), offsets
+
     def step(self, x: torch.Tensor, u: torch.Tensor, system_params: SystemParams) -> SystemState:
         """x[..., X], u[..., A] -> SystemState.  Rows use dynamics_params.member (int32 [...]) or member 0."""
         pk = self.packed(system_params)
