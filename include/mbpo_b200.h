@@ -188,6 +188,9 @@ int mbpo_system_step_general(int system_kind, const MbpoGeneralSystemParams* par
  * keys [B,M,2] = split(particles_rng, N+Np) (:177; NULL for a System that draws nothing).
  * num_particles >= 1: split(key, P) (:155), one rollout per particle key, horizon mean, then the left-to-right mean
  * (MBPO_SUMMARIZE_MEAN) or the max over particles -> values_out [B,M].
+ * With num_particles = P >= 1 the Transition buffers are optional too and carry the particle axis: obs_out /
+ * next_obs_out [B,M,P,H,X] and reward_out [B,M,P,H], particle p being the rollout with key split(keys[b,m], P)[p]
+ * (a System that draws nothing writes its single rollout P times); values_out may then be NULL.
  * num_particles == 0: vmap(rollout_actions) (optimizer_utils.py:11-59) -- ONE rollout per row with keys[b,m] as
  * system_params.key; values_out (horizon mean) and the Transition buffers obs_out [B,M,H,X], reward_out [B,M,H],
  * next_obs_out [B,M,H,X] are each optional. */
@@ -246,6 +249,15 @@ int mbpo_icem_plan_staged(const MbpoIcemCfg* cfg_host, const void* sys_params_ho
  * (use_optimism :112-115, use_pessimism :116-119). */
 int mbpo_icem_penalize(float* values, const float* cost, long long n, int num_particles,
                        int summarize_reward, int summarize_cost, float lambda_constraint, void* stream);
+/* The same tail over P distinct particles (a System that draws from its key, or the ensemble's members):
+ * values_out[i] = summarize_reward_p(mean_t reward[i,p,t]) - lambda * relu(summarize_cost_p(cost[i,p])).
+ * reward [n,P,H] is the Transition reward of every particle (mbpo_system_objective / mbpo_ensemble_rollout_transitions),
+ * cost [n,P] (NULL = no cost_fn).  The horizon mean is a left-to-right sum from 0 divided by H and the particle mean
+ * a left-to-right sum divided by P: with cost == NULL the values are bit-equal to mbpo_system_objective's values_out
+ * and mbpo_ensemble_rollout's returns_out. */
+int mbpo_icem_penalize_particles(float* values_out /*[n]*/, const float* reward /*[n,P,H]*/, int horizon,
+                                 const float* cost /*[n,P] or NULL*/, long long n, int num_particles,
+                                 int summarize_reward, int summarize_cost, float lambda_constraint, void* stream);
 /* jnp.clip(actions, u_min, u_max) with bounds broadcast to [H, A] (icem_optimizer.py:47-48,191):
  * clips the N sampled rows of every problem of actions [B, M, D], D = H*A; u_min/u_max [D]. */
 int mbpo_icem_clip_actions(float* actions, const float* u_min, const float* u_max, int B, int M, int N,
@@ -468,6 +480,13 @@ int mbpo_mlp_dynamics_forward(const MbpoMlpEnsembleParams* params_host, const fl
  * the horizon-mean reward.  One fused tcgen05 kernel (CTA pairs, weights resident in shared memory). */
 int mbpo_ensemble_rollout(const MbpoMlpEnsembleParams* params_host, int horizon, const float* x0,
                           const float* actions, int B, int M, int summarize, float* returns_out, void* stream);
+/* The same rollouts with the Transition fields of every member instead of the summary: obs_out[b,m,e,t] is the
+ * state member e's rollout is in before step t (obs_out[b,m,e,0] = x0[b]) and reward_out[b,m,e,t] the pendulum
+ * reward on (that state, u_t).  Same kernels, roundings and checks as mbpo_ensemble_rollout; mbpo_icem_penalize_particles
+ * turns reward_out into its returns_out, bit for bit. */
+int mbpo_ensemble_rollout_transitions(const MbpoMlpEnsembleParams* params_host, int horizon, const float* x0 /*[B,X]*/,
+                                      const float* actions /*[B,M,H,1]*/, int B, int M,
+                                      float* obs_out /*[B,M,E,H,X]*/, float* reward_out /*[B,M,E,H]*/, void* stream);
 
 /* The learned ensemble as a SAC / PPO env: T wrapped env steps of E envs (the Episode / AutoReset stack of
  * mbpo_env_unroll_general around x_next = x + MLP_m([x, u]), the reward the pendulum reward on (x, u); a System's

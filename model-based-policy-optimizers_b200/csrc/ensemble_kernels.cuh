@@ -259,8 +259,12 @@ __device__ long long g_ens_trace[256];
 #define ENS_TRACE(cond, slot) do { } while (0)
 #endif
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
-    ensemble_rollout_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map) {
+// The kernel body.  TR: the row owners also store member e's Transition fields of each valid row,
+// obs_out [R, E, H, 3] (the state before step t) and reward_out [R, E, H] (the reward term of step t), and leave
+// returns_out alone; the MMA / epilogue / mbarrier schedule is the same either way.
+template <bool TR>
+__device__ __forceinline__ void ensemble_rollout_body(const EnsArgs& a, const CUtensorMap& w_map, float* obs_out,
+                                                      float* reward_out) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int quarter = warp >> 2;                       // which 16 of a round's 64 columns (epilogue warps)
@@ -438,7 +442,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
           float u_next = 0.0f;
           if (row_owner) {
             // reward on the current state and the raw action (pendulum_reward.py:32-40); runs under MMA 0
-            acc = __fadd_rn(acc, reward_from(pc, atan2_bounded(x[1], x[0]), x[2], u));
+            const float rw = reward_from(pc, atan2_bounded(x[1], x[0]), x[2], u);
+            if (TR && valid) {
+              const size_t o = (static_cast<size_t>(row) * a.num_members + e) * a.H + t;
+              obs_out[3 * o] = x[0]; obs_out[3 * o + 1] = x[1]; obs_out[3 * o + 2] = x[2];
+              reward_out[o] = rw;
+            }
+            acc = __fadd_rn(acc, rw);
             if (t + 1 < a.H) u_next = __ldg(act + t + 1);
           }
 #pragma unroll
@@ -520,7 +530,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
     }
     if (row_owner && warp != MMA_WARP) {
       if (a.summarize != MBPO_SUMMARIZE_MAX) summary = __fdiv_rn(summary, static_cast<float>(a.num_members));
-      if (valid) a.returns_out[row] = summary;
+      if (!TR && valid) a.returns_out[row] = summary;   // TR: the caller summarises reward_out
     }
   }
 
@@ -533,9 +543,21 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
   }
 }
 
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
+    ensemble_rollout_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map) {
+  ensemble_rollout_body<false>(a, w_map, nullptr, nullptr);
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
+    ensemble_transitions_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map,
+                                float* __restrict__ obs_out, float* __restrict__ reward_out) {
+  ensemble_rollout_body<true>(a, w_map, obs_out, reward_out);
+}
+
+// obs_out / reward_out null: the summary-only kernel; both set: ensemble_transitions_kernel, which also writes them.
 inline int launch_ensemble_rollout(const MbpoMlpEnsembleParams& p, int horizon, const float* x0, const float* actions,
-                                   int B, int M, int summarize, float* returns_out, cudaStream_t st, char* err,
-                                   size_t errlen) {
+                                   int B, int M, int summarize, float* returns_out, float* obs_out, float* reward_out,
+                                   cudaStream_t st, char* err, size_t errlen) {
   if (p.hidden != HID || p.x_dim != 3 || p.u_dim != 1 || p.num_members < 1) {
     snprintf(err, errlen,
              "ensemble rollout: the tcgen05 kernel needs hidden == 256, x_dim == 3, u_dim == 1 (got %d, %d, %d)",
@@ -563,8 +585,10 @@ inline int launch_ensemble_rollout(const MbpoMlpEnsembleParams& p, int horizon, 
   a.num_members = p.num_members; a.R = B * M; a.H = horizon; a.M = M; a.summarize = summarize;
   a.w_in = p.w_in; a.b_in = p.b_in; a.b_h = p.b_h; a.w_out = p.w_out; a.b_out = p.b_out;
   a.x0 = x0; a.actions = actions; a.returns_out = returns_out; a.reward = p.reward;
-  cudaError_t ce = cudaFuncSetAttribute(ensemble_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        static_cast<int>(Smem::TOTAL));
+  const bool tr = obs_out != nullptr;
+  cudaError_t ce = cudaFuncSetAttribute(tr ? reinterpret_cast<const void*>(ensemble_transitions_kernel)
+                                           : reinterpret_cast<const void*>(ensemble_rollout_kernel),
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(Smem::TOTAL));
   if (ce != cudaSuccess) {
     snprintf(err, errlen, "ensemble rollout: smem attribute: %s", cudaGetErrorString(ce));
     return MBPO_ECUDA;
@@ -574,7 +598,8 @@ inline int launch_ensemble_rollout(const MbpoMlpEnsembleParams& p, int horizon, 
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int groups = (a.R + 2 * TILE_M - 1) / (2 * TILE_M);
   const int pairs = groups < sms / 2 ? groups : sms / 2;
-  ensemble_rollout_kernel<<<2 * pairs, ENS_THREADS, Smem::TOTAL, st>>>(a, map);
+  if (tr) ensemble_transitions_kernel<<<2 * pairs, ENS_THREADS, Smem::TOTAL, st>>>(a, map, obs_out, reward_out);
+  else ensemble_rollout_kernel<<<2 * pairs, ENS_THREADS, Smem::TOTAL, st>>>(a, map);
   return MBPO_OK;
 }
 

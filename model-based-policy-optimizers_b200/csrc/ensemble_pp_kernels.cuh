@@ -48,8 +48,10 @@ struct PpSmem {
 };
 static_assert(PpSmem::TOTAL <= 227 * 1024, "ping-pong ensemble rollout shared memory plan exceeds 227 KB");
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
-    ensemble_rollout_pp_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map) {
+// The kernel body; TR as in ensemble_rollout_body.
+template <bool TR>
+__device__ __forceinline__ void ensemble_rollout_pp_body(const EnsArgs& a, const CUtensorMap& w_map, float* obs_out,
+                                                         float* reward_out) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int quarter = warp >> 2;                       // which 16 of a round's 64 columns (epilogue warps)
@@ -253,7 +255,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
 #pragma unroll
             for (int tl = 0; tl < 2; ++tl) {
               // reward on the current state and the raw action (pendulum_reward.py:32-40)
-              acc[tl] = __fadd_rn(acc[tl], reward_from(pc, atan2_bounded(x[tl][1], x[tl][0]), x[tl][2], u[tl]));
+              const float rw = reward_from(pc, atan2_bounded(x[tl][1], x[tl][0]), x[tl][2], u[tl]);
+              if (TR && valid[tl]) {
+                const size_t o = (static_cast<size_t>(row[tl]) * a.num_members + e) * a.H + t;
+                obs_out[3 * o] = x[tl][0]; obs_out[3 * o + 1] = x[tl][1]; obs_out[3 * o + 2] = x[tl][2];
+                reward_out[o] = rw;
+              }
+              acc[tl] = __fadd_rn(acc[tl], rw);
               if (t + 1 < a.H) u_next[tl] = __ldg(act[tl] + t + 1);
             }
           }
@@ -324,7 +332,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
       for (int tl = 0; tl < 2; ++tl) {
         float s = summary[tl];
         if (a.summarize != MBPO_SUMMARIZE_MAX) s = __fdiv_rn(s, static_cast<float>(a.num_members));
-        if (valid[tl]) a.returns_out[row[tl]] = s;
+        if (!TR && valid[tl]) a.returns_out[row[tl]] = s;
       }
     }
   }
@@ -338,19 +346,33 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
   }
 }
 
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
+    ensemble_rollout_pp_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map) {
+  ensemble_rollout_pp_body<false>(a, w_map, nullptr, nullptr);
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ENS_THREADS, 1)
+    ensemble_transitions_pp_kernel(const __grid_constant__ EnsArgs a, const __grid_constant__ CUtensorMap w_map,
+                                   float* __restrict__ obs_out, float* __restrict__ reward_out) {
+  ensemble_rollout_pp_body<true>(a, w_map, obs_out, reward_out);
+}
+
 // Chooses the kernel: the two-tile kernel needs half as many CTA pairs per row, so it is used whenever the
 // one-tile kernel would need more than one round of CTA pairs (throughput shapes); small row counts keep
 // the one-tile kernel, which spreads them over more SMs (latency shapes).  The row count alone decides
-// (no run-time switch); the tests reach each kernel through its own sizes.
+// (no run-time switch); the tests reach each kernel through its own sizes.  obs_out / reward_out: as in
+// launch_ensemble_rollout.
 inline int launch_ensemble_rollout_auto(const MbpoMlpEnsembleParams& p, int horizon, const float* x0,
                                         const float* actions, int B, int M, int summarize, float* returns_out,
-                                        cudaStream_t st, char* err, size_t errlen) {
+                                        float* obs_out, float* reward_out, cudaStream_t st, char* err, size_t errlen) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long R = static_cast<long long>(B) * M;
   const bool use_pp = R > static_cast<long long>(2 * TILE_M) * (sms / 2);
-  if (!use_pp) return launch_ensemble_rollout(p, horizon, x0, actions, B, M, summarize, returns_out, st, err, errlen);
+  if (!use_pp)
+    return launch_ensemble_rollout(p, horizon, x0, actions, B, M, summarize, returns_out, obs_out, reward_out, st, err,
+                                   errlen);
   if (p.hidden != HID || p.x_dim != 3 || p.u_dim != 1 || p.num_members < 1) {
     snprintf(err, errlen,
              "ensemble rollout: the tcgen05 kernel needs hidden == 256, x_dim == 3, u_dim == 1 (got %d, %d, %d)",
@@ -378,15 +400,18 @@ inline int launch_ensemble_rollout_auto(const MbpoMlpEnsembleParams& p, int hori
   a.num_members = p.num_members; a.R = B * M; a.H = horizon; a.M = M; a.summarize = summarize;
   a.w_in = p.w_in; a.b_in = p.b_in; a.b_h = p.b_h; a.w_out = p.w_out; a.b_out = p.b_out;
   a.x0 = x0; a.actions = actions; a.returns_out = returns_out; a.reward = p.reward;
-  cudaError_t ce = cudaFuncSetAttribute(ensemble_rollout_pp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        static_cast<int>(PpSmem::TOTAL));
+  const bool tr = obs_out != nullptr;
+  cudaError_t ce = cudaFuncSetAttribute(tr ? reinterpret_cast<const void*>(ensemble_transitions_pp_kernel)
+                                           : reinterpret_cast<const void*>(ensemble_rollout_pp_kernel),
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(PpSmem::TOTAL));
   if (ce != cudaSuccess) {
     snprintf(err, errlen, "ensemble rollout: smem attribute: %s", cudaGetErrorString(ce));
     return MBPO_ECUDA;
   }
   const int groups = (a.R + 4 * TILE_M - 1) / (4 * TILE_M);
   const int pairs = groups < sms / 2 ? groups : sms / 2;
-  ensemble_rollout_pp_kernel<<<2 * pairs, ENS_THREADS, PpSmem::TOTAL, st>>>(a, map);
+  if (tr) ensemble_transitions_pp_kernel<<<2 * pairs, ENS_THREADS, PpSmem::TOTAL, st>>>(a, map, obs_out, reward_out);
+  else ensemble_rollout_pp_kernel<<<2 * pairs, ENS_THREADS, PpSmem::TOTAL, st>>>(a, map);
   return MBPO_OK;
 }
 

@@ -569,13 +569,18 @@ int mbpo_system_objective(int system_kind, const MbpoGeneralSystemParams* params
   if (total == 0) return MBPO_OK;
   MBPO_REQUIRE(params_host && x0 && actions, "system_objective: null pointer");
   MBPO_REQUIRE(!keyed || keys, "system_objective: this System draws from system_params.key: keys is null");
-  MBPO_REQUIRE(num_particles == 0 || values_out, "system_objective: values_out is null");
-  MBPO_REQUIRE(num_particles == 0 || !(obs_out || reward_out || next_obs_out),
-               "system_objective: Transition buffers exist for single rollouts (num_particles == 0) only");
+  const bool buffers = obs_out || reward_out || next_obs_out;
+  MBPO_REQUIRE(num_particles == 0 || values_out || buffers, "system_objective: values_out is null");
   const unsigned blocks = static_cast<unsigned>((total + 127) / 128);
   return with_system<PendulumSys, NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
     using Sys = typename decltype(t)::type;
     return with_prng(prng_mode, [&](auto P) {
+      if (num_particles > 0 && buffers) {
+        general_particles_kernel<Sys, P><<<blocks, 128, 0, as_stream(stream)>>>(
+            *params_host, horizon, x0, actions, keys, B, M, num_particles, summarize, values_out, obs_out, reward_out,
+            next_obs_out);
+        return check_launch("general_particles_kernel");
+      }
       general_objective_kernel<Sys, P><<<blocks, 128, 0, as_stream(stream)>>>(
           *params_host, horizon, x0, actions, keys, B, M, num_particles, summarize, values_out, obs_out, reward_out,
           next_obs_out);
@@ -777,6 +782,19 @@ int mbpo_icem_penalize(float* values, const float* cost, long long n, int num_pa
   penalize_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, as_stream(stream)>>>(
       values, cost, n, num_particles, summarize_reward, summarize_cost, lambda_constraint);
   return check_launch("penalize_kernel");
+}
+
+int mbpo_icem_penalize_particles(float* values_out, const float* reward, int horizon, const float* cost, long long n,
+                                 int num_particles, int summarize_reward, int summarize_cost, float lambda_constraint,
+                                 void* stream) {
+  MBPO_REQUIRE(n >= 0 && num_particles >= 1 && horizon >= 1, "penalize_particles: bad sizes");
+  MBPO_REQUIRE((summarize_reward == 0 || summarize_reward == 1) && (summarize_cost == 0 || summarize_cost == 1),
+               "penalize_particles: bad summarize");
+  if (n == 0) return MBPO_OK;
+  MBPO_REQUIRE(values_out && reward, "penalize_particles: null pointer");
+  penalize_particles_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, as_stream(stream)>>>(
+      values_out, reward, horizon, cost, n, num_particles, summarize_reward, summarize_cost, lambda_constraint);
+  return check_launch("penalize_particles_kernel");
 }
 
 int mbpo_icem_clip_actions(float* actions, const float* u_min, const float* u_max, int B, int M, int N, int D,
@@ -1062,10 +1080,24 @@ int mbpo_ensemble_rollout(const MbpoMlpEnsembleParams* p, int horizon, const flo
   MBPO_REQUIRE(horizon >= 1 && B >= 0 && M >= 0, "ensemble_rollout: bad sizes");
   MBPO_REQUIRE(summarize == 0 || summarize == 1, "ensemble_rollout: bad summarize %d", summarize);
   if (static_cast<long long>(B) * M == 0) return MBPO_OK;
-  const int rc = ens::launch_ensemble_rollout_auto(*p, horizon, x0, actions, B, M, summarize, returns_out,
-                                              as_stream(stream), g_err, sizeof(g_err));
+  const int rc = ens::launch_ensemble_rollout_auto(*p, horizon, x0, actions, B, M, summarize, returns_out, nullptr,
+                                                   nullptr, as_stream(stream), g_err, sizeof(g_err));
   if (rc != MBPO_OK) return rc;
   return check_launch("ensemble_rollout_kernel");
+}
+
+int mbpo_ensemble_rollout_transitions(const MbpoMlpEnsembleParams* p, int horizon, const float* x0,
+                                      const float* actions, int B, int M, float* obs_out, float* reward_out,
+                                      void* stream) {
+  MBPO_REQUIRE(p && x0 && actions && obs_out && reward_out, "ensemble_rollout_transitions: null pointer");
+  MBPO_REQUIRE(p->w_in && p->b_in && p->w_h && p->b_h && p->w_out && p->b_out,
+               "ensemble_rollout_transitions: null weights");
+  MBPO_REQUIRE(horizon >= 1 && B >= 0 && M >= 0, "ensemble_rollout_transitions: bad sizes");
+  if (static_cast<long long>(B) * M == 0) return MBPO_OK;
+  const int rc = ens::launch_ensemble_rollout_auto(*p, horizon, x0, actions, B, M, MBPO_SUMMARIZE_MEAN, nullptr,
+                                                   obs_out, reward_out, as_stream(stream), g_err, sizeof(g_err));
+  if (rc != MBPO_OK) return rc;
+  return check_launch("ensemble_transitions_kernel");
 }
 
 // ---- the learned ensemble as a SAC / PPO env (ensemble_env_kernels.cuh) ----------------------------------------

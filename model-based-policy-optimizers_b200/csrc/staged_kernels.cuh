@@ -184,6 +184,37 @@ __global__ void penalize_kernel(float* values, const float* __restrict__ cost, l
   values[i] = v;
 }
 
+// The same tail over P distinct particles (a keyed System, or the ensemble's members): per particle the horizon mean
+// of reward [n, P, H] (a left-to-right sum from 0, divided by H, as general_rollout and the ensemble kernels round
+// it), then the left-to-right mean or the max over particles; the same for cost [n, P] (may be null).
+__global__ void penalize_particles_kernel(float* __restrict__ values_out, const float* __restrict__ reward, int H,
+                                          const float* __restrict__ cost, long long n, int P, int summarize_reward,
+                                          int summarize_cost, float lambda) {
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float* rw = reward + static_cast<size_t>(i) * P * H;
+  float sum = 0.0f, mx = 0.0f;
+  for (int p = 0; p < P; ++p) {
+    float acc = 0.0f;
+    for (int t = 0; t < H; ++t) acc = __fadd_rn(acc, __ldg(rw + static_cast<size_t>(p) * H + t));
+    const float ret = __fdiv_rn(acc, static_cast<float>(H));
+    sum = __fadd_rn(sum, ret);
+    mx = (p == 0) ? ret : fmaxf(mx, ret);
+  }
+  float v = (summarize_reward == MBPO_SUMMARIZE_MAX) ? mx : __fdiv_rn(sum, static_cast<float>(P));
+  if (cost) {
+    float csum = 0.0f, cmx = 0.0f;
+    for (int p = 0; p < P; ++p) {
+      const float c = __ldg(cost + static_cast<size_t>(i) * P + p);
+      csum = __fadd_rn(csum, c);
+      cmx = (p == 0) ? c : fmaxf(cmx, c);
+    }
+    const float c = (summarize_cost == MBPO_SUMMARIZE_MAX) ? cmx : __fdiv_rn(csum, static_cast<float>(P));
+    v = __fsub_rn(v, __fmul_rn(lambda, fmaxf(c, 0.0f)));
+  }
+  values_out[i] = v;
+}
+
 // jnp.clip(actions, u_min, u_max) with bounds broadcast to [H, A] (icem_optimizer.py:47-48,191): the N
 // sampled rows of every problem; the kept-elite rows (n >= N) are not clipped (:192).
 __global__ void clip_actions_kernel(float* actions, const float* __restrict__ u_min, const float* __restrict__ u_max,

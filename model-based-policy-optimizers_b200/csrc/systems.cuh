@@ -240,4 +240,38 @@ __global__ void __launch_bounds__(128)
   values_out[r] = out;
 }
 
+// general_objective_kernel's P >= 1 path with the Transition buffers of every particle: particle p of row r writes
+// obs / next_obs [r, p, H, X] and reward [r, p, H] from the rollout with key split(key, P)[p] (:155); an unkeyed System
+// runs its one rollout P times, so the P copies and the summary are those of P identical particles.  values_out
+// (optional) gets the summary general_objective_kernel computes.  A kernel of its own, so that the summary-only
+// kernel stays as it is.
+template <class Sys, int PRNG>
+__global__ void __launch_bounds__(128)
+    general_particles_kernel(const MbpoGeneralSystemParams gp, int H, const float* __restrict__ x0,
+                             const float* __restrict__ actions, const uint32_t* __restrict__ keys, int B, int M, int P,
+                             int summarize, float* __restrict__ values_out, float* __restrict__ obs_out,
+                             float* __restrict__ reward_out, float* __restrict__ next_obs_out) {
+  const long long r = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (r >= static_cast<long long>(B) * M) return;
+  const int b = static_cast<int>(r / M);
+  const Sys sys(gp);
+  float s0[Sys::X];
+#pragma unroll
+  for (int k = 0; k < Sys::X; ++k) s0[k] = x0[static_cast<size_t>(b) * Sys::X + k];
+  const float* acts = actions + static_cast<size_t>(r) * H * Sys::A;
+  Key2 key{0u, 0u};
+  if (Sys::KEYED) key = Key2{keys[2 * r], keys[2 * r + 1]};
+  float acc = 0.0f, mx = 0.0f;
+  for (int p = 0; p < P; ++p) {
+    const Key2 pk = Sys::KEYED ? split_at<PRNG>(key, static_cast<uint32_t>(P), static_cast<uint32_t>(p)) : key;
+    const size_t o = (static_cast<size_t>(r) * P + p) * H;
+    const float ret = general_rollout<Sys, PRNG>(sys, s0, acts, H, pk, obs_out ? obs_out + o * Sys::X : nullptr,
+                                                 reward_out ? reward_out + o : nullptr,
+                                                 next_obs_out ? next_obs_out + o * Sys::X : nullptr, nullptr);
+    acc = __fadd_rn(acc, ret);
+    mx = (p == 0) ? ret : fmaxf(mx, ret);
+  }
+  if (values_out) values_out[r] = (summarize == MBPO_SUMMARIZE_MAX) ? mx : __fdiv_rn(acc, static_cast<float>(P));
+}
+
 }  // namespace mbpo

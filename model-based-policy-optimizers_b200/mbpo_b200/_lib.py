@@ -134,6 +134,7 @@ SIGNATURES = {
     "mbpo_icem_workspace_bytes": (_SZ, [C.POINTER(IcemCfgC), _I]),
     "mbpo_icem_plan_staged": (_I, [C.POINTER(IcemCfgC), _P, _P, _P, _P, _I, _P, _P, _P, _P, _SZ, _P]),
     "mbpo_icem_penalize": (_I, [_P, _P, C.c_longlong, _I, _I, _I, _F, _P]),
+    "mbpo_icem_penalize_particles": (_I, [_P, _P, _I, _P, C.c_longlong, _I, _I, _I, _F, _P]),
     "mbpo_icem_clip_actions": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "mbpo_icem_mpc_closed_loop": (_I, [C.POINTER(IcemCfgC), _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_icem_mpc_closed_loop_clustered": (_I, [C.POINTER(IcemCfgC), _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I,
@@ -157,6 +158,7 @@ SIGNATURES = {
     "mbpo_lambda_return_vjp": (_I, [_P, _I, _I, _LL, _LL, C.c_double, C.c_double, _P, _P, _P]),
     "mbpo_mlp_dynamics_forward": (_I, [C.POINTER(MlpEnsembleParamsC), _P, _P, _I, _P, _P]),
     "mbpo_ensemble_rollout": (_I, [C.POINTER(MlpEnsembleParamsC), _I, _P, _P, _I, _I, _I, _P, _P]),
+    "mbpo_ensemble_rollout_transitions": (_I, [C.POINTER(MlpEnsembleParamsC), _I, _P, _P, _I, _I, _P, _P, _P]),
     "mbpo_ensemble_env_rollout": (_I, [C.POINTER(MlpEnsembleParamsC), _I, C.POINTER(PolicyParamsC), _I, _I, _P, _I,
                                        _I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mbpo_prng_randint": (_I, [_P, _I, _I, _I, _I, _I, _P, _P]),

@@ -221,26 +221,40 @@ class iCemTO(BaseOptimizer):
                       trace: bool = False):
         """iCemTO.optimize with a constraint cost (:161-166) and / or array-valued bounds (:47-48): the
         per-stage C-ABI kernels composed on the caller's stream.  Every number is produced by the CUDA
-        library except the user's own cost function, which is vmapped torch code on the same device."""
-        from ...systems.pendulum_system import PendulumSystem
+        library except the user's own cost function, which is vmapped torch code on the same device.
+
+        With a cost, each iteration rolls out with Transition buffers, evaluates the cost on their observations and
+        penalises the objective; one route per System kind:
+
+        * PendulumSystem / PointMassSystem (deterministic, P identical particles): one rollout per candidate
+          (mbpo_rollout_actions / mbpo_system_objective with P = 0), cost on [B, M, H, X], mbpo_icem_penalize.
+        * NoisyPendulumSystem (draws from its key): mbpo_system_objective with P particles, cost on [B, M, P, H, X],
+          mbpo_icem_penalize_particles.
+        * MLPEnsembleSystem (particle p = member p): mbpo_ensemble_rollout_transitions, cost on [B, M, E, H, X],
+          mbpo_icem_penalize_particles.
+
+        The buffers of the particle routes take 4 * B * M * P * H * (X + 1) bytes per iteration (e.g. ~150 MB for
+        the ensemble at B = 36, M = 1,039, P = 5, H = 50)."""
         cfg = self._cfg()
         L = _lib
         dev = x0.device
         B, X = x0.shape
         H, A = self.opt_dim
         N, Np, S = cfg.num_samples, cfg.num_prev_elites, cfg.num_steps
-        M, D = N + Np, H * A
+        M, D, P = N + Np, H * A, cfg.num_particles
         p = self.opt_params
-        if self.cost_fn is not None and not isinstance(self.system, PendulumSystem):
-            raise L.MbpoUnsupported(L.MBPO_EUNSUPPORTED, "cost_fn needs a System whose rollout kernel writes the "
-                                    "Transition observations (PendulumSystem)")
+        kind = self.system.system_kind
+        general, ensemble = is_general(self.system), kind == L.SYSTEM_MLP_ENSEMBLE
         params = self.system.pack_params(system_params)
+        if ensemble and P != params.num_members:
+            raise L.MbpoUnsupported(L.MBPO_EUNSUPPORTED, "the ensemble System rolls particle p through member p; "
+                                    "num_particles (%d) must equal num_members (%d)" % (P, params.num_members))
         lo = hi = None
         if self._array_bounds():
             lo, hi = _array_bound(p.u_min, self.opt_dim, dev), _array_bound(p.u_max, self.opt_dim, dev)
-        cost_batched = None
-        if self.cost_fn is not None:
-            cost_batched = torch.vmap(torch.vmap(self.cost_fn))          # over problems, then candidates (:162)
+        cost_on = self.cost_fn is not None
+        # a particle axis where the particles differ: a System that draws from its key, or the ensemble's members
+        per_particle = cost_on and (ensemble or (general and self.system.keyed))
         st = L.stream_ptr(dev)
         ks = jr.split(key, 2)                                             # optimizer_key, key  (:246)
         carry, out_key = ks[:, 0].contiguous(), ks[:, 1].contiguous()
@@ -252,37 +266,52 @@ class iCemTO(BaseOptimizer):
         bseq, bval = mean.clone(), torch.full((B,), float("-inf"), dtype=torch.float32, device=dev)   # :244,:235
         actions = torch.empty((B, M, H, A), dtype=torch.float32, device=dev)
         values = torch.empty((B, M), dtype=torch.float32, device=dev)
-        obs = torch.empty((B, M, H, X), dtype=torch.float32, device=dev) if cost_batched is not None else None
+        lead = (B, M, P, H) if per_particle else (B, M, H)
+        obs = torch.empty(lead + (X,), dtype=torch.float32, device=dev) if cost_on else None
+        rew = torch.empty(lead, dtype=torch.float32, device=dev) if per_particle else None
         s_rew = L.SUMMARIZE_MAX if self.use_optimism else L.SUMMARIZE_MEAN    # :112-115
         s_cost = L.SUMMARIZE_MAX if self.use_pessimism else L.SUMMARIZE_MEAN  # :116-119
+        lam = float(p.lambda_constraint)
         tr = {n: [] for n in ("actions", "values", "elite_idx", "mean", "std", "best_value")} if trace else None
         with L.cuda_guard(x0):
             for _ in range(S):
                 nxt_carry = torch.empty_like(carry)
-                general = is_general(self.system)
                 pkeys = torch.empty((B, M, 2), dtype=torch.uint32, device=dev) if general else None
                 L.check(L.lib.mbpo_icem_sample_actions(L.C.byref(cfg), L.ptr(carry), L.ptr(mean), L.ptr(std), B,
                                                        L.ptr(actions), L.ptr(nxt_carry), L.ptr(pkeys), st))
                 if lo is not None:
                     L.check(L.lib.mbpo_icem_clip_actions(L.ptr(actions), L.ptr(lo), L.ptr(hi), B, M, N, D, st))
-                if general:
-                    # one rollout per particle key, horizon mean, mean / max over the particles (:144-160)
-                    L.check(L.lib.mbpo_system_objective(self.system.system_kind, L.C.byref(params), config.prng_mode, H,
-                                                        L.ptr(x0), L.ptr(actions), L.ptr(pkeys), B, M,
-                                                        cfg.num_particles, s_rew, L.ptr(values), None, None, None, st))
-                elif self.system.system_kind == L.SYSTEM_MLP_ENSEMBLE:
+                if per_particle:
+                    if ensemble:
+                        L.check(L.lib.mbpo_ensemble_rollout_transitions(L.C.byref(params), H, L.ptr(x0),
+                                                                        L.ptr(actions), B, M, L.ptr(obs), L.ptr(rew),
+                                                                        st))
+                    else:
+                        L.check(L.lib.mbpo_system_objective(kind, L.C.byref(params), config.prng_mode, H, L.ptr(x0),
+                                                            L.ptr(actions), L.ptr(pkeys), B, M, P, s_rew, None,
+                                                            L.ptr(obs), L.ptr(rew), None, st))
+                    cost = self._cost(obs, actions, (B, M, P))
+                    L.check(L.lib.mbpo_icem_penalize_particles(L.ptr(values), L.ptr(rew), H, L.ptr(cost), B * M, P,
+                                                               s_rew, s_cost, lam, st))
+                elif general:
+                    # one rollout per particle key, horizon mean, mean / max over the particles (:144-160); with a
+                    # cost, the one rollout of a deterministic System and the tail over its P identical particles
+                    L.check(L.lib.mbpo_system_objective(kind, L.C.byref(params), config.prng_mode, H, L.ptr(x0),
+                                                        L.ptr(actions), L.ptr(pkeys), B, M, 0 if cost_on else P,
+                                                        s_rew, L.ptr(values), L.ptr(obs), None, None, st))
+                    if cost_on:
+                        L.check(L.lib.mbpo_icem_penalize(L.ptr(values), L.ptr(self._cost(obs, actions, (B, M))),
+                                                         B * M, P, s_rew, s_cost, lam, st))
+                elif ensemble:
                     # particles = members; the rollout kernel summarises over them itself (:160)
                     L.check(L.lib.mbpo_ensemble_rollout(L.C.addressof(params), H, L.ptr(x0), L.ptr(actions), B, M,
                                                         s_rew, L.ptr(values), st))
                 else:
-                    L.check(L.lib.mbpo_rollout_actions(self.system.system_kind, L.C.addressof(params),
-                                                       config.math_mode_id, H, A, X, L.ptr(x0), L.ptr(actions), B, M,
-                                                       L.ptr(values), L.ptr(obs), None, None, st))
-                    cost = None
-                    if cost_batched is not None:
-                        cost = cost_batched(obs, actions).to(torch.float32).reshape(B, M).contiguous()
-                    L.check(L.lib.mbpo_icem_penalize(L.ptr(values), L.ptr(cost), B * M, cfg.num_particles, s_rew,
-                                                     s_cost, float(p.lambda_constraint), st))
+                    L.check(L.lib.mbpo_rollout_actions(kind, L.C.addressof(params), config.math_mode_id, H, A, X,
+                                                       L.ptr(x0), L.ptr(actions), B, M, L.ptr(values), L.ptr(obs),
+                                                       None, None, st))
+                    cost = self._cost(obs, actions, (B, M)) if cost_on else None
+                    L.check(L.lib.mbpo_icem_penalize(L.ptr(values), L.ptr(cost), B * M, P, s_rew, s_cost, lam, st))
                 n_mean, n_std = torch.empty_like(mean), torch.empty_like(std)
                 n_bval, n_bseq = torch.empty_like(bval), torch.empty_like(bseq)
                 eidx = torch.empty((B, cfg.num_elites), dtype=torch.int32, device=dev) if trace else None
@@ -297,6 +326,21 @@ class iCemTO(BaseOptimizer):
         if trace:
             tr = {n: torch.stack(v) for n, v in tr.items()}
         return bseq, bval, out_key, tr
+
+    def _cost(self, obs: torch.Tensor, actions: torch.Tensor, lead) -> torch.Tensor:
+        """The user's one-trajectory cost (:162) vmapped over the leading axes `lead` of obs [*lead, H, X]: problems,
+        candidates and, where they differ, particles (whose actions are the candidate's, an expanded view) ->
+        contiguous float32 [*lead]."""
+        fn = self.cost_fn
+        for _ in lead:
+            fn = torch.vmap(fn)
+        acts = actions if len(lead) == 2 else actions.unsqueeze(2).expand(lead + tuple(actions.shape[2:]))
+        cost = fn(obs, acts)
+        if not isinstance(cost, torch.Tensor) or cost.numel() != obs.shape[:len(lead)].numel():
+            raise ValueError("cost_fn must return one scalar per trajectory (states [H, X], actions [H, A]); got %s "
+                             "for %s trajectories" % (tuple(cost.shape) if isinstance(cost, torch.Tensor)
+                                                      else type(cost).__name__, tuple(lead)))
+        return cost.to(torch.float32).reshape(lead).contiguous()
 
     def _canon(self, initial_state: torch.Tensor, opt_state: iCemOptimizerState):
         single = initial_state.dim() == 1

@@ -64,14 +64,17 @@ class _GeneralSystem(System):
                   num_particles: int = 0, use_optimism: bool = False, full: bool = False):
         """vmap(vmap(objective)): x0 [B, X], actions [B, M, H, A], keys [B, M, 2] -> values [B, M]
         (num_particles = 0: one rollout per row with keys[b, m] as the System's key; ``full`` adds the Transition
-        buffers observation / reward / next_observation)."""
+        buffers observation / reward / next_observation, [B, M, H, X] / [B, M, H] / [B, M, H, X] -- with
+        num_particles = P >= 1 they carry the particle axis, [B, M, P, H, X] / [B, M, P, H] / [B, M, P, H, X], particle
+        p being the rollout with key split(keys[b, m], P)[p])."""
         B, M, H, A = actions.shape
         dev = x0.device
         values = torch.empty((B, M), dtype=torch.float32, device=dev)
         obs = rew = nxt = None
         if full:
-            obs = torch.empty((B, M, H, self.x_dim), dtype=torch.float32, device=dev)
-            rew = torch.empty((B, M, H), dtype=torch.float32, device=dev)
+            lead = (B, M, int(num_particles), H) if num_particles else (B, M, H)
+            obs = torch.empty(lead + (self.x_dim,), dtype=torch.float32, device=dev)
+            rew = torch.empty(lead, dtype=torch.float32, device=dev)
             nxt = torch.empty_like(obs)
         params = self._general(system_params)
         keys = keys.contiguous() if keys is not None else None

@@ -169,3 +169,19 @@ class MLPEnsembleSystem(System):
                                                       _lib.SUMMARIZE_MAX if use_optimism else _lib.SUMMARIZE_MEAN,
                                                       _lib.ptr(out), _lib.stream_ptr(x0.device)))
         return out
+
+    def ensemble_transitions(self, system_params: SystemParams, init_state: torch.Tensor, actions: torch.Tensor):
+        """init_state [B, X], actions [B, M, H, A] -> (obs [B, M, E, H, X], reward [B, M, E, H]): the Transition
+        fields of every member's rollout (obs[..., e, t, :] is the state before step t, obs[..., 0, :] = init_state)."""
+        pk = self.packed(system_params)
+        x0 = init_state.to(torch.float32).contiguous()
+        acts = actions.to(torch.float32).contiguous()
+        B, M, H, _ = acts.shape
+        E = system_params.dynamics_params.num_members
+        obs = torch.empty((B, M, E, H, self.x_dim), dtype=torch.float32, device=x0.device)
+        rew = torch.empty((B, M, E, H), dtype=torch.float32, device=x0.device)
+        with _lib.cuda_guard(x0):
+            _lib.check(_lib.lib.mbpo_ensemble_rollout_transitions(_lib.C.byref(pk.struct), H, _lib.ptr(x0),
+                                                                  _lib.ptr(acts), B, M, _lib.ptr(obs), _lib.ptr(rew),
+                                                                  _lib.stream_ptr(x0.device)))
+        return obs, rew
