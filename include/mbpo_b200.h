@@ -220,7 +220,9 @@ int mbpo_icem_plan(const MbpoIcemCfg* cfg_host, const void* sys_params_host,
  * iteration's noise under the rollouts (csrc/icem_cluster_kernels.cuh).  Results are bit-identical for every
  * cluster size.  cluster_size: -1 = the library's choice for (B, num_samples) -- what mbpo_icem_plan uses; 1 = one
  * CTA per problem; 2, 4, 8, 16 (at most 256 candidates per CTA).  mbpo_icem_plan_cluster_size returns that choice
- * (0 or 1: no cluster).
+ * (0 or 1: no cluster).  The general Systems (MBPO_SYSTEM_NOISY_PENDULUM, MBPO_SYSTEM_POINT_MASS) take the same sizes;
+ * their CTAs own candidate rows of num_samples + num_prev_elites and run one (candidate, particle) rollout per thread
+ * (csrc/icem_general_cluster_kernels.cuh), at most 256 rows per CTA.
  * Reference: icem_optimizer.py:134-252 at B = 1 is tests/test_icemopt.py's shape. */
 int mbpo_icem_plan_clustered(const MbpoIcemCfg* cfg_host, const void* sys_params_host, const float* x0,
                              const uint32_t* key_in, const float* best_seq_in, int B, float* best_seq_out,
@@ -274,6 +276,19 @@ int mbpo_icem_mpc_closed_loop_clustered(const MbpoIcemCfg* cfg_host, const void*
                                         const uint32_t* key_in, const float* best_seq_in, int B, int num_mpc_steps,
                                         float* states_out, float* rewards_out, float* actions_out,
                                         float* best_seq_out, uint32_t* key_out, int cluster_size, void* stream);
+/* The closed loop over a general System (MBPO_SYSTEM_NOISY_PENDULUM, MBPO_SYSTEM_POINT_MASS) in one launch: T times
+ * { plan; System.step on the plan's first action with the problem's own System key; warm start }.  A System that
+ * draws (NoisyPendulum) needs sys_keys_in, its system_params.key, and advances it exactly as system.step does;
+ * sys_keys_out (optional) receives the key after the last step.  A System that does not draw ignores the keys and
+ * passes them through.  T = 0 passes x0's plan state through (best_seq_out = best_seq_in, key_out = key_in).
+ * cluster_size as in mbpo_icem_plan_clustered; every size gives the same bits. */
+int mbpo_icem_mpc_closed_loop_general(const MbpoIcemCfg* cfg_host, const MbpoGeneralSystemParams* sys_params_host,
+                                      const float* x0 /*[B,X]*/, const uint32_t* key_in /*[B,2]*/,
+                                      const float* best_seq_in /*[B,H,A]*/, const uint32_t* sys_keys_in /*[B,2]|NULL*/,
+                                      int B, int num_mpc_steps, float* states_out /*[T,B,X]*/,
+                                      float* rewards_out /*[T,B]*/, float* actions_out /*[T,B,A]*/,
+                                      float* best_seq_out /*[B,H,A]*/, uint32_t* key_out /*[B,2]*/,
+                                      uint32_t* sys_keys_out /*[B,2]|NULL*/, int cluster_size, void* stream);
 
 
 /* ---- vmapped env rollouts for SAC/PPO collection ---------------------------------------- */

@@ -438,147 +438,284 @@ struct GenPlanSmem {
   }
 };
 
+// Shared-memory carve-up of one general planning CTA (GenPlanSmem::bytes; the closed loop appends GenMpcExtra).
+template <int H, int A>
+struct GenCtaSmem {
+  float* act;            // [N + 1][RS], row N all zeros
+  uint32_t* skey;        // [M]
+  float* mean;           // [H*A] in the ABI's (t, a) order
+  float* std_;
+  float* best_seq;
+  int* elite_idx;
+  int* sel_idx;
+  uint32_t* scratch;
+  float* best_value;
+  uint32_t* carry;
+  __device__ __forceinline__ GenCtaSmem(uint32_t* base, int N, int M, int K) {
+    constexpr int D = H * A, RS = GenPlanSmem<H, A>::RS;
+    act = reinterpret_cast<float*>(base);
+    skey = base + static_cast<size_t>(N + 1) * RS;
+    mean = reinterpret_cast<float*>(skey + M);
+    std_ = mean + D;
+    best_seq = std_ + D;
+    elite_idx = reinterpret_cast<int*>(best_seq + D);
+    sel_idx = elite_idx + K;
+    scratch = reinterpret_cast<uint32_t*>(sel_idx + K);
+    best_value = reinterpret_cast<float*>(scratch + select_scratch_words(K, M));
+    carry = reinterpret_cast<uint32_t*>(best_value + 1);
+  }
+};
+
+// iCemTO.optimize for ONE problem over a general System, executed by the whole CTA: initial state s0, warm-start
+// sequence `prev` ([H*A], must not alias sm.best_seq), opt_state.key `key_in`; the new opt_state.key is returned
+// through k_new (valid in thread 0 only), the best sequence / value are left in sm.  `slot` of `slots` indexes the
+// trace dumps ([S, slots, ...]).  Ends with a barrier.
+template <class Sys, int H, int PRNG>
+__device__ __forceinline__ void plan_problem_general(const PlanArgs& a, const GenCtaSmem<H, Sys::A>& sm, const Sys& sys,
+                                                     const RefitScalars& rs, const float (&s0)[Sys::X],
+                                                     const float* prev, Key2 key_in, Key2& k_new, int slot, int slots) {
+  constexpr int A = Sys::A, X = Sys::X, D = H * A, RS = GenPlanSmem<H, A>::RS, THREADS = 256;
+  const int N = a.N, M = a.N + a.Np, K = a.K;
+  float* act = sm.act;
+  uint32_t* skey = sm.skey;
+  float* mean = sm.mean;
+  float* std_ = sm.std_;
+  float* best_seq = sm.best_seq;
+  int* elite_idx = sm.elite_idx;
+  float* best_value = sm.best_value;
+  uint32_t* carry = sm.carry;
+  const int tid = threadIdx.x;
+  // element d = t * A + ad of candidate i (ABI order) in the dimension-major shared row
+  auto elem = [&](int i, int d) { return i < N ? act[static_cast<size_t>(i) * RS + (d % A) * H + d / A] : 0.0f; };
+
+  // ---- prologue (:235-249): warm start shifts by one step = A elements --------------------------------
+  for (int d = tid; d < D; d += THREADS) {
+    float m = 0.0f;
+    if (a.warm_start) m = prev[(d + A < D) ? d + A : (D - A + d % A)];
+    mean[d] = m;
+    std_[d] = a.init_std;
+    best_seq[d] = m;
+  }
+  for (int d = tid; d < RS; d += THREADS) act[static_cast<size_t>(N) * RS + d] = 0.0f;
+  k_new = Key2{0u, 0u};
+  if (tid == 0) {
+    *best_value = __int_as_float(0xFF800000);
+    Key2 k_opt;
+    split2<PRNG>(key_in, k_opt, k_new);
+    carry[0] = k_opt.k0;
+    carry[1] = k_opt.k1;
+  }
+  __syncthreads();
+  float zero_value = 0.0f;   // deterministic System: the objective of the all-zero row, computed once (thread 0)
+
+  for (int it = 0; it < a.S; ++it) {
+    const size_t tslot = static_cast<size_t>(it) * slots + slot;
+    Key2 ck{carry[0], carry[1]}, sampling_rng, particles_rng;
+    split2<PRNG>(ck, sampling_rng, particles_rng);                                            // :174
+    __syncthreads();  // every thread has read carry
+    if (tid == 0) {
+      const Key2 nk = split_at<PRNG>(sampling_rng, static_cast<uint32_t>(N + 1), 0u);         // :176
+      carry[0] = nk.k0;
+      carry[1] = nk.k1;
+    }
+    // candidates 0 .. N-1 are sampled; N .. M-1 are the zero rows (rolled out only if the System draws, or once)
+    const int jobs = Sys::KEYED ? M : ((it == 0) ? N + 1 : N);
+    for (int n = tid; n < jobs; n += THREADS) {
+      float* row = act + static_cast<size_t>(n < N ? n : N) * RS;
+      if (n < N) {
+        const Key2 sk = split_at<PRNG>(sampling_rng, static_cast<uint32_t>(N + 1), static_cast<uint32_t>(n + 1));
+#pragma unroll 1
+        for (int ad = 0; ad < A; ++ad) {
+          const Key2 dk = split_at<PRNG>(sk, static_cast<uint32_t>(A), static_cast<uint32_t>(ad));   // :180
+          float* dim = row + ad * H;
+          colored_noise_row<H, PRNG>(dk, a.scale, dim, nullptr, [&](int t, float y) {
+            const float v = __fadd_rn(mean[t * A + ad], __fmul_rn(y, std_[t * A + ad]));              // :190
+            dim[t] = fminf(fmaxf(v, a.u_min), a.u_max);                                               // :191
+          });
+        }
+      }
+      // ---- objective (:144-160) ----------------------------------------------------------------------
+      float val;
+      auto roll = [&](Key2 key) {
+        float s[X];
+#pragma unroll
+        for (int k = 0; k < X; ++k) s[k] = s0[k];
+        float acc = 0.0f;
+        for (int t = 0; t < H; ++t) acc = __fadd_rn(acc, sys.template step<PRNG>(s, row + t, H, key));
+        return __fdiv_rn(acc, static_cast<float>(H));
+      };
+      if (!Sys::KEYED) {
+        const float ret = roll(Key2{0u, 0u});
+        if (a.summarize == MBPO_SUMMARIZE_MAX || a.P == 1) {
+          val = ret;
+        } else {
+          float acc = 0.0f;
+          for (int p = 0; p < a.P; ++p) acc = __fadd_rn(acc, ret);
+          val = __fdiv_rn(acc, static_cast<float>(a.P));
+        }
+      } else {
+        const Key2 pkey = split_at<PRNG>(particles_rng, static_cast<uint32_t>(M), static_cast<uint32_t>(n));   // :177
+        float acc = 0.0f, mx = 0.0f;
+        for (int p = 0; p < a.P; ++p) {
+          const float ret = roll(split_at<PRNG>(pkey, static_cast<uint32_t>(a.P), static_cast<uint32_t>(p)));  // :155
+          acc = __fadd_rn(acc, ret);
+          mx = (p == 0) ? ret : fmaxf(mx, ret);
+        }
+        val = (a.summarize == MBPO_SUMMARIZE_MAX) ? mx : __fdiv_rn(acc, static_cast<float>(a.P));
+      }
+      if (n < N || Sys::KEYED) {
+        skey[n] = total_order_key(val);
+        if (a.trace.values) a.trace.values[tslot * M + n] = val;
+      } else {
+        zero_value = val;                                   // n == N, deterministic System, iteration 0: thread N % THREADS
+        for (int j = N; j < M; ++j) skey[j] = total_order_key(val);
+      }
+      if (a.trace.actions) {
+        float* dst = a.trace.actions + (tslot * M + n) * D;
+        for (int d = 0; d < D; ++d) dst[d] = (n < N) ? row[(d % A) * H + d / A] : 0.0f;
+      }
+    }
+    __syncthreads();
+    if (!Sys::KEYED && (a.trace.values || a.trace.actions)) {   // the zero rows' dumps (one value serves them all)
+      const float zv = value_of_key(skey[N]);
+      for (int j = N + tid; j < M; j += THREADS) {
+        if (a.trace.values) a.trace.values[tslot * M + j] = zv;
+        if (a.trace.actions && !(j == N && it == 0)) {
+          float* dst = a.trace.actions + (tslot * M + j) * D;
+          for (int d = 0; d < D; ++d) dst[d] = 0.0f;
+        }
+      }
+    }
+    (void)zero_value;
+    cta_select_refit<THREADS>(rs, skey, elite_idx, sm.sel_idx, sm.scratch, elem, mean, std_, best_seq, best_value);
+    if (a.trace.elite_idx)
+      for (int e = tid; e < K; e += THREADS) a.trace.elite_idx[tslot * K + e] = elite_idx[e];
+    for (int d = tid; d < D; d += THREADS) {
+      if (a.trace.mean) a.trace.mean[tslot * D + d] = mean[d];
+      if (a.trace.std) a.trace.std[tslot * D + d] = std_[d];
+    }
+    if (a.trace.best_value && tid == 0) a.trace.best_value[tslot] = *best_value;
+    __syncthreads();
+  }
+}
+
 template <class Sys, int H, int PRNG>
 __global__ void __launch_bounds__(256, 1) icem_plan_general_kernel(const __grid_constant__ PlanArgs a) {
-  constexpr int A = Sys::A, X = Sys::X, D = H * A, RS = GenPlanSmem<H, A>::RS, THREADS = 256;
+  constexpr int A = Sys::A, X = Sys::X, D = H * A, THREADS = 256;
   extern __shared__ __align__(16) uint32_t smem_u32[];
   const int N = a.N, M = a.N + a.Np, K = a.K;
-  float* act = reinterpret_cast<float*>(smem_u32);               // [N + 1][RS], row N all zeros
-  uint32_t* skey = smem_u32 + static_cast<size_t>(N + 1) * RS;   // [M]
-  float* mean = reinterpret_cast<float*>(skey + M);              // [H*A] in the ABI's (t, a) order
-  float* std_ = mean + D;
-  float* best_seq = std_ + D;
-  int* elite_idx = reinterpret_cast<int*>(best_seq + D);
-  int* sel_idx = elite_idx + K;
-  uint32_t* scratch = reinterpret_cast<uint32_t*>(sel_idx + K);
-  float* best_value = reinterpret_cast<float*>(scratch + select_scratch_words(K, M));
-  uint32_t* carry = reinterpret_cast<uint32_t*>(best_value + 1);
+  const GenCtaSmem<H, A> sm(smem_u32, N, M, K);
   const int tid = threadIdx.x;
   const Sys sys(a.gsys);
   RefitScalars rs;
   rs.M = M; rs.K = K; rs.D = D; rs.alpha = a.alpha; rs.one_minus_alpha = a.one_minus_alpha;
-  // element d = t * A + ad of candidate i (ABI order) in the dimension-major shared row
-  auto elem = [&](int i, int d) { return i < N ? act[static_cast<size_t>(i) * RS + (d % A) * H + d / A] : 0.0f; };
 
   for (int b = blockIdx.x; b < a.B; b += gridDim.x) {
     float s0[X];
 #pragma unroll
     for (int k = 0; k < X; ++k) s0[k] = a.x0[static_cast<size_t>(b) * X + k];
-    // ---- prologue (:235-249): warm start shifts by one step = A elements --------------------------------
-    const float* prev = a.best_seq_in + static_cast<size_t>(b) * D;
-    for (int d = tid; d < D; d += THREADS) {
-      float m = 0.0f;
-      if (a.warm_start) m = prev[(d + A < D) ? d + A : (D - A + d % A)];
-      mean[d] = m;
-      std_[d] = a.init_std;
-      best_seq[d] = m;
-    }
-    for (int d = tid; d < RS; d += THREADS) act[static_cast<size_t>(N) * RS + d] = 0.0f;
-    Key2 k_new{0u, 0u};
+    Key2 k_new;
+    plan_problem_general<Sys, H, PRNG>(a, sm, sys, rs, s0, a.best_seq_in + static_cast<size_t>(b) * D,
+                                       Key2{a.key_in[2 * b], a.key_in[2 * b + 1]}, k_new, b, a.B);
+    for (int d = tid; d < D; d += THREADS) a.best_seq_out[static_cast<size_t>(b) * D + d] = sm.best_seq[d];
     if (tid == 0) {
-      *best_value = __int_as_float(0xFF800000);
-      Key2 k_opt;
-      split2<PRNG>(Key2{a.key_in[2 * b], a.key_in[2 * b + 1]}, k_opt, k_new);
-      carry[0] = k_opt.k0;
-      carry[1] = k_opt.k1;
-    }
-    __syncthreads();
-    float zero_value = 0.0f;   // deterministic System: the objective of the all-zero row, computed once (thread 0)
-
-    for (int it = 0; it < a.S; ++it) {
-      const size_t tslot = static_cast<size_t>(it) * a.B + b;
-      Key2 ck{carry[0], carry[1]}, sampling_rng, particles_rng;
-      split2<PRNG>(ck, sampling_rng, particles_rng);                                            // :174
-      __syncthreads();  // every thread has read carry
-      if (tid == 0) {
-        const Key2 nk = split_at<PRNG>(sampling_rng, static_cast<uint32_t>(N + 1), 0u);         // :176
-        carry[0] = nk.k0;
-        carry[1] = nk.k1;
-      }
-      // candidates 0 .. N-1 are sampled; N .. M-1 are the zero rows (rolled out only if the System draws, or once)
-      const int jobs = Sys::KEYED ? M : ((it == 0) ? N + 1 : N);
-      for (int n = tid; n < jobs; n += THREADS) {
-        float* row = act + static_cast<size_t>(n < N ? n : N) * RS;
-        if (n < N) {
-          const Key2 sk = split_at<PRNG>(sampling_rng, static_cast<uint32_t>(N + 1), static_cast<uint32_t>(n + 1));
-#pragma unroll 1
-          for (int ad = 0; ad < A; ++ad) {
-            const Key2 dk = split_at<PRNG>(sk, static_cast<uint32_t>(A), static_cast<uint32_t>(ad));   // :180
-            float* dim = row + ad * H;
-            colored_noise_row<H, PRNG>(dk, a.scale, dim, nullptr, [&](int t, float y) {
-              const float v = __fadd_rn(mean[t * A + ad], __fmul_rn(y, std_[t * A + ad]));              // :190
-              dim[t] = fminf(fmaxf(v, a.u_min), a.u_max);                                               // :191
-            });
-          }
-        }
-        // ---- objective (:144-160) ----------------------------------------------------------------------
-        float val;
-        auto roll = [&](Key2 key) {
-          float s[X];
-#pragma unroll
-          for (int k = 0; k < X; ++k) s[k] = s0[k];
-          float acc = 0.0f;
-          for (int t = 0; t < H; ++t) acc = __fadd_rn(acc, sys.template step<PRNG>(s, row + t, H, key));
-          return __fdiv_rn(acc, static_cast<float>(H));
-        };
-        if (!Sys::KEYED) {
-          const float ret = roll(Key2{0u, 0u});
-          if (a.summarize == MBPO_SUMMARIZE_MAX || a.P == 1) {
-            val = ret;
-          } else {
-            float acc = 0.0f;
-            for (int p = 0; p < a.P; ++p) acc = __fadd_rn(acc, ret);
-            val = __fdiv_rn(acc, static_cast<float>(a.P));
-          }
-        } else {
-          const Key2 pkey = split_at<PRNG>(particles_rng, static_cast<uint32_t>(M), static_cast<uint32_t>(n));   // :177
-          float acc = 0.0f, mx = 0.0f;
-          for (int p = 0; p < a.P; ++p) {
-            const float ret = roll(split_at<PRNG>(pkey, static_cast<uint32_t>(a.P), static_cast<uint32_t>(p)));  // :155
-            acc = __fadd_rn(acc, ret);
-            mx = (p == 0) ? ret : fmaxf(mx, ret);
-          }
-          val = (a.summarize == MBPO_SUMMARIZE_MAX) ? mx : __fdiv_rn(acc, static_cast<float>(a.P));
-        }
-        if (n < N || Sys::KEYED) {
-          skey[n] = total_order_key(val);
-          if (a.trace.values) a.trace.values[tslot * M + n] = val;
-        } else {
-          zero_value = val;                                   // n == N, deterministic System, iteration 0: thread N % THREADS
-          for (int j = N; j < M; ++j) skey[j] = total_order_key(val);
-        }
-        if (a.trace.actions) {
-          float* dst = a.trace.actions + (tslot * M + n) * D;
-          for (int d = 0; d < D; ++d) dst[d] = (n < N) ? row[(d % A) * H + d / A] : 0.0f;
-        }
-      }
-      __syncthreads();
-      if (!Sys::KEYED && (a.trace.values || a.trace.actions)) {   // the zero rows' dumps (one value serves them all)
-        const float zv = value_of_key(skey[N]);
-        for (int j = N + tid; j < M; j += THREADS) {
-          if (a.trace.values) a.trace.values[tslot * M + j] = zv;
-          if (a.trace.actions && !(j == N && it == 0)) {
-            float* dst = a.trace.actions + (tslot * M + j) * D;
-            for (int d = 0; d < D; ++d) dst[d] = 0.0f;
-          }
-        }
-      }
-      (void)zero_value;
-      cta_select_refit<THREADS>(rs, skey, elite_idx, sel_idx, scratch, elem, mean, std_, best_seq, best_value);
-      if (a.trace.elite_idx)
-        for (int e = tid; e < K; e += THREADS) a.trace.elite_idx[tslot * K + e] = elite_idx[e];
-      for (int d = tid; d < D; d += THREADS) {
-        if (a.trace.mean) a.trace.mean[tslot * D + d] = mean[d];
-        if (a.trace.std) a.trace.std[tslot * D + d] = std_[d];
-      }
-      if (a.trace.best_value && tid == 0) a.trace.best_value[tslot] = *best_value;
-      __syncthreads();
-    }
-    for (int d = tid; d < D; d += THREADS) a.best_seq_out[static_cast<size_t>(b) * D + d] = best_seq[d];
-    if (tid == 0) {
-      a.best_value_out[b] = *best_value;
+      a.best_value_out[b] = *sm.best_value;
       a.key_out[2 * b] = k_new.k0;
       a.key_out[2 * b + 1] = k_new.k1;
+    }
+    __syncthreads();
+  }
+}
+
+// Closed-loop MPC over a general System (tests/test_icemopt.py:19-32): T times { plan; the true System.step on the
+// first action with the problem's own System key (a System that draws advances it as system.step does); warm start }.
+struct GeneralMpcArgs {
+  int T;
+  float* states_out;           // [T,B,X]
+  float* rewards_out;          // [T,B]
+  float* actions_out;          // [T,B,A]
+  const uint32_t* sys_key_in;  // [B,2] or null (a System that does not draw)
+  uint32_t* sys_key_out;       // [B,2] or null
+};
+
+// Words the closed loop keeps besides a plan's shared memory: the warm-start sequence [H*A], the true state [<= 4],
+// the planner key [2] and the System key [2].
+template <int H, int A>
+constexpr int gen_mpc_extra_words() { return H * A + 8; }
+
+// One problem's true System.step on the first action of best_seq (ABI order: the A elements of t = 0), in thread
+// `tid == 0` of the caller; x and key are updated in place and the outputs of MPC step t are written if `write`.
+template <class Sys, int PRNG>
+__device__ __forceinline__ void general_mpc_step(const Sys& sys, const GeneralMpcArgs& m, int B, int b, int t,
+                                                 const float* best_seq, float* x, uint32_t* key, bool write) {
+  constexpr int X = Sys::X, A = Sys::A;
+  float s[X], u[A];
+#pragma unroll
+  for (int k = 0; k < X; ++k) s[k] = x[k];
+#pragma unroll
+  for (int k = 0; k < A; ++k) u[k] = best_seq[k];                           // opt_state.action (:67-69)
+  Key2 sk{key[0], key[1]};
+  const float r = sys.template step<PRNG>(s, u, 1, sk);
+#pragma unroll
+  for (int k = 0; k < X; ++k) x[k] = s[k];
+  key[0] = sk.k0;
+  key[1] = sk.k1;
+  if (write) {
+    const size_t o = static_cast<size_t>(t) * B + b;
+#pragma unroll
+    for (int k = 0; k < X; ++k)
+      if (m.states_out) m.states_out[o * X + k] = s[k];
+    if (m.rewards_out) m.rewards_out[o] = r;
+#pragma unroll
+    for (int k = 0; k < A; ++k)
+      if (m.actions_out) m.actions_out[o * A + k] = u[k];
+  }
+}
+
+// The closed loop, one CTA per problem (grid-stride over problems), the whole loop in one launch.
+template <class Sys, int H, int PRNG>
+__global__ void __launch_bounds__(256, 1)
+    icem_mpc_general_kernel(const __grid_constant__ PlanArgs a, const __grid_constant__ GeneralMpcArgs m) {
+  constexpr int A = Sys::A, X = Sys::X, D = H * A, THREADS = 256;
+  extern __shared__ __align__(16) uint32_t smem_u32[];
+  const int N = a.N, M = a.N + a.Np, K = a.K;
+  const GenCtaSmem<H, A> sm(smem_u32, N, M, K);
+  float* prev = sm.best_value + 8;                              // [D] warm-start sequence of the next plan
+  float* xs = prev + D;                                         // [4] true state
+  uint32_t* pkey = reinterpret_cast<uint32_t*>(xs + 4);         // [2] opt_state.key
+  uint32_t* syskey = pkey + 2;                                  // [2] system_params.key
+  const int tid = threadIdx.x;
+  const Sys sys(a.gsys);
+  RefitScalars rs;
+  rs.M = M; rs.K = K; rs.D = D; rs.alpha = a.alpha; rs.one_minus_alpha = a.one_minus_alpha;
+
+  for (int b = blockIdx.x; b < a.B; b += gridDim.x) {
+    for (int d = tid; d < D; d += THREADS) prev[d] = a.best_seq_in[static_cast<size_t>(b) * D + d];
+    if (tid < X) xs[tid] = a.x0[static_cast<size_t>(b) * X + tid];
+    if (tid == 0) {
+      pkey[0] = a.key_in[2 * b]; pkey[1] = a.key_in[2 * b + 1];
+      syskey[0] = m.sys_key_in ? m.sys_key_in[2 * b] : 0u;
+      syskey[1] = m.sys_key_in ? m.sys_key_in[2 * b + 1] : 0u;
+    }
+    __syncthreads();
+    for (int t = 0; t < m.T; ++t) {
+      float s0[X];
+#pragma unroll
+      for (int k = 0; k < X; ++k) s0[k] = xs[k];
+      Key2 k_new;
+      plan_problem_general<Sys, H, PRNG>(a, sm, sys, rs, s0, prev, Key2{pkey[0], pkey[1]}, k_new, 0, 1);
+      if (tid == 0) {
+        pkey[0] = k_new.k0; pkey[1] = k_new.k1;
+        general_mpc_step<Sys, PRNG>(sys, m, a.B, b, t, sm.best_seq, xs, syskey, true);
+      }
+      for (int d = tid; d < D; d += THREADS) prev[d] = sm.best_seq[d];
+      __syncthreads();
+    }
+    for (int d = tid; d < D; d += THREADS) a.best_seq_out[static_cast<size_t>(b) * D + d] = prev[d];
+    if (tid == 0) {
+      a.key_out[2 * b] = pkey[0];
+      a.key_out[2 * b + 1] = pkey[1];
+      if (m.sys_key_out) { m.sys_key_out[2 * b] = syskey[0]; m.sys_key_out[2 * b + 1] = syskey[1]; }
     }
     __syncthreads();
   }

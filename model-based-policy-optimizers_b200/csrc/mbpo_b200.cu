@@ -195,11 +195,13 @@ int plan_fusable(const MbpoIcemCfg* c, bool set_error) {
 struct ClusterCaps { int cap[4]; };
 ClusterCaps cluster_caps(const MbpoIcemCfg* c, bool mpc) {
   static std::mutex mu;
-  static std::map<std::tuple<int, int, int, int, int, int, int, int>, ClusterCaps> cache;
+  static std::map<std::tuple<int, int, int, int, int, int, int, int, int, int>, ClusterCaps> cache;
   int dev = 0;
   cudaGetDevice(&dev);
-  const auto key = std::make_tuple(dev, c->horizon, c->prng_mode, c->math_mode, mpc ? 1 : 0, c->num_samples,
-                                   c->num_prev_elites, c->num_elites);
+  const bool general = general_plan_kind(c->system_kind);
+  // the general cluster kernels' block size depends on the particles as well
+  const auto key = std::make_tuple(dev, c->system_kind, c->horizon, c->prng_mode, c->math_mode, mpc ? 1 : 0,
+                                   c->num_samples, c->num_prev_elites, c->num_elites, general ? c->num_particles : 0);
   std::lock_guard<std::mutex> lock(mu);
   const auto it = cache.find(key);
   if (it != cache.end()) return it->second;
@@ -210,8 +212,11 @@ ClusterCaps cluster_caps(const MbpoIcemCfg* c, bool mpc) {
     switch (c->horizon) {
 #define X(h)                                                                                                      \
   case h:                                                                                                         \
-    caps.cap[i] = plan_cluster_capacity<h>(c->prng_mode, c->math_mode, mpc, c->num_samples, c->num_prev_elites, \
-                                           c->num_elites, cl);                                                    \
+    caps.cap[i] = general ? general_plan_cluster_capacity<h>(c->system_kind, c->prng_mode, mpc, c->num_samples,   \
+                                                             c->num_prev_elites, c->num_elites, c->num_particles,  \
+                                                             cl)                                                   \
+                          : plan_cluster_capacity<h>(c->prng_mode, c->math_mode, mpc, c->num_samples,             \
+                                                     c->num_prev_elites, c->num_elites, cl);                      \
     break;
       MBPO_FOR_EACH_H(X)
 #undef X
@@ -220,6 +225,69 @@ ClusterCaps cluster_caps(const MbpoIcemCfg* c, bool mpc) {
   }
   cache[key] = caps;
   return caps;
+}
+
+// The cluster size to run: the caller's, or for -1 the library's choice for B problems (0 / 1: one CTA each).
+int plan_cluster_size(const MbpoIcemCfg* c, int B, bool mpc, int cluster_size) {
+  if (cluster_size >= 0) return cluster_size;
+  if (!horizon_supported(c->horizon) || c->num_samples + c->num_prev_elites < 36) return 0;
+  const ClusterCaps caps = cluster_caps(c, mpc);
+  return plan_cluster_choice(B, c->num_samples, caps.cap);
+}
+
+// Runs dispatch(cluster) and, where the library chose the size and the device refuses it, falls back: a refused 16
+// runs at 8, a refused cluster at one CTA per problem (the same bits).
+template <class F>
+int dispatch_with_fallback(int cluster, int cluster_size, F&& dispatch) {
+  int rc = dispatch(cluster);
+  if (rc == MBPO_ECUDA && cluster_size < 0 && cluster == 16) {
+    cudaGetLastError();                 // the device refused the non-portable size the library picked: use 8
+    cluster = 8;
+    rc = dispatch(8);
+  }
+  if (rc == MBPO_ECUDA && cluster_size < 0 && cluster > 1) {
+    cudaGetLastError();                 // no cluster of the library's own choice can be placed (e.g. a partitioned
+    rc = dispatch(1);                   // device): the one-CTA kernel gives the same bits
+  }
+  return rc;
+}
+
+// The cluster sizes a plan takes: 2, 4, 8, 16, with the population limits of the cluster kernels.
+int check_cluster_size(const MbpoIcemCfg* c, int cluster) {
+  MBPO_REQUIRE(cluster == 2 || cluster == 4 || cluster == 8 || cluster == 16,
+               "plan: cluster_size %d (use -1, 1, 2, 4, 8 or 16)", cluster);
+  const int N = c->num_samples, Np = c->num_prev_elites;
+  // the pendulum's CTAs own candidates of N, the general Systems' candidate rows of N + Np
+  const int R = ((general_plan_kind(c->system_kind) ? N + Np : N) + cluster - 1) / cluster;
+  if (R > 256) return fail(MBPO_EUNSUPPORTED, "plan: %d candidates per CTA of a %d-cluster (at most 256)", R, cluster);
+  if (N + Np < 36)   // the cluster kernel keeps its elite list in the selection scratch (words 299 .. 300 + K)
+    return fail(MBPO_EUNSUPPORTED, "plan: population (%d + %d) outside what a %d-cluster handles", N, Np, cluster);
+  return MBPO_OK;
+}
+
+// Fused plan (gm == nullptr) or closed loop over a general System.
+int run_general_plan(const MbpoIcemCfg* c, const MbpoGeneralSystemParams* gp, const float* x0, const uint32_t* key_in,
+                     const float* best_seq_in, int B, float* best_seq_out, float* best_value_out, uint32_t* key_out,
+                     const MbpoIcemTrace* trace, const GeneralMpcArgs* gm, int cluster_size, void* stream) {
+  PlanArgs g;
+  fill_plan_args(g, c, nullptr, x0, key_in, best_seq_in, B, best_seq_out, best_value_out, key_out, trace);
+  g.gsys = *gp;
+  const int cluster = plan_cluster_size(c, B, gm != nullptr, cluster_size);
+  if (cluster > 1) {
+    const int rc = check_cluster_size(c, cluster);
+    if (rc != MBPO_OK) return rc;
+  }
+  return dispatch_with_fallback(cluster, cluster_size, [&](int cl) -> int {
+    switch (c->horizon) {
+#define X(h) \
+  case h:    \
+    return general_plan_entry<h>(c->system_kind, c->prng_mode, g, gm, as_stream(stream), cl);
+      MBPO_FOR_EACH_H(X)
+#undef X
+      default:
+        return fail(MBPO_EUNSUPPORTED, "horizon %d has no compiled kernel", c->horizon);
+    }
+  });
 }
 
 int run_plan(const MbpoIcemCfg* c, const void* sys_params_host, const float* x0, const uint32_t* key_in,
@@ -234,19 +302,10 @@ int run_plan(const MbpoIcemCfg* c, const void* sys_params_host, const float* x0,
   MBPO_REQUIRE(mpc != nullptr || best_value_out != nullptr, "plan: best_value_out is null");
   if (general_plan_kind(c->system_kind)) {
     if (mpc != nullptr)
-      return fail(MBPO_EUNSUPPORTED, "closed loop in one launch exists for the pendulum System only");
-    PlanArgs g;
-    fill_plan_args(g, c, nullptr, x0, key_in, best_seq_in, B, best_seq_out, best_value_out, key_out, trace);
-    g.gsys = *static_cast<const MbpoGeneralSystemParams*>(sys_params_host);
-    switch (c->horizon) {
-#define X(h) \
-  case h:    \
-    return general_plan_entry<h>(c->system_kind, c->prng_mode, g, as_stream(stream));
-      MBPO_FOR_EACH_H(X)
-#undef X
-      default:
-        return fail(MBPO_EUNSUPPORTED, "horizon %d has no compiled kernel", c->horizon);
-    }
+      return fail(MBPO_EUNSUPPORTED, "closed loop over a general System: use mbpo_icem_mpc_closed_loop_general, "
+                  "which carries the System's keys");
+    return run_general_plan(c, static_cast<const MbpoGeneralSystemParams*>(sys_params_host), x0, key_in, best_seq_in,
+                            B, best_seq_out, best_value_out, key_out, trace, nullptr, cluster_size, stream);
   }
   // the fused kernel's reward wrap has no fmod slow path (pendulum.cuh wrap_diff<true>): |theta - target + pi| < 4 pi
   if (!(std::fabs(static_cast<const MbpoPendulumParams*>(sys_params_host)->target_angle) <= 6.0f))
@@ -255,27 +314,16 @@ int run_plan(const MbpoIcemCfg* c, const void* sys_params_host, const float* x0,
   fill_plan_args(a, c, static_cast<const MbpoPendulumParams*>(sys_params_host), x0, key_in, best_seq_in, B,
                  best_seq_out, best_value_out, key_out, trace);
   // few problems: spread each over a thread-block cluster (same bits; icem_cluster_kernels.cuh)
-  int cluster = cluster_size;
-  if (cluster < 0) {
-    cluster = 0;
-    if (horizon_supported(c->horizon) && a.N + a.Np >= 36) {
-      const ClusterCaps caps = cluster_caps(c, mpc != nullptr);
-      cluster = plan_cluster_choice(B, a.N, caps.cap);
-    }
-  }
+  const int cluster = plan_cluster_size(c, B, mpc != nullptr, cluster_size);
   if (!horizon_supported(c->horizon)) {
     if (cluster_size > 1) return fail(MBPO_EUNSUPPORTED, "plan: clusters exist for the unrolled horizons (" MBPO_H_LIST_STR ")");
     return plan_entry_rt(c->prng_mode, c->math_mode, a, mpc, as_stream(stream));
   }
   if (cluster > 1) {
-    MBPO_REQUIRE(cluster == 2 || cluster == 4 || cluster == 8 || cluster == 16,
-                 "plan: cluster_size %d (use -1, 1, 2, 4, 8 or 16)", cluster);
-    const int R = (a.N + cluster - 1) / cluster;
-    if (R > 256) return fail(MBPO_EUNSUPPORTED, "plan: %d candidates per CTA of a %d-cluster (at most 256)", R, cluster);
-    if (a.N + a.Np < 36)   // the cluster kernel keeps its elite list in the selection scratch (words 299 .. 300 + K)
-      return fail(MBPO_EUNSUPPORTED, "plan: population (%d + %d) outside what a %d-cluster handles", a.N, a.Np, cluster);
+    const int rc2 = check_cluster_size(c, cluster);
+    if (rc2 != MBPO_OK) return rc2;
   }
-  const auto dispatch = [&](int cl) -> int {
+  return dispatch_with_fallback(cluster, cluster_size, [&](int cl) -> int {
     switch (c->horizon) {
 #define X(h) \
   case h:    \
@@ -285,18 +333,7 @@ int run_plan(const MbpoIcemCfg* c, const void* sys_params_host, const float* x0,
       default:
         return fail(MBPO_EUNSUPPORTED, "horizon %d has no compiled kernel", c->horizon);
     }
-  };
-  int rc2 = dispatch(cluster);
-  if (rc2 == MBPO_ECUDA && cluster_size < 0 && cluster == 16) {
-    cudaGetLastError();                 // the device refused the non-portable size the library picked: use 8
-    cluster = 8;
-    rc2 = dispatch(8);
-  }
-  if (rc2 == MBPO_ECUDA && cluster_size < 0 && cluster > 1) {
-    cudaGetLastError();                 // no cluster of the library's own choice can be placed (e.g. a partitioned
-    rc2 = dispatch(1);                  // device): the one-CTA kernel gives the same bits
-  }
-  return rc2;
+  });
 }
 
 }  // namespace
@@ -640,17 +677,12 @@ int mbpo_icem_plan_clustered(const MbpoIcemCfg* cfg, const void* sys_params_host
 }
 
 int mbpo_icem_plan_cluster_size(const MbpoIcemCfg* cfg, int B) {
-  if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || !horizon_supported(cfg->horizon) ||
-      general_plan_kind(cfg->system_kind) || cfg->num_samples + cfg->num_prev_elites < 36)
-    return 0;
-  const ClusterCaps caps = cluster_caps(cfg, false);
-  return plan_cluster_choice(B, cfg->num_samples, caps.cap);
+  if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || B < 0) return 0;
+  return plan_cluster_size(cfg, B, false, -1);
 }
 
 int mbpo_icem_plan_cluster_capacity(const MbpoIcemCfg* cfg, int cluster_size) {
-  if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || !horizon_supported(cfg->horizon) ||
-      general_plan_kind(cfg->system_kind))
-    return 0;
+  if (validate_cfg(cfg) != MBPO_OK || !plan_fusable(cfg, false) || !horizon_supported(cfg->horizon)) return 0;
   const ClusterCaps caps = cluster_caps(cfg, false);
   switch (cluster_size) {
     case 16: return caps.cap[0];
@@ -829,6 +861,41 @@ int mbpo_icem_mpc_closed_loop_clustered(const MbpoIcemCfg* cfg, const void* sys_
   m.actions_out = actions_out;
   return run_plan(cfg, sys_params_host, x0, key_in, best_seq_in, B, best_seq_out, nullptr, key_out, nullptr, &m,
                   cluster_size, stream);
+}
+
+int mbpo_icem_mpc_closed_loop_general(const MbpoIcemCfg* cfg, const MbpoGeneralSystemParams* sys_params_host,
+                                      const float* x0, const uint32_t* key_in, const float* best_seq_in,
+                                      const uint32_t* sys_keys_in, int B, int num_mpc_steps, float* states_out,
+                                      float* rewards_out, float* actions_out, float* best_seq_out, uint32_t* key_out,
+                                      uint32_t* sys_keys_out, int cluster_size, void* stream) {
+  int rc = validate_cfg(cfg);
+  if (rc != MBPO_OK) return rc;
+  MBPO_REQUIRE(B >= 0, "mpc_closed_loop_general: B < 0");
+  MBPO_REQUIRE(num_mpc_steps >= 0, "mpc_closed_loop_general: num_mpc_steps < 0");
+  int X, A;
+  bool keyed = false;
+  if (!general_plan_kind(cfg->system_kind, &X, &A))
+    return fail(MBPO_EUNSUPPORTED, "mpc_closed_loop_general: system_kind %d is not a general System (the pendulum "
+                "has mbpo_icem_mpc_closed_loop)", cfg->system_kind);
+  general_system_dims(cfg->system_kind, &X, &A, &keyed);
+  if (!plan_fusable(cfg, true)) return MBPO_EUNSUPPORTED;
+  if (B == 0) return MBPO_OK;
+  MBPO_REQUIRE(sys_params_host && x0 && key_in && best_seq_in && best_seq_out && key_out,
+               "mpc_closed_loop_general: null pointer");
+  MBPO_REQUIRE(num_mpc_steps == 0 || (states_out && rewards_out && actions_out),
+               "mpc_closed_loop_general: null output");
+  MBPO_REQUIRE(!keyed || sys_keys_in, "mpc_closed_loop_general: system_kind %d draws from its key: sys_keys_in is null",
+               cfg->system_kind);
+  MBPO_REQUIRE(sys_keys_out == nullptr || sys_keys_in, "mpc_closed_loop_general: sys_keys_out without sys_keys_in");
+  GeneralMpcArgs m;
+  m.T = num_mpc_steps;
+  m.states_out = states_out;
+  m.rewards_out = rewards_out;
+  m.actions_out = actions_out;
+  m.sys_key_in = sys_keys_in;
+  m.sys_key_out = sys_keys_out;
+  return run_general_plan(cfg, sys_params_host, x0, key_in, best_seq_in, B, best_seq_out, nullptr, key_out, nullptr,
+                          &m, cluster_size, stream);
 }
 
 // ---- policy in the env loop: actor_step / generate_unroll / get_experience ------------------------------

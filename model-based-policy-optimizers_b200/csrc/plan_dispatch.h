@@ -4,6 +4,7 @@
 #pragma once
 #include "host_util.h"
 #include "icem_cluster_kernels.cuh"
+#include "icem_general_cluster_kernels.cuh"
 #include "icem_kernels.cuh"
 
 namespace mbpo {
@@ -17,9 +18,16 @@ int plan_entry(int prng_mode, int math_mode, const PlanArgs& a, const MpcArgs* m
 // The same for a horizon without an unrolled instance (plan_rt.cu; PlanArgs::H).
 int plan_entry_rt(int prng_mode, int math_mode, const PlanArgs& a, const MpcArgs* mpc, cudaStream_t st);
 
-// Fused plan over the general Systems (MBPO_SYSTEM_NOISY_PENDULUM, MBPO_SYSTEM_POINT_MASS): icem_plan_general_kernel.
+// Fused plan (mpc == nullptr) or closed-loop MPC over the general Systems (MBPO_SYSTEM_NOISY_PENDULUM,
+// MBPO_SYSTEM_POINT_MASS): one CTA per problem (cluster 0 / 1: icem_plan_general_kernel, icem_mpc_general_kernel) or
+// one cluster of that many CTAs per problem (icem_general_cluster_kernels.cuh; same bits).
 template <int H>
-int general_plan_entry(int system_kind, int prng_mode, const PlanArgs& a, cudaStream_t st);
+int general_plan_entry(int system_kind, int prng_mode, const PlanArgs& a, const GeneralMpcArgs* mpc, cudaStream_t st,
+                       int cluster);
+
+// plan_cluster_capacity for the general cluster kernels (their block size depends on the particles P as well).
+template <int H>
+int general_plan_cluster_capacity(int system_kind, int prng_mode, bool mpc, int N, int Np, int K, int P, int cluster);
 
 // How many clusters of `cluster` CTAs of the cluster plan (mpc: of the closed loop) run at once on the current device
 // (cudaOccupancyMaxActiveClusters: the GPCs, not the SM count, decide -- 7 of 16, 15 of 8, 33 of 4, 74 of 2 on a

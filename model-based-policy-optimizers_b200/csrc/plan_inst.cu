@@ -173,26 +173,135 @@ int plan_cluster_capacity<MBPO_INST_H>(int prng_mode, int math_mode, bool mpc, i
 
 namespace {
 template <class Sys, int PRNG>
-int launch_general(const PlanArgs& a, cudaStream_t st) {
-  const size_t smem = GenPlanSmem<kH, Sys::A>::bytes(a.N, a.Np, a.K);
-  auto kernel = icem_plan_general_kernel<Sys, kH, PRNG>;
+int launch_general(const PlanArgs& a, const GeneralMpcArgs* mpc, cudaStream_t st) {
+  const size_t smem = GenPlanSmem<kH, Sys::A>::bytes(a.N, a.Np, a.K) +
+                      (mpc ? 4 * gen_mpc_extra_words<kH, Sys::A>() : 0);
   if (smem > 227 * 1024) return fail(MBPO_EUNSUPPORTED, "general fused plan: %zu B of shared memory", smem);
-  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-  if (e != cudaSuccess) return fail(MBPO_ECUDA, "general plan smem attr (%zu): %s", smem, cudaGetErrorString(e));
-  int per_sm = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-  const long long resident = static_cast<long long>(per_sm) * device_sm_count();
-  const int grid = static_cast<int>(a.B < resident ? a.B : resident);
-  kernel<<<grid, 256, smem, st>>>(a);
-  return check_launch("icem_plan_general_kernel");
+  auto run = [&](auto kernel, const char* name, auto... extra) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    if (e != cudaSuccess) return fail(MBPO_ECUDA, "general plan smem attr (%zu): %s", smem, cudaGetErrorString(e));
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+    const long long resident = static_cast<long long>(per_sm) * device_sm_count();
+    const int grid = static_cast<int>(a.B < resident ? a.B : resident);
+    kernel<<<grid, 256, smem, st>>>(a, extra...);
+    return check_launch(name);
+  };
+  if (mpc == nullptr) return run(icem_plan_general_kernel<Sys, kH, PRNG>, "icem_plan_general_kernel");
+  return run(icem_mpc_general_kernel<Sys, kH, PRNG>, "icem_mpc_general_kernel", *mpc);
+}
+
+// Block size of a general cluster CTA with R rows of Pe rollouts and A action dimensions each: a thread per rollout
+// and per sampled noise row, at least 256 threads for the selection and the refit.
+int general_cluster_threads(int R, int Pe, int A) {
+  const int work = R * Pe > R * A ? R * Pe : R * A;
+  const int threads = (work + 31) / 32 * 32;
+  return threads < 256 ? 256 : (threads > CLUSTER_MAX_THREADS ? CLUSTER_MAX_THREADS : threads);
+}
+
+template <class Sys>
+size_t general_cluster_smem(int N, int Np, int K, int P, int cluster, int* R_out) {
+  const int R = (N + Np + cluster - 1) / cluster;
+  *R_out = R;
+  return cluster_smem_alloc(GenClusterSmem<kH, Sys::A>::bytes(R, Sys::KEYED ? P : 1, N, Np, K));
+}
+
+cudaLaunchConfig_t cluster_launch_config(int clusters, int cluster, int threads, size_t smem, cudaStream_t st,
+                                         cudaLaunchAttribute* attr) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(static_cast<unsigned>(clusters * cluster), 1, 1);
+  cfg.blockDim = dim3(static_cast<unsigned>(threads), 1, 1);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = static_cast<unsigned>(cluster);
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cfg;
+}
+
+template <class Sys, int PRNG>
+int general_cluster_capacity(bool mpc, int N, int Np, int K, int P, int cluster) {
+  int R = 0;
+  const size_t smem = general_cluster_smem<Sys>(N, Np, K, P, cluster, &R);
+  if (R > 256 || smem > 227 * 1024) return 0;
+  cudaLaunchAttribute attr[1];
+  const cudaLaunchConfig_t cfg = cluster_launch_config(1, cluster, general_cluster_threads(R, Sys::KEYED ? P : 1, Sys::A),
+                                                       smem, nullptr, attr);
+  int n = 0;
+  cudaError_t e;
+  if (mpc) {
+    auto kernel = icem_mpc_general_cluster_kernel<Sys, kH, PRNG>;
+    e = prepare_cluster_kernel(kernel, cluster, smem);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveClusters(&n, kernel, &cfg);
+  } else {
+    auto kernel = icem_plan_general_cluster_kernel<Sys, kH, PRNG>;
+    e = prepare_cluster_kernel(kernel, cluster, smem);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveClusters(&n, kernel, &cfg);
+  }
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
+  }
+  return n;
+}
+
+// One problem per cluster of `cluster` CTAs (icem_general_cluster_kernels.cuh).
+template <class Sys, int PRNG>
+int launch_general_cluster(const PlanArgs& a, const GeneralMpcArgs* mpc, cudaStream_t st, int cluster) {
+  int R = 0;
+  const size_t smem = general_cluster_smem<Sys>(a.N, a.Np, a.K, a.P, cluster, &R);
+  if (R > 256)
+    return fail(MBPO_EUNSUPPORTED, "plan: %d candidate rows per CTA of a %d-cluster (at most 256)", R, cluster);
+  if (smem > 227 * 1024) return fail(MBPO_EUNSUPPORTED, "general cluster plan: %zu B of shared memory", smem);
+  const int threads = general_cluster_threads(R, Sys::KEYED ? a.P : 1, Sys::A);
+  long long clusters = device_sm_count() / cluster;
+  if (clusters > a.B) clusters = a.B;
+  cudaLaunchAttribute attr[1];
+  const cudaLaunchConfig_t cfg = cluster_launch_config(static_cast<int>(clusters), cluster, threads, smem, st, attr);
+  cudaError_t e;
+  if (mpc == nullptr) {
+    auto kernel = icem_plan_general_cluster_kernel<Sys, kH, PRNG>;
+    e = prepare_cluster_kernel(kernel, cluster, smem);
+    if (e != cudaSuccess)
+      return fail(MBPO_ECUDA, "general cluster plan attributes (cluster %d, smem %zu): %s", cluster, smem,
+                  cudaGetErrorString(e));
+    e = cudaLaunchKernelEx(&cfg, kernel, a, R);
+    if (e != cudaSuccess) return fail(MBPO_ECUDA, "icem_plan_general_cluster_kernel launch: %s", cudaGetErrorString(e));
+    return check_launch("icem_plan_general_cluster_kernel");
+  }
+  auto kernel = icem_mpc_general_cluster_kernel<Sys, kH, PRNG>;
+  e = prepare_cluster_kernel(kernel, cluster, smem);
+  if (e != cudaSuccess)
+    return fail(MBPO_ECUDA, "general cluster mpc attributes (cluster %d, smem %zu): %s", cluster, smem,
+                cudaGetErrorString(e));
+  e = cudaLaunchKernelEx(&cfg, kernel, a, *mpc, R);
+  if (e != cudaSuccess) return fail(MBPO_ECUDA, "icem_mpc_general_cluster_kernel launch: %s", cudaGetErrorString(e));
+  return check_launch("icem_mpc_general_cluster_kernel");
 }
 }  // namespace
 
 template <>
-int general_plan_entry<MBPO_INST_H>(int system_kind, int prng_mode, const PlanArgs& a, cudaStream_t st) {
+int general_plan_entry<MBPO_INST_H>(int system_kind, int prng_mode, const PlanArgs& a, const GeneralMpcArgs* mpc,
+                                    cudaStream_t st, int cluster) {
   return with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
-    return with_prng(prng_mode, [&](auto P) { return launch_general<typename decltype(t)::type, P>(a, st); });
+    using Sys = typename decltype(t)::type;
+    return with_prng(prng_mode, [&](auto P) {
+      return cluster > 1 ? launch_general_cluster<Sys, P>(a, mpc, st, cluster) : launch_general<Sys, P>(a, mpc, st);
+    });
   });
+}
+
+template <>
+int general_plan_cluster_capacity<MBPO_INST_H>(int system_kind, int prng_mode, bool mpc, int N, int Np, int K, int P,
+                                               int cluster) {
+  const int n = with_system<NoisyPendulumSys, PointMassSys>(system_kind, [&](auto t) {
+    using Sys = typename decltype(t)::type;
+    return with_prng(prng_mode, [&](auto PR) { return general_cluster_capacity<Sys, PR>(mpc, N, Np, K, P, cluster); });
+  });
+  return n > 0 ? n : 0;
 }
 
 template <>

@@ -139,6 +139,8 @@ SIGNATURES = {
     "mbpo_icem_mpc_closed_loop": (_I, [C.POINTER(IcemCfgC), _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_icem_mpc_closed_loop_clustered": (_I, [C.POINTER(IcemCfgC), _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _I,
                                                  _P]),
+    "mbpo_icem_mpc_closed_loop_general": (_I, [C.POINTER(IcemCfgC), C.POINTER(GeneralSystemParamsC), _P, _P, _P, _P, _I,
+                                               _I, _P, _P, _P, _P, _P, _P, _I, _P]),
     "mbpo_env_rollout": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_env_unroll": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mbpo_actor_rollout": (_I, [_I, _P, _I, _I, C.POINTER(PolicyParamsC), _I, _I, _P, _I, _I, _P, _P, _P, _P, _I, _I,

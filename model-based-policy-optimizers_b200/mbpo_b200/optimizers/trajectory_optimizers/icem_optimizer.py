@@ -373,13 +373,19 @@ class iCemTO(BaseOptimizer):
     def closed_loop(self, initial_state: torch.Tensor, opt_state: iCemOptimizerState, num_steps: int,
                     cluster: int = -1):
         """Returns (states [T, (B,) X], rewards [T, (B)], actions [T, (B,) A], new opt_state).  cluster: as in
-        ``_plan_raw`` (a single problem is spread over 8 SMs by default)."""
+        ``_plan_raw`` (a single problem is spread over 8 SMs by default).  The pendulum and the general Systems
+        (NoisyPendulumSystem, PointMassSystem) run the whole loop in one launch; a System that draws steps with
+        opt_state.system_params.key ([B, 2], or [2] for a single problem) as ``system.step`` does."""
         assert self.system is not None, "iCem optimizer requires system to be defined."
         single, x0, key, seq = self._canon(initial_state, opt_state)
         cfg = self._cfg()
         params = self.system.pack_params(opt_state.system_params)
+        kind = self.system.system_kind
+        general = kind in (_lib.SYSTEM_NOISY_PENDULUM, _lib.SYSTEM_POINT_MASS)
+        sys_key = opt_state.system_params.key if general and self.system.keyed else None
         if (self.cost_fn is not None or self._array_bounds() or not self._fused(cfg, params)
-                or self.system.system_kind != _lib.SYSTEM_PENDULUM):      # the one-launch loop is the pendulum's
+                or not (kind == _lib.SYSTEM_PENDULUM or general)
+                or (general and self.system.keyed and sys_key is None)):   # (system.step raises for the missing key)
             return self._closed_loop_staged(single, x0, key, seq, opt_state, num_steps)
         B, dev = x0.shape[0], x0.device
         H, A = self.opt_dim
@@ -389,10 +395,22 @@ class iCemTO(BaseOptimizer):
         out_seq = torch.empty((B, H, A), dtype=torch.float32, device=dev)
         out_key = torch.empty((B, 2), dtype=torch.uint32, device=dev)
         with _lib.cuda_guard(x0):
-            _lib.check(_lib.lib.mbpo_icem_mpc_closed_loop_clustered(
-                _lib.C.byref(cfg), _lib.C.addressof(params), _lib.ptr(x0), _lib.ptr(key), _lib.ptr(seq), B, num_steps,
-                _lib.ptr(states), _lib.ptr(rewards), _lib.ptr(actions), _lib.ptr(out_seq), _lib.ptr(out_key),
-                int(cluster), _lib.stream_ptr(dev)))
+            if general:
+                sys_keys = sys_key_out = None
+                if sys_key is not None:
+                    sys_keys = sys_key.reshape(-1, 2).contiguous()
+                    if sys_keys.shape[0] != B:
+                        raise ValueError("system_params.key holds %d keys for %d problems" % (sys_keys.shape[0], B))
+                    sys_key_out = torch.empty_like(sys_keys)
+                _lib.check(_lib.lib.mbpo_icem_mpc_closed_loop_general(
+                    _lib.C.byref(cfg), _lib.C.byref(params), _lib.ptr(x0), _lib.ptr(key), _lib.ptr(seq),
+                    _lib.ptr(sys_keys), B, num_steps, _lib.ptr(states), _lib.ptr(rewards), _lib.ptr(actions),
+                    _lib.ptr(out_seq), _lib.ptr(out_key), _lib.ptr(sys_key_out), int(cluster), _lib.stream_ptr(dev)))
+            else:
+                _lib.check(_lib.lib.mbpo_icem_mpc_closed_loop_clustered(
+                    _lib.C.byref(cfg), _lib.C.addressof(params), _lib.ptr(x0), _lib.ptr(key), _lib.ptr(seq), B,
+                    num_steps, _lib.ptr(states), _lib.ptr(rewards), _lib.ptr(actions), _lib.ptr(out_seq),
+                    _lib.ptr(out_key), int(cluster), _lib.stream_ptr(dev)))
         if single:
             states, rewards, actions, out_seq, out_key = states[:, 0], rewards[:, 0], actions[:, 0], out_seq[0], out_key[0]
         return states, rewards, actions, opt_state.replace(key=out_key, best_sequence=out_seq)
