@@ -304,7 +304,7 @@ class iCemTO(BaseOptimizer):
                                                          B * M, P, s_rew, s_cost, lam, st))
                 elif ensemble:
                     # particles = members; the rollout kernel summarises over them itself (:160)
-                    L.check(L.lib.mbpo_ensemble_rollout(L.C.addressof(params), H, L.ptr(x0), L.ptr(actions), B, M,
+                    L.check(L.lib.mbpo_ensemble_rollout(L.C.byref(params), H, L.ptr(x0), L.ptr(actions), B, M,
                                                         s_rew, L.ptr(values), st))
                 else:
                     L.check(L.lib.mbpo_rollout_actions(kind, L.C.addressof(params), config.math_mode_id, H, A, X,
